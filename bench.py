@@ -19,8 +19,17 @@ A "step" = encode all B*12 pictures to .dsv streams, then decode those streams b
   verified  the cpu_baseline leg's reference streams / pictures are compared with the GPU's for the same
           sequences; on a mismatch no line is printed.
   --config 2|3|4|5  BASELINE.json configs (5 = headline metric, default).
-  cpu_baseline  the UNMODIFIED reference (oracle/_ref/libdsv1ref.so, built from /root/reference by
-          oracle/Makefile) single-threaded on a bounded sample of the same workload, rank 0, N=1.
+  cpu_baseline  the UNMODIFIED reference (oracle/_ref/libdsv1ref.so, built by oracle/Makefile from the reference's
+          source tree, its REF) single-threaded on a bounded sample of the same workload, rank 0, N=1.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last device-resident step returned to its caller (rank 0's
+sequences): stream_lengths.npy (float64, one per sequence), streams_sample.npy (float32, sequences x a fixed, seeded set
+of relative positions in each stream) and pictures_sample.npy (float32, sequences x pictures x a fixed, seeded set of
+byte positions in the decoded picture), together at most 64 MB.  The inputs depend on the arguments only, so two builds
+run with the same arguments can be compared output for output.  Two limits: the timed decoder decodes the streams of
+the untimed first step (parked in HBM before timing), so pictures_sample.npy reflects the encoder of that step and the
+timed encoder shows only in the streams; and the stream positions are fractions of each stream's own length, so a
+stream whose length changed is caught by stream_lengths.npy but its sampled bytes no longer line up byte for byte.
 
 `--impl reference` times the reference's own CPU implementation on all host cores (one process per core, the
 reference is not thread-safe), same metric / unit / config.
@@ -108,7 +117,7 @@ def run_reference(args):
     if rank != 0:
         return
     if not L.have_ref():
-        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/libdsv1ref.so missing (built here from /root/reference)"}))
+        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/libdsv1ref.so missing (built by oracle/Makefile from the reference's source tree)"}))
         return
     cores = os.cpu_count() or 1
     procs = max(1, min(cores, 64))
@@ -305,6 +314,24 @@ def measured_traffic():
         return {}
 
 
+def dump_outputs(path, np, torch, d_out, h_streams, cap, lens, seq_bytes):
+    """a fixed, seeded sample of the streams and decoded pictures of the last step (see --dump-outputs), <= 64 MB"""
+    B = len(lens)
+    k = max(1, min(65536, (16 << 20) // (4 * B)))
+    m = max(1, min(8192, (40 << 20) // (4 * B * NFR)))
+    fb = seq_bytes // NFR
+    u = np.random.default_rng(0).random(k)
+    hs = h_streams.numpy()
+    streams = np.stack([hs[s * cap + (u * lens[s]).astype(np.int64)] for s in range(B)]).astype(np.float32)
+    pos = np.sort(np.random.default_rng(1).choice(fb, size=min(m, fb), replace=False))
+    idx = (torch.arange(B * NFR, device=d_out.device)[:, None] * fb + torch.from_numpy(pos).to(d_out.device)[None, :]).reshape(-1)
+    pictures = d_out[idx].cpu().numpy().reshape(B, NFR, len(pos)).astype(np.float32)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "stream_lengths.npy"), np.asarray(lens, dtype=np.float64))
+    np.save(os.path.join(path, "streams_sample.npy"), streams)
+    np.save(os.path.join(path, "pictures_sample.npy"), pictures)
+
+
 def run_product(args):
     import numpy as np
     import torch
@@ -476,6 +503,8 @@ def run_product(args):
     sampler = ClockSampler(local) if rank == 0 else None
     ms_dev, lens, _, _, _, _, split_dev = timed(False, args.steps, args.warmup)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, np, torch, d_out, h_streams, cap, lens, seq_bytes)
     ms_e2e, lens_h, es_h, ds_h, _, _, _ = timed(True, args.steps, args.warmup)
     # the same device-resident steps once more with every launch bracketed by timing events: kernel table + roofline
     ms_prof, _, es, ds, ekt, dkt, _ = timed(False, args.steps, 1, kernel_timing=True)
@@ -587,6 +616,8 @@ def main():
     ap.add_argument("--e2e-parts", type=int, default=1,
                     help="e2e arm: engine pairs the step's sequences are dealt to (measured on one B200, 64 sequences: 1 -> 63 ms per "
                          "step, 2 -> 69, 4 -> 82, 8 -> 109: small engines lose more than the shorter pipeline fill wins)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the last device-resident step's streams and decoded pictures to DIR/*.npy")
     ap.add_argument("--no-e2e-pipeline", dest="e2e_pipeline", action="store_false",
                     help="e2e arm: strictly one step at a time instead of decode(k) overlapping encode(k+1)")
     args = ap.parse_args()

@@ -10,8 +10,7 @@ sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    # checker libraries: the port always builds; the reference only where /root/reference exists
-    # (the GPU box uses the prebuilt oracle/_ref/*.so that travelled with the snapshot)
+    # checker libraries: the port always builds; the reference only where its source tree is present (oracle/Makefile REF)
     try:
         subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "all"], check=True,
                        stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
@@ -33,12 +32,19 @@ def pytest_collection_modifyitems(config, items):
             it.add_marker(skip)
 
 
-@pytest.fixture(scope="session")
-def ref():
+@pytest.fixture
+def ref(request):
+    """The unmodified reference: the library itself where oracle/_ref/libdsv1ref.so is built, otherwise its recorded
+    results (tests/refdigest.py) checked against the library the test exercises."""
     import dsvlibs
-    if not dsvlibs.have_ref():
-        pytest.skip("oracle/_ref/libdsv1ref.so not built (needs /root/reference)")
-    return dsvlibs.ref()
+    import refdigest
+    if dsvlibs.have_ref():
+        lib = dsvlibs.ref()
+        return refdigest.Recorder(lib) if os.environ.get("DSV1_RECORD_REFERENCE") == "1" else lib
+    for name in ("gpu", "emu", "port"):
+        if name in request.fixturenames:
+            return refdigest.RecordedReference(request.getfixturevalue(name))
+    raise LookupError("the ref fixture needs the gpu, emu or port fixture beside it")
 
 
 @pytest.fixture(scope="session")

@@ -1,11 +1,11 @@
 #!/usr/bin/env python3
 """Regenerates tests/golden/streams.json by running the UNMODIFIED reference (oracle/_ref/libdsv1ref.so,
-built by oracle/Makefile from /root/reference) on SURVEY.md Appendix-C synthetic content.
+built by oracle/Makefile from the reference's source tree, its REF) on SURVEY.md Appendix-C synthetic content.
 
 output_options.json pins the decoder's output options (debug overlay, 4:2:0 conversion) the same way.
 
 Each entry pins: md5 of the input yuv, md5 + length of the reference .dsv stream (CRF, -rc_mode1 in CLI
-terms) and md5 of the reference decoder's output.  Run in the build container:  python tests/golden/make_golden.py
+terms) and md5 of the reference decoder's output.  Run:  python tests/golden/make_golden.py
 """
 import hashlib
 import json

@@ -8,6 +8,7 @@ import subprocess
 import pytest
 
 import dsvlibs as L
+import refdigest
 
 REF_MAIN = "/root/reference/dsv_main.c"
 
@@ -78,27 +79,34 @@ def test_every_declared_function_is_exported():
     assert listed - declared <= {"dsv_lvlname"}, sorted(listed - declared)  # the only data symbol
 
 
-def test_public_frame_helpers_match_reference():
+def _frame_helpers(lib):
+    import numpy as np
+    outs = []
+    for (w, h, fmt, seed) in FRAME_HELPER_CASES:
+        sub = L.SUBSAMP[fmt]
+        yuv = L.synth_sequence(w, h, fmt, 1, seed, 0)
+        cap = 64 + ((w + 1) // 2 + 128) * ((h + 1) // 2 + 128) + L.frame_bytes(w, h, sub)
+        o = np.zeros(cap, dtype=np.uint8)
+        f = lib.fn("frame_helpers_probe", api=True)
+        f.restype = ctypes.c_long
+        n = f(L.ptr(yuv), w, h, sub, L.ptr(o), ctypes.c_long(cap))
+        assert n > 0, n
+        outs.append(o[:n])
+    return outs
+
+
+FRAME_HELPER_CASES = [(64, 48, "420", 1), (90, 70, "444", 2), (54, 38, "422", 3), (176, 144, "411", 4)]
+
+
+def test_public_frame_helpers_match_reference(gpu, ref):
     """dsv.h also declares host frame helpers the codec path does not call (dsv_ds2x_frame_luma,
     dsv_extend_frame_luma, dsv_frame_avg_luma, dsv_frame_add, dsv_plane_xy): same caller code
     (tools/api_harness.c: frame_helpers_probe) against both libraries, byte for byte.  Host-only, no GPU."""
     import numpy as np
-    if not L.have_ref():
-        pytest.skip("reference library not built")
-    ref, gpu = L.ref(), L.gpu()
-    for (w, h, fmt, seed) in [(64, 48, "420", 1), (90, 70, "444", 2), (54, 38, "422", 3), (176, 144, "411", 4)]:
-        sub = L.SUBSAMP[fmt]
-        yuv = L.synth_sequence(w, h, fmt, 1, seed, 0)
-        cap = 64 + ((w + 1) // 2 + 128) * ((h + 1) // 2 + 128) + L.frame_bytes(w, h, sub)
-        outs = []
-        for lib in (ref, gpu):
-            o = np.zeros(cap, dtype=np.uint8)
-            f = lib.fn("frame_helpers_probe", api=True)
-            f.restype = ctypes.c_long
-            n = f(L.ptr(yuv), w, h, sub, L.ptr(o), ctypes.c_long(cap))
-            assert n > 0, n
-            outs.append(o[:n])
-        assert np.array_equal(outs[0], outs[1]), (w, h, fmt)
+    got = _frame_helpers(gpu)
+    want = refdigest.table(ref, "frame_helpers_probe", _frame_helpers)
+    for a, b, case in zip(want, got, FRAME_HELPER_CASES):
+        assert np.array_equal(a, b), case
 
 
 def test_nothing_the_reference_headers_declare_is_missing():

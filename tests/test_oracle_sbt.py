@@ -2,6 +2,8 @@
 import numpy as np
 import pytest
 
+import refdigest
+
 SIZES = [  # (plane w, plane h, coef w, coef h)
     (60, 34, 60, 34), (120, 68, 120, 68), (54, 86, 54, 86), (352, 288, 352, 288), (176, 144, 176, 144),
     (427, 240, 428, 240), (959, 539, 960, 540), (135, 67, 136, 68), (16, 16, 16, 16), (480, 270, 480, 270),
@@ -43,10 +45,11 @@ def test_hd_luma(ref, port):
         assert np.array_equal(ref.inv_sbt(co, 313, isP, 0, 1920, 1080), port.inv_sbt(co, 313, isP, 0, 1920, 1080))
 
 
+def _quant_tables(lib):
+    quant = [lib.fn("get_quant")(q, isP, lvl) for q in range(0, 2048, 7) for isP in (0, 1) for lvl in (0, 1, 2)]
+    lb2 = [lib.fn("lb2")(n) for n in list(range(0, 70)) + [255, 256, 257, 4095, 4096, 4097, 1 << 20]]
+    return quant, lb2
+
+
 def test_quant_tables(ref, port):
-    for q in range(0, 2048, 7):
-        for isP in (0, 1):
-            for lvl in (0, 1, 2):
-                assert ref.lib.ref_get_quant(q, isP, lvl) == port.lib.port_get_quant(q, isP, lvl)
-    for n in list(range(0, 70)) + [255, 256, 257, 4095, 4096, 4097, 1 << 20]:
-        assert ref.lib.ref_lb2(n) == port.lib.port_lb2(n)
+    assert refdigest.table(ref, "quant_tables", _quant_tables) == _quant_tables(port)
