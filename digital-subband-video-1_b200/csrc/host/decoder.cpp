@@ -131,12 +131,7 @@ DecEngine::DecEngine(const DSV_META &md, int lanes)
         CUDA_CHECK(cudaMalloc(&l.coef, g.coef_total * sizeof(int32_t)));
         CUDA_CHECK(cudaMemset(l.coef, 0, g.coef_total * sizeof(int32_t)));
         CUDA_CHECK(cudaMalloc(&l.tflags, (size_t) g.total_tiles + 16));
-        for (int p = 0, off = 0; p < 3; off += g.tiles[p], p++) {
-            SbtJob probe;
-            memset(&probe, 0, sizeof(probe));
-            sbt_fill_geometry(&probe, g.pw[p], g.ph[p], g.cw[p], g.ch[p], 1, p);
-            CUDA_CHECK(cudaMemset(l.tflags + off, hz_flag_base(probe.dg), (size_t) g.tiles[p] + (p == 2 ? 16 : 0)));
-        }
+        dec_init_flags(l.tflags, g);
         for (int p = 0; p < 3; p++) {
             CUDA_CHECK(cudaMalloc(&l.llx[p], sbt_llx_elems(g.cw[p], g.ch[p]) * sizeof(int32_t)));
             HzDecPlan pl;
@@ -392,32 +387,9 @@ void DecEngine::step(int n, const int *lane_ids, const PktRef *pkts, const OutRe
         const DevFrame &cur = l.out[l.cur];
         const int isP = l.has_ref;
         for (int p = 0; p < 3; p++) {
-            SbtJob &s = sj[n_sj];
-            memset(&s, 0, sizeof(s));
-            sbt_fill_geometry(&s, g.pw[p], g.ph[p], g.cw[p], g.ch[p], isP, p);
-            sbt_fill_quant(&s, l.quant, isP, p, g.nbh, g.nbv);
-            s.pix = s.opix = cur.p[p];
-            s.pstride = s.ostride = cur.stride[p];
-            s.coef = l.coef + g.coef_off[p];
-            s.llx = l.llx[p];
-            s.stable = d_stab_ + (size_t) li * step_nblk;
-            s.tflags = l.tflags + (p > 0 ? g.tiles[0] : 0) + (p > 1 ? g.tiles[1] : 0);
             HzJob h;
-            memset(&h, 0, sizeof(h));
-            h.cw = g.cw[p];
-            h.ch = g.ch[p];
-            h.plane = p;
-            h.isP = isP;
-            h.pq = s.pq;
-            h.dg = s.dg;
-            hz_fill_regions(&h.rg, g.cw[p], g.ch[p]);
-            h.coef = s.coef;
-            h.stable = s.stable;
-            h.tflags = s.tflags;
-            h.tiles_x = s.tiles_x;
-            /* dsv_decoder.c:405: coefficient planes start zeroed.  Planes that were never coded (corrupt plen) stay
-             * all-zero here; the reference leaves the zeroed residual plane untouched instead. */
-            hzdec_fill_clean(&clean[n_clean++], h, s.tiles_y);
+            dec_fill_plane(&sj[n_sj], &h, &clean[n_clean++], g, p, isP, l.quant, cur, l.coef, l.llx[p], l.tflags,
+                           d_stab_ + (size_t) li * step_nblk);
             if (p < l.nplanes) {
                 hzdec_fill_job(hzj + hzdec_job_size() * (size_t) dims.njobs, h, l.pd[p], l.hz[p], &dims);
             }

@@ -422,15 +422,7 @@ void EncEngine::alloc_lane(EncLane &l)
         CUDA_CHECK(cudaMalloc(&l.dv[p], sbt_dv_elems(g.cw[p], g.ch[p]) * sizeof(int32_t)));
         CUDA_CHECK(cudaMemset(l.dv[p], 0, sbt_dv_elems(g.cw[p], g.ch[p]) * sizeof(int32_t)));
     }
-    /* The reference sizes its packet by a heuristic (w*h*{2,4,6}, dsv_encoder.c:472-491) that noise-like content at
-     * top quality can exceed.  Here the bound is structural: a coefficient costs at most UEG(run = 0) + NEG(symbol)
-     * = 1 + 2 * 17 + 2 bits for symbols below 2^17 (8-bit samples through 6 levels of 3.2x LL gain, divided by a
-     * quantiser >= 16, stay below 2^14), i.e. < 4.75 bytes; hzcc_prefix_kernel refuses what still would not fit. */
-    size_t ub = (size_t) g.w * g.h;
-    ub *= (g.subsamp == DSV_SUBSAMP_444) ? 6 : (g.subsamp == DSV_SUBSAMP_422) ? 4 : 2;
-    size_t pkt_cap = ub + 4096 + (size_t) g.nblk * 48;
-    const size_t bound = g.coef_total * 19 / 4 + 4096 + (size_t) g.nblk * 48;
-    pkt_cap = ((pkt_cap > bound ? pkt_cap : bound) + 255) & ~(size_t) 255;
+    const size_t pkt_cap = enc_packet_cap(g);
     l.pkt_cap = pkt_cap;
     CUDA_CHECK(cudaMalloc(&l.d_pkt, pkt_cap));
     CUDA_CHECK(cudaMemset(l.d_pkt, 0, pkt_cap));
@@ -926,59 +918,25 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
             n_zero++;
         }
         for (int p = 0; p < 3; p++) {
-            SbtJob &s = sj[3 * k + p];
-            memset(&s, 0, sizeof(s));
-            sbt_fill_geometry(&s, g.pw[p], g.ph[p], g.cw[p], g.ch[p], isP, p);
-            sbt_fill_quant(&s, l.quant, isP, p, g.nbh, g.nbv);
-            s.pix = fwd_in.p[p];
-            s.pstride = fwd_in.stride[p];
-            s.opix = inv_out.p[p];
-            s.ostride = inv_out.stride[p];
-            if (isP) {
-                s.addp = l.pred.p[p];
-                s.addstride = l.pred.stride[p];
-            }
-            s.coef = l.coef + g.coef_off[p];
-            s.llx = l.llx[p];
-            s.dv = l.dv[p];
-            s.tflags = l.tflags + (p > 0 ? g.tiles[0] : 0) + (p > 1 ? g.tiles[1] : 0);
-            s.stable = d_stab_ + (size_t) li * g.nblk;
-            s.do_quant = 1;
-
-            HzJob &h = hj[3 * k + p];
-            memset(&h, 0, sizeof(h));
-            h.cw = g.cw[p];
-            h.ch = g.ch[p];
-            h.plane = p;
-            h.isP = isP;
-            h.pq = s.pq;
-            h.dg = s.dg;
-            hz_fill_regions(&h.rg, g.cw[p], g.ch[p]);
-            h.nchunks = g.chunks[p];
-            h.coef = s.coef;
-            h.dv = s.dv;
-            h.tflags = s.tflags;
-            h.tiles_x = ceil_div(g.cw[p], SBT_TW);
-            /* list scratch: the pack pass then reads no coefficient.  P pictures have a handful of dense chunks at
-             * most; those are walked again rather than paying for the dense pack kernel's launch */
-            h.dense = l.hz_dense + (size_t) ((p > 0 ? g.chunks[0] : 0) + (p > 1 ? g.chunks[1] : 0)) * HZ_DENSE_BYTES;
-            h.list_mode = isP ? HZ_LISTS_SPARSE : HZ_LISTS_BOTH;
-            h.stable = s.stable;
-            h.chunk_base = k * g.total_chunks + (p > 0 ? g.chunks[0] : 0) + (p > 1 ? g.chunks[1] : 0);
-            h.frame = k;
+            EncPlaneIO io;
+            io.in = fwd_in.p[p];
+            io.in_stride = fwd_in.stride[p];
+            io.out = inv_out.p[p];
+            io.out_stride = inv_out.stride[p];
+            io.pred = l.pred.p[p];
+            io.pred_stride = l.pred.stride[p];
+            io.coef = l.coef + g.coef_off[p];
+            io.llx = l.llx[p];
+            io.dv = l.dv[p];
+            io.tflags = l.tflags;
+            io.hz_dense = l.hz_dense;
+            io.stable = d_stab_ + (size_t) li * g.nblk;
+            enc_fill_plane(&sj[3 * k + p], &hj[3 * k + p], g, p, k, isP, l.quant, io);
             if (l.is_ref) {
                 ext[3 * qi + p] = plane_ref(l.recon[l.cur], p);
             }
         }
-        HzFrame &hf = h_frames_[k];
-        memset(&hf, 0, sizeof(hf));
-        hf.pkt = l.d_pkt;
-        hf.cap = (unsigned) l.pkt_cap;
-        hf.start_byte = l.head_bytes;
-        hf.nplanes = 3;
-        hf.job[0] = 3 * k;
-        hf.job[1] = 3 * k + 1;
-        hf.job[2] = 3 * k + 2;
+        enc_fill_frame(&h_frames_[k], l.d_pkt, (unsigned) l.pkt_cap, l.head_bytes, k);
         if (l.is_ref) {
             qi++;
         }

@@ -46,6 +46,28 @@ void plan_blocks(CodecGeom *g, int blk_w, int blk_h);
 int size4dim(int dim);
 void predict_mv(const DevMV *mvs, int nbh, int x, int y, int *px, int *py);
 
+/* per-plane job descriptors of picture k of a step (plane_jobs.cpp): the engines and the kernel-level batch entry
+ * points (kernel_api.cu) fill them with the same code */
+struct EncPlaneIO {
+    const uint8_t *in; /* forward input: the picture (I) or its residual (P) */
+    int in_stride;
+    uint8_t *out; /* the inverse's reconstruction */
+    int out_stride;
+    const uint8_t *pred; /* P pictures: prediction the inverse adds on its way out */
+    int pred_stride;
+    int32_t *coef, *llx, *dv; /* this plane's */
+    uint8_t *tflags, *hz_dense; /* the picture's, all three planes */
+    const uint8_t *stable;
+};
+void enc_fill_plane(SbtJob *s, HzJob *h, const CodecGeom &g, int p, int k, int isP, int quant, const EncPlaneIO &io);
+/* bytes of a lane's packet buffer: the largest coded picture of the format plus its head */
+size_t enc_packet_cap(const CodecGeom &g);
+void enc_fill_frame(HzFrame *f, uint8_t *pkt, unsigned cap, unsigned start_byte, int k);
+void dec_fill_plane(SbtJob *s, HzJob *h, HzCleanItem *c, const CodecGeom &g, int p, int isP, int quant, const DevFrame &cur,
+                    int32_t *coef, int32_t *llx, uint8_t *tflags, const uint8_t *stable);
+/* a lane's decoder tile flags before its first picture: every tile at the plane's base value (hz_flag_base) */
+void dec_init_flags(uint8_t *d_tflags, const CodecGeom &g);
+
 /* where one input / output picture lives */
 struct PicRef {
     const uint8_t *plane[3];

@@ -1,0 +1,115 @@
+/*
+ * plane_jobs.cpp -- the per-plane job descriptors of one picture, filled the same way by the engines (encoder.cpp,
+ * decoder.cpp) and by the batch entry points of the kernel-level API (kernel_api.cu) that check them.
+ */
+#include "engine.h"
+
+namespace dsv {
+
+void enc_fill_plane(SbtJob *s, HzJob *h, const CodecGeom &g, int p, int k, int isP, int quant, const EncPlaneIO &io)
+{
+    memset(s, 0, sizeof(*s));
+    sbt_fill_geometry(s, g.pw[p], g.ph[p], g.cw[p], g.ch[p], isP, p);
+    sbt_fill_quant(s, quant, isP, p, g.nbh, g.nbv);
+    s->pix = const_cast<uint8_t *>(io.in);
+    s->pstride = io.in_stride;
+    s->opix = io.out;
+    s->ostride = io.out_stride;
+    if (isP) {
+        s->addp = io.pred;
+        s->addstride = io.pred_stride;
+    }
+    s->coef = io.coef;
+    s->llx = io.llx;
+    s->dv = io.dv;
+    s->tflags = io.tflags ? io.tflags + (p > 0 ? g.tiles[0] : 0) + (p > 1 ? g.tiles[1] : 0) : nullptr;
+    s->stable = io.stable;
+    s->do_quant = 1;
+
+    memset(h, 0, sizeof(*h));
+    h->cw = g.cw[p];
+    h->ch = g.ch[p];
+    h->plane = p;
+    h->isP = isP;
+    h->pq = s->pq;
+    h->dg = s->dg;
+    hz_fill_regions(&h->rg, g.cw[p], g.ch[p]);
+    h->nchunks = g.chunks[p];
+    h->coef = s->coef;
+    h->dv = s->dv;
+    h->tflags = s->tflags;
+    h->tiles_x = ceil_div(g.cw[p], SBT_TW);
+    /* list scratch: the pack pass then reads no coefficient.  P pictures have a handful of dense chunks at most; those
+     * are walked again rather than paying for the dense pack kernel's launch */
+    h->dense = io.hz_dense ? io.hz_dense + (size_t) ((p > 0 ? g.chunks[0] : 0) + (p > 1 ? g.chunks[1] : 0)) * HZ_DENSE_BYTES : nullptr;
+    h->list_mode = isP ? HZ_LISTS_SPARSE : HZ_LISTS_BOTH;
+    h->stable = s->stable;
+    h->chunk_base = k * g.total_chunks + (p > 0 ? g.chunks[0] : 0) + (p > 1 ? g.chunks[1] : 0);
+    h->frame = k;
+}
+
+size_t enc_packet_cap(const CodecGeom &g)
+{
+    /* The reference sizes its packet by a heuristic (w*h*{2,4,6}, dsv_encoder.c:472-491) that noise-like content at
+     * top quality can exceed.  Here the bound is structural: a coefficient costs at most UEG(run = 0) + NEG(symbol)
+     * = 1 + 2 * 17 + 2 bits for symbols below 2^17 (8-bit samples through 6 levels of 3.2x LL gain, divided by a
+     * quantiser >= 16, stay below 2^14), i.e. < 4.75 bytes; hzcc_prefix_kernel refuses what still would not fit. */
+    size_t ub = (size_t) g.w * g.h;
+    ub *= (g.subsamp == DSV_SUBSAMP_444) ? 6 : (g.subsamp == DSV_SUBSAMP_422) ? 4 : 2;
+    const size_t cap = ub + 4096 + (size_t) g.nblk * 48;
+    const size_t bound = g.coef_total * 19 / 4 + 4096 + (size_t) g.nblk * 48;
+    return ((cap > bound ? cap : bound) + 255) & ~(size_t) 255;
+}
+
+void enc_fill_frame(HzFrame *f, uint8_t *pkt, unsigned cap, unsigned start_byte, int k)
+{
+    memset(f, 0, sizeof(*f));
+    f->pkt = pkt;
+    f->cap = cap;
+    f->start_byte = start_byte;
+    f->nplanes = 3;
+    f->job[0] = 3 * k;
+    f->job[1] = 3 * k + 1;
+    f->job[2] = 3 * k + 2;
+}
+
+void dec_fill_plane(SbtJob *s, HzJob *h, HzCleanItem *c, const CodecGeom &g, int p, int isP, int quant, const DevFrame &cur,
+                    int32_t *coef, int32_t *llx, uint8_t *tflags, const uint8_t *stable)
+{
+    memset(s, 0, sizeof(*s));
+    sbt_fill_geometry(s, g.pw[p], g.ph[p], g.cw[p], g.ch[p], isP, p);
+    sbt_fill_quant(s, quant, isP, p, g.nbh, g.nbv);
+    s->pix = s->opix = cur.p[p];
+    s->pstride = s->ostride = cur.stride[p];
+    s->coef = coef + g.coef_off[p];
+    s->llx = llx;
+    s->stable = stable;
+    s->tflags = tflags + (p > 0 ? g.tiles[0] : 0) + (p > 1 ? g.tiles[1] : 0);
+    memset(h, 0, sizeof(*h));
+    h->cw = g.cw[p];
+    h->ch = g.ch[p];
+    h->plane = p;
+    h->isP = isP;
+    h->pq = s->pq;
+    h->dg = s->dg;
+    hz_fill_regions(&h->rg, g.cw[p], g.ch[p]);
+    h->coef = s->coef;
+    h->stable = s->stable;
+    h->tflags = s->tflags;
+    h->tiles_x = s->tiles_x;
+    /* dsv_decoder.c:405: coefficient planes start zeroed.  Planes that were never coded (corrupt plen) stay all-zero
+     * here; the reference leaves the zeroed residual plane untouched instead. */
+    hzdec_fill_clean(c, *h, s->tiles_y);
+}
+
+void dec_init_flags(uint8_t *d_tflags, const CodecGeom &g)
+{
+    for (int p = 0, off = 0; p < 3; off += g.tiles[p], p++) {
+        SbtJob probe;
+        memset(&probe, 0, sizeof(probe));
+        sbt_fill_geometry(&probe, g.pw[p], g.ph[p], g.cw[p], g.ch[p], 1, p);
+        CUDA_CHECK(cudaMemset(d_tflags + off, hz_flag_base(probe.dg), (size_t) g.tiles[p] + (p == 2 ? 16 : 0)));
+    }
+}
+
+} // namespace dsv

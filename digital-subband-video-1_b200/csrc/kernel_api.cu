@@ -10,6 +10,11 @@
 #include "sbt.cuh"
 #include "hzcc.cuh"
 #include "hzcc_dec.cuh"
+#include "frame.cuh"
+#include "motion.cuh"
+#include "dsv1_b200.h"
+#include "dsv1_b200_kernels.h"
+#include "host/engine.h"
 
 #include <vector>
 
@@ -216,9 +221,6 @@ extern "C" int dsvk_decode_plane(const uint8_t *in, int plen, int cw, int ch, in
 }
 
 /* ---- motion: pyramid, HME, BMC ------------------------------------------------------------------ */
-#include "frame.cuh"
-#include "motion.cuh"
-#include "dsv1_b200.h"
 
 namespace {
 
@@ -441,5 +443,479 @@ extern "C" int dsvk_add_pred(const void *mvs, int w, int h, int subsamp, int blk
     devframe_free(&io);
     devframe_free(&ref);
     return 0;
+    DSV_API_END(-100)
+}
+
+/* ---- batch entry points: the engines' own job filling and launch sequence (host/plane_jobs.cpp) ------------------- */
+namespace {
+
+template <typename T> T *dev_alloc(size_t n, bool zero = true)
+{
+    T *p = nullptr;
+    CUDA_CHECK(cudaMalloc(&p, n * sizeof(T) + 16));
+    if (zero) {
+        CUDA_CHECK(cudaMemset(p, 0, n * sizeof(T) + 16));
+    }
+    return p;
+}
+
+void upload_packed(const DevFrame &f, const uint8_t *src)
+{
+    for (int c = 0; c < 3; c++) {
+        CUDA_CHECK(cudaMemcpy2D(f.p[c], f.stride[c], src, f.w[c], f.w[c], f.h[c], cudaMemcpyHostToDevice));
+        src += (size_t) f.w[c] * f.h[c];
+    }
+}
+
+/* one lane of EncEngine (encoder.cpp alloc_lane): the buffers a picture's phase 3 reads and writes */
+struct KLane {
+    DevFrame in, pred, recon;
+    int32_t *coef = nullptr, *llx[3] = {}, *dv[3] = {};
+    uint8_t *tflags = nullptr, *hz_dense = nullptr, *pkt = nullptr;
+    unsigned pkt_dirty = 0;
+};
+
+} // namespace
+
+#define DSVK_PKT_GUARD 4096 /* bytes past the largest cap, where nothing may ever be written */
+
+struct DsvkEnc {
+    CodecGeom g;
+    int max_pics;
+    size_t pkt_bytes, dv_pitch;
+    std::vector<KLane> lanes;
+    HzChunk *chunks = nullptr;
+    HzFrame *frames = nullptr;
+    SbtJob *d_sj = nullptr;
+    HzJob *d_hj = nullptr;
+    ZeroItem *d_zero = nullptr;
+};
+
+extern "C" void *dsvk_enc_create(int w, int h, int subsamp, int blk_w, int blk_h, int max_pics)
+{
+    DSV_API_BEGIN
+    if (w < 16 || h < 16 || (w & 1) || (h & 1) || max_pics < 1) {
+        return nullptr;
+    }
+    DsvkEnc *e = new DsvkEnc;
+    plan_geometry(&e->g, w, h, subsamp);
+    plan_blocks(&e->g, blk_w, blk_h);
+    const CodecGeom &g = e->g;
+    e->max_pics = max_pics;
+    e->pkt_bytes = enc_packet_cap(g);
+    e->dv_pitch = sbt_dv_elems(g.cw[0], g.ch[0]);
+    e->lanes.resize((size_t) max_pics);
+    for (auto &l : e->lanes) {
+        devframe_alloc(&l.in, w, h, subsamp);
+        devframe_alloc(&l.pred, w, h, subsamp);
+        devframe_alloc(&l.recon, w, h, subsamp);
+        l.coef = dev_alloc<int32_t>(g.coef_total);
+        for (int p = 0; p < 3; p++) {
+            l.llx[p] = dev_alloc<int32_t>(sbt_llx_elems(g.cw[p], g.ch[p]));
+            l.dv[p] = dev_alloc<int32_t>(sbt_dv_elems(g.cw[p], g.ch[p]));
+        }
+        l.tflags = dev_alloc<uint8_t>((size_t) g.total_tiles);
+        CUDA_CHECK(cudaMemset(l.tflags, 3, (size_t) g.total_tiles + 16));
+        l.hz_dense = dev_alloc<uint8_t>((size_t) g.total_chunks * HZ_DENSE_BYTES, false);
+        l.pkt = dev_alloc<uint8_t>(e->pkt_bytes + DSVK_PKT_GUARD);
+    }
+    e->chunks = dev_alloc<HzChunk>((size_t) max_pics * g.total_chunks, false);
+    e->frames = dev_alloc<HzFrame>((size_t) max_pics);
+    e->d_sj = dev_alloc<SbtJob>((size_t) 3 * max_pics);
+    e->d_hj = dev_alloc<HzJob>((size_t) 3 * max_pics);
+    e->d_zero = dev_alloc<ZeroItem>((size_t) 2 * max_pics);
+    return e;
+    DSV_API_END(nullptr)
+}
+
+extern "C" long dsvk_enc_pkt_bytes(void *handle) { return (long) static_cast<DsvkEnc *>(handle)->pkt_bytes; }
+
+extern "C" void dsvk_enc_destroy(void *handle)
+{
+    DsvkEnc *e = static_cast<DsvkEnc *>(handle);
+    if (!e) {
+        return;
+    }
+    for (auto &l : e->lanes) {
+        devframe_free(&l.in);
+        devframe_free(&l.pred);
+        devframe_free(&l.recon);
+        cudaFree(l.coef);
+        for (int p = 0; p < 3; p++) {
+            cudaFree(l.llx[p]);
+            cudaFree(l.dv[p]);
+        }
+        cudaFree(l.tflags);
+        cudaFree(l.hz_dense);
+        cudaFree(l.pkt);
+    }
+    cudaFree(e->chunks);
+    cudaFree(e->frames);
+    cudaFree(e->d_sj);
+    cudaFree(e->d_hj);
+    cudaFree(e->d_zero);
+    delete e;
+}
+
+/* phase 3 of EncEngine::step (encoder.cpp) on n pictures, lane k = picture k */
+extern "C" int dsvk_enc_run(void *handle, int n, const DSVK_PIC *pics, const uint8_t *in, const uint8_t *pred, uint8_t *pkt_out,
+                            unsigned *info_out, int32_t *coef_out, int32_t *dv_out, uint8_t *tflags_out, uint8_t *recon_out)
+{
+    DSV_API_BEGIN
+    DsvkEnc *e = static_cast<DsvkEnc *>(handle);
+    const CodecGeom &g = e->g;
+    if (n < 1 || n > e->max_pics) {
+        return -1;
+    }
+    std::vector<SbtJob> sj((size_t) 3 * n);
+    std::vector<HzJob> hj((size_t) 3 * n);
+    std::vector<HzFrame> hf((size_t) n);
+    std::vector<ZeroItem> zero;
+    size_t max_zero = 0;
+    int n_p = 0;
+    for (int k = 0; k < n; k++) {
+        KLane &l = e->lanes[(size_t) k];
+        const DSVK_PIC &pc = pics[k];
+        if (pc.cap > e->pkt_bytes || pc.start_byte + 64 > pc.cap) {
+            return -1;
+        }
+        upload_packed(l.in, in + g.frame_bytes * k);
+        if (pred && pc.isP) {
+            upload_packed(l.pred, pred + g.frame_bytes * k);
+        }
+        /* as the engine: the forward transform ORs its tile flags into zeroed bytes; the packet's dirty prefix is cleared */
+        zero.push_back({l.tflags, ((size_t) g.total_tiles + 15) & ~(size_t) 15});
+        if (l.pkt_dirty) {
+            zero.push_back({l.pkt, ((size_t) l.pkt_dirty + 64 + 15) & ~(size_t) 15});
+        }
+        n_p += pc.isP != 0;
+    }
+    for (const ZeroItem &z : zero) {
+        max_zero = max_zero > z.bytes ? max_zero : z.bytes;
+    }
+    uint8_t *d_stab = dev_alloc<uint8_t>((size_t) g.nblk * n, false);
+    for (int k = 0; k < n; k++) {
+        CUDA_CHECK(cudaMemcpy(d_stab + (size_t) g.nblk * k, pics[k].stable, (size_t) g.nblk, cudaMemcpyHostToDevice));
+        KLane &l = e->lanes[(size_t) k];
+        const int isP = pics[k].isP != 0;
+        for (int p = 0; p < 3; p++) {
+            EncPlaneIO io;
+            io.in = l.in.p[p];
+            io.in_stride = l.in.stride[p];
+            io.out = l.recon.p[p];
+            io.out_stride = l.recon.stride[p];
+            io.pred = pred ? l.pred.p[p] : nullptr;
+            io.pred_stride = l.pred.stride[p];
+            io.coef = l.coef + g.coef_off[p];
+            io.llx = l.llx[p];
+            io.dv = l.dv[p];
+            io.tflags = l.tflags;
+            io.hz_dense = l.hz_dense;
+            io.stable = d_stab + (size_t) g.nblk * k;
+            enc_fill_plane(&sj[(size_t) 3 * k + p], &hj[(size_t) 3 * k + p], g, p, k, isP, pics[k].quant, io);
+        }
+        enc_fill_frame(&hf[(size_t) k], l.pkt, pics[k].cap, pics[k].start_byte, k);
+    }
+    const SbtDims sdims = sbt_assign_tiles(sj.data(), 3 * n);
+    CUDA_CHECK(cudaMemcpy(e->d_sj, sj.data(), sizeof(SbtJob) * sj.size(), cudaMemcpyHostToDevice));
+    CUDA_CHECK(cudaMemcpy(e->d_hj, hj.data(), sizeof(HzJob) * hj.size(), cudaMemcpyHostToDevice));
+    CUDA_CHECK(cudaMemcpy(e->frames, hf.data(), sizeof(HzFrame) * hf.size(), cudaMemcpyHostToDevice));
+    CUDA_CHECK(cudaMemcpy(e->d_zero, zero.data(), sizeof(ZeroItem) * zero.size(), cudaMemcpyHostToDevice));
+    zero_launch(e->d_zero, (int) zero.size(), max_zero, 0);
+    sbt_fwd_launch(e->d_sj, sdims, g.lo_smem, 0);
+    hzcc_enc_launch(e->d_hj, 3 * n, e->chunks, n * g.total_chunks, e->frames, n, 0, g.total_chunks, g.chunks[0], g.chunks[1], n_p < n);
+    sbt_inv_launch(e->d_sj, sdims, g.lo_smem, 0);
+    CUDA_CHECK(cudaDeviceSynchronize());
+    CUDA_CHECK(cudaMemcpy(hf.data(), e->frames, sizeof(HzFrame) * hf.size(), cudaMemcpyDeviceToHost));
+    cudaFree(d_stab);
+    for (int k = 0; k < n; k++) {
+        KLane &l = e->lanes[(size_t) k];
+        const HzFrame &f = hf[(size_t) k];
+        /* as the engine: an overflowed packet is dirty up to its cap */
+        l.pkt_dirty = f.overflow ? pics[k].cap - 64 : f.total_bytes;
+        unsigned *info = info_out + 8 * k;
+        info[0] = f.overflow;
+        info[1] = f.total_bytes;
+        for (int p = 0; p < 3; p++) {
+            info[2 + p] = f.plane_bytes[p];
+            info[5 + p] = (unsigned) sj[(size_t) 3 * k + p].dg.total;
+        }
+        CUDA_CHECK(cudaMemcpy(pkt_out + (e->pkt_bytes + DSVK_PKT_GUARD) * k, l.pkt, e->pkt_bytes + DSVK_PKT_GUARD, cudaMemcpyDeviceToHost));
+        CUDA_CHECK(cudaMemcpy(coef_out + g.coef_total * k, l.coef, g.coef_total * sizeof(int32_t), cudaMemcpyDeviceToHost));
+        for (int p = 0; p < 3; p++) {
+            CUDA_CHECK(cudaMemcpy(dv_out + e->dv_pitch * (3 * k + p), l.dv[p], sbt_dv_elems(g.cw[p], g.ch[p]) * sizeof(int32_t),
+                                  cudaMemcpyDeviceToHost));
+        }
+        CUDA_CHECK(cudaMemcpy(tflags_out + (size_t) g.total_tiles * k, l.tflags, (size_t) g.total_tiles, cudaMemcpyDeviceToHost));
+        download_frame(l.recon, recon_out + g.frame_bytes * k);
+    }
+    return 0;
+    DSV_API_END(-100)
+}
+
+/* the entropy-coding half of phase 3 on caller coefficients and caller tile flags: quantise + dequantise in place
+ * (hzcc_quant_kernel, which the forward transform's epilogue does in the engine), then scan / prefix / pack with the
+ * engine's list scratch and list modes.  Lets a caller place non-zeros at chosen scan positions and chunk edges. */
+extern "C" int dsvk_hz_enc_batch(int w, int h, int subsamp, int blk_w, int blk_h, int n, const DSVK_PIC *pics, int32_t *coef_io,
+                                 const uint8_t *tflags, uint8_t *pkt_out, unsigned *info_out, int32_t *dv_out)
+{
+    DSV_API_BEGIN
+    if (w < 16 || h < 16 || (w & 1) || (h & 1) || n < 1) {
+        return -1;
+    }
+    CodecGeom g;
+    plan_geometry(&g, w, h, subsamp);
+    plan_blocks(&g, blk_w, blk_h);
+    const size_t pkt_bytes = enc_packet_cap(g), dv_pitch = sbt_dv_elems(g.cw[0], g.ch[0]);
+    std::vector<SbtJob> sj((size_t) 3 * n);
+    std::vector<HzJob> hj((size_t) 3 * n);
+    std::vector<HzFrame> hf((size_t) n);
+    std::vector<void *> bufs;
+    auto keep = [&](void *p) { bufs.push_back(p); return p; };
+    int n_p = 0;
+    for (int k = 0; k < n; k++) {
+        if (pics[k].cap > pkt_bytes || pics[k].start_byte + 64 > pics[k].cap) {
+            for (void *b : bufs) {
+                cudaFree(b);
+            }
+            return -1;
+        }
+        int32_t *coef = static_cast<int32_t *>(keep(dev_alloc<int32_t>(g.coef_total, false)));
+        CUDA_CHECK(cudaMemcpy(coef, coef_io + g.coef_total * k, g.coef_total * sizeof(int32_t), cudaMemcpyHostToDevice));
+        uint8_t *tf = nullptr;
+        if (tflags) {
+            tf = static_cast<uint8_t *>(keep(dev_alloc<uint8_t>((size_t) g.total_tiles)));
+            CUDA_CHECK(cudaMemcpy(tf, tflags + (size_t) g.total_tiles * k, (size_t) g.total_tiles, cudaMemcpyHostToDevice));
+        }
+        uint8_t *dense = static_cast<uint8_t *>(keep(dev_alloc<uint8_t>((size_t) g.total_chunks * HZ_DENSE_BYTES, false)));
+        uint8_t *stab = static_cast<uint8_t *>(keep(dev_alloc<uint8_t>((size_t) g.nblk, false)));
+        CUDA_CHECK(cudaMemcpy(stab, pics[k].stable, (size_t) g.nblk, cudaMemcpyHostToDevice));
+        uint8_t *pkt = static_cast<uint8_t *>(keep(dev_alloc<uint8_t>(pkt_bytes + DSVK_PKT_GUARD)));
+        const int isP = pics[k].isP != 0;
+        n_p += isP;
+        for (int p = 0; p < 3; p++) {
+            EncPlaneIO io;
+            memset(&io, 0, sizeof(io));
+            io.coef = coef + g.coef_off[p];
+            io.dv = static_cast<int32_t *>(keep(dev_alloc<int32_t>(sbt_dv_elems(g.cw[p], g.ch[p]))));
+            io.tflags = tf;
+            io.hz_dense = dense;
+            io.stable = stab;
+            enc_fill_plane(&sj[(size_t) 3 * k + p], &hj[(size_t) 3 * k + p], g, p, k, isP, pics[k].quant, io);
+        }
+        enc_fill_frame(&hf[(size_t) k], pkt, pics[k].cap, pics[k].start_byte, k);
+    }
+    HzJob *d_hj = static_cast<HzJob *>(keep(dev_alloc<HzJob>(hj.size(), false)));
+    HzFrame *d_hf = static_cast<HzFrame *>(keep(dev_alloc<HzFrame>(hf.size(), false)));
+    HzChunk *d_ck = static_cast<HzChunk *>(keep(dev_alloc<HzChunk>((size_t) n * g.total_chunks, false)));
+    CUDA_CHECK(cudaMemcpy(d_hj, hj.data(), sizeof(HzJob) * hj.size(), cudaMemcpyHostToDevice));
+    CUDA_CHECK(cudaMemcpy(d_hf, hf.data(), sizeof(HzFrame) * hf.size(), cudaMemcpyHostToDevice));
+    hzcc_quant_launch(d_hj, 3 * n, g.cw[0] * g.ch[0], 0);
+    hzcc_enc_launch(d_hj, 3 * n, d_ck, n * g.total_chunks, d_hf, n, 0, g.total_chunks, g.chunks[0], g.chunks[1], n_p < n);
+    CUDA_CHECK(cudaDeviceSynchronize());
+    CUDA_CHECK(cudaMemcpy(hf.data(), d_hf, sizeof(HzFrame) * hf.size(), cudaMemcpyDeviceToHost));
+    for (int k = 0; k < n; k++) {
+        const HzFrame &f = hf[(size_t) k];
+        unsigned *info = info_out + 8 * k;
+        info[0] = f.overflow;
+        info[1] = f.total_bytes;
+        for (int p = 0; p < 3; p++) {
+            const HzJob &hp = hj[(size_t) 3 * k + p];
+            info[2 + p] = f.plane_bytes[p];
+            info[5 + p] = (unsigned) hp.dg.total;
+            CUDA_CHECK(cudaMemcpy(dv_out + dv_pitch * (3 * k + p), hp.dv, sbt_dv_elems(g.cw[p], g.ch[p]) * sizeof(int32_t),
+                                  cudaMemcpyDeviceToHost));
+        }
+        CUDA_CHECK(cudaMemcpy(pkt_out + (pkt_bytes + DSVK_PKT_GUARD) * k, f.pkt, pkt_bytes + DSVK_PKT_GUARD, cudaMemcpyDeviceToHost));
+        CUDA_CHECK(cudaMemcpy(coef_io + g.coef_total * k, hj[(size_t) 3 * k].coef, g.coef_total * sizeof(int32_t),
+                              cudaMemcpyDeviceToHost));
+    }
+    for (void *b : bufs) {
+        cudaFree(b);
+    }
+    return 0;
+    DSV_API_END(-100)
+}
+
+/* the inverse transform of n pictures in one launch sequence, each picture with its own format */
+extern "C" int dsvk_inv_batch(int n, const int *geo, const DSVK_PIC *pics, const int32_t *coef, const uint8_t *tflags,
+                              const uint8_t *pred, uint8_t *out)
+{
+    DSV_API_BEGIN
+    if (n < 1) {
+        return -1;
+    }
+    std::vector<CodecGeom> g((size_t) n);
+    std::vector<SbtJob> sj((size_t) 3 * n);
+    std::vector<DevFrame> fo((size_t) n), fp((size_t) n);
+    std::vector<void *> bufs;
+    size_t lo_smem = 0;
+    const int32_t *c_at = coef;
+    const uint8_t *t_at = tflags, *p_at = pred;
+    for (int k = 0; k < n; k++) {
+        CodecGeom &gk = g[(size_t) k];
+        if (geo[3 * k] < 16 || geo[3 * k + 1] < 16 || (geo[3 * k] & 1) || (geo[3 * k + 1] & 1)) {
+            return -1;
+        }
+        plan_geometry(&gk, geo[3 * k], geo[3 * k + 1], geo[3 * k + 2]);
+        plan_blocks(&gk, 16, 16);
+        lo_smem = lo_smem > gk.lo_smem ? lo_smem : gk.lo_smem;
+        devframe_alloc(&fo[(size_t) k], gk.w, gk.h, gk.subsamp);
+        devframe_alloc(&fp[(size_t) k], gk.w, gk.h, gk.subsamp);
+        if (pred) {
+            upload_packed(fp[(size_t) k], p_at);
+            p_at += gk.frame_bytes;
+        }
+        int32_t *dc = dev_alloc<int32_t>(gk.coef_total, false);
+        CUDA_CHECK(cudaMemcpy(dc, c_at, gk.coef_total * sizeof(int32_t), cudaMemcpyHostToDevice));
+        c_at += gk.coef_total;
+        bufs.push_back(dc);
+        uint8_t *dt = nullptr;
+        if (tflags) {
+            dt = dev_alloc<uint8_t>((size_t) gk.total_tiles);
+            CUDA_CHECK(cudaMemcpy(dt, t_at, (size_t) gk.total_tiles, cudaMemcpyHostToDevice));
+            t_at += gk.total_tiles;
+            bufs.push_back(dt);
+        }
+        for (int p = 0; p < 3; p++) {
+            int32_t *llx = dev_alloc<int32_t>(sbt_llx_elems(gk.cw[p], gk.ch[p]), false);
+            bufs.push_back(llx);
+            EncPlaneIO io;
+            memset(&io, 0, sizeof(io));
+            io.in = fo[(size_t) k].p[p];
+            io.in_stride = fo[(size_t) k].stride[p];
+            io.out = fo[(size_t) k].p[p];
+            io.out_stride = fo[(size_t) k].stride[p];
+            io.pred = pred ? fp[(size_t) k].p[p] : nullptr;
+            io.pred_stride = fp[(size_t) k].stride[p];
+            io.coef = dc + gk.coef_off[p];
+            io.llx = llx;
+            io.tflags = dt;
+            HzJob unused;
+            enc_fill_plane(&sj[(size_t) 3 * k + p], &unused, gk, p, k, pics[k].isP != 0, pics[k].quant, io);
+        }
+    }
+    const SbtDims sdims = sbt_assign_tiles(sj.data(), 3 * n);
+    SbtJob *d_sj = dev_alloc<SbtJob>(sj.size(), false);
+    CUDA_CHECK(cudaMemcpy(d_sj, sj.data(), sizeof(SbtJob) * sj.size(), cudaMemcpyHostToDevice));
+    sbt_inv_launch(d_sj, sdims, lo_smem, 0);
+    CUDA_CHECK(cudaDeviceSynchronize());
+    uint8_t *o_at = out;
+    for (int k = 0; k < n; k++) {
+        download_frame(fo[(size_t) k], o_at);
+        o_at += g[(size_t) k].frame_bytes;
+        devframe_free(&fo[(size_t) k]);
+        devframe_free(&fp[(size_t) k]);
+    }
+    cudaFree(d_sj);
+    for (void *b : bufs) {
+        cudaFree(b);
+    }
+    return 0;
+    DSV_API_END(-100)
+}
+
+/* one lane of DecEngine (decoder.cpp): coefficient planes and tile flags carry over from picture to picture */
+struct DsvkDec {
+    CodecGeom g;
+    int32_t *coef = nullptr;
+    uint8_t *tflags = nullptr;
+    HzDecPlaneBufs hz[3];
+};
+
+extern "C" void *dsvk_dec_create(int w, int h, int subsamp, int blk_w, int blk_h)
+{
+    DSV_API_BEGIN
+    if (w < 16 || h < 16 || (w & 1) || (h & 1)) {
+        return nullptr;
+    }
+    DsvkDec *d = new DsvkDec;
+    plan_geometry(&d->g, w, h, subsamp);
+    plan_blocks(&d->g, blk_w, blk_h);
+    d->coef = dev_alloc<int32_t>(d->g.coef_total);
+    CUDA_CHECK(cudaMalloc(&d->tflags, (size_t) d->g.total_tiles + 16));
+    dec_init_flags(d->tflags, d->g);
+    for (int p = 0; p < 3; p++) {
+        HzDecPlan pl;
+        hzdec_plan(&pl, d->g.cw[p], d->g.ch[p]);
+        hzdec_plane_alloc(&d->hz[p], pl);
+    }
+    return d;
+    DSV_API_END(nullptr)
+}
+
+extern "C" void dsvk_dec_destroy(void *handle)
+{
+    DsvkDec *d = static_cast<DsvkDec *>(handle);
+    if (!d) {
+        return;
+    }
+    cudaFree(d->coef);
+    cudaFree(d->tflags);
+    for (int p = 0; p < 3; p++) {
+        hzdec_plane_free(&d->hz[p]);
+    }
+    delete d;
+}
+
+/* the coefficient half of DecEngine::step on one picture: planes = the three plane records (32-bit plen, then the
+ * plane's bytes) back to back, len bytes.  Returns the number of planes decoded. */
+extern "C" int dsvk_dec_run(void *handle, const DSVK_PIC *pic, const uint8_t *planes, int len, int32_t *coef_out, uint8_t *tflags_out)
+{
+    DSV_API_BEGIN
+    DsvkDec *d = static_cast<DsvkDec *>(handle);
+    const CodecGeom &g = d->g;
+    if (len <= 0) {
+        return -1;
+    }
+    uint8_t *d_pkt = dev_alloc<uint8_t>((size_t) len + 64);
+    CUDA_CHECK(cudaMemcpy(d_pkt, planes, (size_t) len, cudaMemcpyHostToDevice));
+    uint8_t *d_stab = dev_alloc<uint8_t>((size_t) g.nblk, false);
+    CUDA_CHECK(cudaMemcpy(d_stab, pic->stable, (size_t) g.nblk, cudaMemcpyHostToDevice));
+    /* plane directory (decoder.cpp) */
+    HzPlaneData pd[3];
+    int nplanes = 0;
+    unsigned at = 0;
+    for (int p = 0; p < 3; p++) {
+        if (at + 4 > (unsigned) len) {
+            break;
+        }
+        const int plen = (int) (((unsigned) planes[at] << 24) | ((unsigned) planes[at + 1] << 16) | ((unsigned) planes[at + 2] << 8) | planes[at + 3]);
+        at += 4;
+        const int framesz = g.cw[p] * g.ch[p] * (int) sizeof(int32_t);
+        if (plen <= 0 || plen > framesz * 2 || at >= (unsigned) len) {
+            break;
+        }
+        hzdec_parse_head(planes + at, (unsigned) len - at, (unsigned) plen, &pd[p]);
+        pd[p].body = d_pkt + at;
+        at += (unsigned) plen;
+        nplanes++;
+    }
+    DevFrame unused;
+    SbtJob sj[3];
+    HzCleanItem clean[3];
+    std::vector<uint8_t> hzj(hzdec_job_size() * 3);
+    HzDecDims dims;
+    for (int p = 0; p < 3; p++) {
+        HzJob h;
+        dec_fill_plane(&sj[p], &h, &clean[p], g, p, pic->isP != 0, pic->quant, unused, d->coef, nullptr, d->tflags, d_stab);
+        if (p < nplanes) {
+            hzdec_fill_job(hzj.data() + hzdec_job_size() * (size_t) dims.njobs, h, pd[p], d->hz[p], &dims);
+        }
+    }
+    HzCleanItem *d_clean = dev_alloc<HzCleanItem>(3, false);
+    void *d_hzj = dev_alloc<uint8_t>(hzj.size(), false);
+    CUDA_CHECK(cudaMemcpy(d_clean, clean, sizeof(clean), cudaMemcpyHostToDevice));
+    CUDA_CHECK(cudaMemcpy(d_hzj, hzj.data(), hzj.size(), cudaMemcpyHostToDevice));
+    hzdec_clean_launch(d_clean, 3, g.tiles[0], 0);
+    hzdec_launch_jobs(d_hzj, dims, 0);
+    CUDA_CHECK(cudaDeviceSynchronize());
+    CUDA_CHECK(cudaMemcpy(coef_out, d->coef, g.coef_total * sizeof(int32_t), cudaMemcpyDeviceToHost));
+    CUDA_CHECK(cudaMemcpy(tflags_out, d->tflags, (size_t) g.total_tiles, cudaMemcpyDeviceToHost));
+    cudaFree(d_pkt);
+    cudaFree(d_stab);
+    cudaFree(d_clean);
+    cudaFree(d_hzj);
+    return nplanes;
     DSV_API_END(-100)
 }

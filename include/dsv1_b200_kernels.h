@@ -58,6 +58,54 @@ int dsvk_sub_pred(const void *mvs, int w, int h, int subsamp, int blk_w, int blk
 int dsvk_add_pred(const void *mvs, int w, int h, int subsamp, int blk_w, int blk_h, const uint8_t *resid_yuv,
                   const uint8_t *ref_yuv, uint8_t *out_yuv);
 
+/* ---- batch entry points: the transform and entropy-coding kernels configured as the engines launch them ----------
+ * One call is one launch sequence over n pictures x 3 planes, with the engines' own job filling: tile flags, the
+ * encoder's list scratch and dense pack pass, the fused prediction add, the multi-picture job mapping.  Frames are
+ * packed planar (w x h luma, then two chroma planes of the subsampled size); coefficient planes are the three
+ * planes' dense coefficients back to back (chroma sizes rounded up to even); tile flags are one byte per 128x64 tile
+ * of each plane, planes back to back (bit 0: level-1 band blocks hold a non-zero, bit 1: level-2). */
+typedef struct DSVK_PIC {
+    int isP;               /* P picture (inter quantiser tables; the encoder adds the prediction in its inverse) */
+    int quant;             /* frame quantiser */
+    const uint8_t *stable; /* encoder, decoder: nbh * nbv stability bytes of the handle's block grid */
+    unsigned start_byte;   /* encoder: length of the packet head, plane 0 starts here */
+    unsigned cap;          /* encoder: packet bytes the coder may use, <= dsvk_enc_pkt_bytes() */
+} DSVK_PIC;
+
+/* encoder lanes for up to max_pics pictures of one format; each lane keeps its packet buffer (only the dirty prefix
+ * is cleared before the next call), list scratch and tile flags from call to call */
+void *dsvk_enc_create(int w, int h, int subsamp, int blk_w, int blk_h, int max_pics);
+long dsvk_enc_pkt_bytes(void *enc);
+void dsvk_enc_destroy(void *enc);
+/* forward transform + quantiser -> HZCC scan / prefix / pack -> inverse (+ prediction) of pictures 0..n-1 in lanes
+ * 0..n-1.  in: n frames (the picture, or its residual for P); pred: n frames or NULL.  Out, per picture k:
+ * pkt_out[k * (dsvk_enc_pkt_bytes() + 4096)...] the whole packet buffer including a 4096-byte guard past the largest
+ * cap; info_out[8k..8k+7] = overflow, total bytes, plane bytes Y/U/V, dv counts Y/U/V; coef_out = the dequantised
+ * coefficients; dv_out[(3k + p) * dv_pitch...] the plane's double-visit side buffer, dv_pitch = 2 * (w + h) + 16;
+ * tflags_out = the flags the forward kernel wrote; recon_out = the reconstruction. */
+int dsvk_enc_run(void *enc, int n, const DSVK_PIC *pics, const uint8_t *in, const uint8_t *pred, uint8_t *pkt_out,
+                 unsigned *info_out, int32_t *coef_out, int32_t *dv_out, uint8_t *tflags_out, uint8_t *recon_out);
+
+/* the entropy-coding half of dsvk_enc_run on caller coefficients (coef_io: raw in, dequantised out) and caller tile
+ * flags (NULL: no chunk is skipped): quantiser, then scan / prefix / pack with the engine's list scratch (I pictures:
+ * sparse and dense lists, P: sparse lists).  pkt_out, info_out and dv_out as for dsvk_enc_run; the packet buffer per
+ * picture is enc_packet_cap of the format (dsvk_enc_pkt_bytes of a handle of that format) + 4096 bytes. */
+int dsvk_hz_enc_batch(int w, int h, int subsamp, int blk_w, int blk_h, int n, const DSVK_PIC *pics, int32_t *coef_io,
+                      const uint8_t *tflags, uint8_t *pkt_out, unsigned *info_out, int32_t *dv_out);
+
+/* inverse transform of n pictures in one launch, geo[3k..3k+2] = w, h, subsamp of picture k (formats may differ).
+ * coef: the pictures' coefficient planes back to back; tflags: their tile flags back to back, or NULL (no skipping);
+ * pred: n frames, added on the way out to the P pictures (as the engines do), or NULL. */
+int dsvk_inv_batch(int n, const int *geo, const DSVK_PIC *pics, const int32_t *coef, const uint8_t *tflags,
+                   const uint8_t *pred, uint8_t *out);
+
+/* decoder lane: coefficient planes and tile flags carry over from one picture to the next */
+void *dsvk_dec_create(int w, int h, int subsamp, int blk_w, int blk_h);
+void dsvk_dec_destroy(void *dec);
+/* entropy decoding of one picture: planes = the three plane records (32-bit big-endian plen, then plen bytes) back to
+ * back.  Returns the number of planes decoded; coef_out / tflags_out receive the lane's planes and flags. */
+int dsvk_dec_run(void *dec, const DSVK_PIC *pic, const uint8_t *planes, int len, int32_t *coef_out, uint8_t *tflags_out);
+
 #ifdef __cplusplus
 }
 #endif
