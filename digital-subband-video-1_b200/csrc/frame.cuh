@@ -70,6 +70,13 @@ struct CopyItem { /* control-plane data moved by SMs through mapped pinned host 
     const void *src;
     size_t bytes;
 };
+struct SseJob { /* *out += sum over the pw x ph samples of (src - rec)^2 (quality.cu); both planes bordered DevFrame planes */
+    const uint8_t *src;
+    const uint8_t *rec;
+    int src_stride, rec_stride;
+    int pw, ph;
+    unsigned long long *out;
+};
 struct DevMV;
 struct DrawItem { /* debug overlay (overlay.cu) painted in place on a picture whose three planes are dense */
     uint8_t *dst[3];
@@ -128,6 +135,8 @@ void copy1_launch(void *dst, const void *src, size_t bytes, cudaStream_t st);
 void copyn_launch(const CopyItem *items, int n, cudaStream_t st);
 void overlay_launch(const DrawItem *d_items, int n, cudaStream_t st);
 void to420_launch(const To420Item *d_items, int n, int max_dw, int max_dh, cudaStream_t st);
+/* squared error of every job's plane in ONE launch; the outputs must be zeroed before (quality.cu) */
+void sse_launch(const SseJob *d_jobs, int n, int max_h, cudaStream_t st);
 
 /* single-frame conveniences used by the kernel-level API (kernel_api.cu) */
 void frame_extend_launch(const DevFrame &f, int nplanes, cudaStream_t st);

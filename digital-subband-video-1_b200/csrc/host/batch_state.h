@@ -28,6 +28,9 @@ struct DSVB_ENC {
     size_t cache_bytes = 0;
     cudaStream_t cache_stream = nullptr;
     cudaEvent_t cache_ev[2] = {nullptr, nullptr};
+    /* picture report of the last encode call: records per sequence, valid when the report was on and the call succeeded */
+    bool info_valid = false;
+    std::vector<std::vector<DSVB_PICINFO>> info;
 };
 
 struct DSVB_DEC {
@@ -52,4 +55,6 @@ struct DecSegment {
     int frames;                /* out: pictures decoded */
 };
 int decode_segments(DSVB_DEC *d, int nseg, DecSegment *segs, int out_on_device);
+/* dsvb_enc_picture_info / dsvb_multi_picture_info */
+int copy_picture_info(bool valid, const std::vector<std::vector<DSVB_PICINFO>> &info, int seq, DSVB_PICINFO *out, int cap);
 } // namespace dsv

@@ -458,6 +458,7 @@ void EncEngine::free_lane(EncLane &l)
     cudaFreeHost(l.h_head);
     devframe_free(&l.xf);
     devframe_free(&l.pred);
+    devframe_free(&l.qrec);
     for (int i = 0; i < 2; i++) {
         devframe_free(&l.pad[i]);
         devframe_free(&l.recon[i]);
@@ -492,6 +493,8 @@ EncEngine::~EncEngine()
     cudaFree(d_frames_);
     cudaFreeHost(h_frames_);
     cudaFreeHost(h_pk_);
+    cudaFree(d_sse_);
+    cudaFreeHost(h_sse_);
     for (auto &e : ev_) {
         cudaEventDestroy(e);
     }
@@ -503,6 +506,29 @@ EncEngine::~EncEngine()
     }
     cudaStreamDestroy(st_copy_);
     cudaStreamDestroy(st_);
+}
+
+/* The picture report's buffers, made when a step first runs with it on (no step is in flight then: step() ends with a
+ * stream synchronisation): the sums, the step arena and packet copy list grown by the SSE jobs, their zero item and
+ * the sums' copy item, and for intra-only engines a reconstruction target per lane (their inverse would write in
+ * place over the source). */
+void EncEngine::enable_picture_info()
+{
+    const size_t sums = (sizeof(unsigned long long) * 3 * (size_t) L_ + 15) & ~(size_t) 15;
+    const size_t arena = arena_.cap + (3 * sizeof(SseJob) + 16) * (size_t) L_ + sizeof(ZeroItem) + 64;
+    arena_.destroy();
+    arena_.create(arena);
+    cudaFreeHost(h_pk_);
+    h_pk_ = nullptr;
+    CUDA_CHECK(cudaMallocHost(&h_pk_, sizeof(CopyItem) * ((size_t) L_ + 1)));
+    CUDA_CHECK(cudaMalloc(&d_sse_, sums));
+    CUDA_CHECK(cudaMallocHost(&h_sse_, sums));
+    if (!inter_) {
+        for (auto &l : lanes_) {
+            devframe_alloc(&l.qrec, g_.w, g_.h, g_.subsamp);
+        }
+    }
+    pi_ready_ = true;
 }
 
 static bool packed_pic(const CodecGeom &g, const PicRef &r)
@@ -633,6 +659,10 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
     const bool timed = time_kernels;
     KtActivate kt_on(timed ? &ktimes : nullptr);
     ktimes.open(0);
+    const bool report = picture_info && !analyse;
+    if (report && !pi_ready_) {
+        enable_picture_info();
+    }
     arena_.reset();
 
     /* ---- phase 1: ingest, pyramid, luma sums, motion search -------------------------------------- */
@@ -896,16 +926,21 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
     PlaneRef *ext = n_ref > 0 ? arena_.push_n<PlaneRef>((size_t) 3 * n_ref, &d_ext) : nullptr;
     int qi = 0;
     ZeroItem *d_zero;
-    ZeroItem *zero = arena_.push_n<ZeroItem>((size_t) 2 * n, &d_zero);
+    ZeroItem *zero = arena_.push_n<ZeroItem>((size_t) 2 * n + (report ? 1 : 0), &d_zero);
     int n_zero = 0;
     size_t max_zero = 0;
+    SseJob *d_sse_jobs = nullptr;
+    SseJob *sse_jobs = report ? arena_.push_n<SseJob>((size_t) 3 * n, &d_sse_jobs) : nullptr;
     for (int k = 0; k < n; k++) {
         const int li = lane_ids[k];
         EncLane &l = lanes_[(size_t) li];
         const int isP = l.has_ref;
         const DevFrame &fwd_in = isP ? l.xf : (inter_ ? l.pad[l.cur] : l.xf);
         /* P pictures: the inverse transform adds the prediction on its way out and writes the reconstruction */
-        const DevFrame &inv_out = inter_ ? l.recon[l.cur] : l.xf;
+        const DevFrame &inv_out = inter_ ? l.recon[l.cur] : (report ? l.qrec : l.xf);
+        if (report) { /* the ingested source against the reconstruction */
+            sse_fill_picture(&sse_jobs[3 * k], g, inter_ ? l.pad[l.cur] : l.xf, inv_out, d_sse_ + 3 * k);
+        }
         /* tile flags (sbt.cuh): the forward transform ORs into zeroed bytes */
         zero[n_zero].p = l.tflags;
         zero[n_zero].bytes = ((size_t) g.total_tiles + 15) & ~(size_t) 15;
@@ -941,6 +976,12 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
             qi++;
         }
     }
+    if (report) {
+        zero[n_zero].p = d_sse_;
+        zero[n_zero].bytes = (sizeof(unsigned long long) * 3 * (size_t) n + 15) & ~(size_t) 15;
+        max_zero = max_zero > zero[n_zero].bytes ? max_zero : zero[n_zero].bytes;
+        n_zero++;
+    }
     const SbtDims sdims = sbt_assign_tiles(sj, 3 * n);
     {
         CopyItem up[3] = {{nullptr, nullptr, 0}, {d_stab_, h_stab_, (size_t) g.nblk * L_}, {d_hf, h_frames_, sizeof(HzFrame) * (size_t) n}};
@@ -953,11 +994,20 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
     stats.kernel_launches += 6;
     copy1_launch(h_frames_, d_hf, sizeof(HzFrame) * (size_t) n, st);
     CUDA_CHECK(cudaEventRecord(ev_sizes_, st));
-    if (n_ref) {
+    /* the report also needs the reconstruction of pictures that are not references (intra-only engines) */
+    const int n_inv = report ? n : n_ref;
+    if (n_inv) {
         /* closed loop: reconstruct exactly what the decoder will (dsv_encoder.c:525,662-674) */
         sbt_inv_launch(d_sj, sdims, g.lo_smem, st, timed ? ev_[2] : nullptr, timed ? ev_[3] : nullptr);
+        stats.kernel_launches += 3;
+    }
+    if (n_ref) {
         extend_launch(d_ext, 3 * n_ref, g.w, g.h, st);
-        stats.kernel_launches += 4;
+        stats.kernel_launches += 1;
+    }
+    if (report) {
+        sse_launch(d_sse_jobs, 3 * n, g.h, st);
+        stats.kernel_launches += 1;
     }
     CUDA_CHECK(cudaEventSynchronize(ev_sizes_)); /* packet sizes are known; reconstruction keeps running */
     CopyItem *pk = reinterpret_cast<CopyItem *>(h_pk_); /* mapped pinned: read by the copy kernel in place */
@@ -1032,10 +1082,38 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
         bufs[k][nb++] = outbuf;
         nbufs[k] = nb;
     }
+    if (report) { /* the sums leave with the packets */
+        pk[n_pk].dst = h_sse_;
+        pk[n_pk].src = d_sse_;
+        pk[n_pk].bytes = sizeof(unsigned long long) * 3 * (size_t) n;
+        max_pk = max_pk > pk[n_pk].bytes ? max_pk : pk[n_pk].bytes;
+        n_pk++;
+    }
     copy_launch(pk, n_pk, max_pk, st);
     CUDA_CHECK(cudaStreamSynchronize(st));
     ktimes.collect(0);
     stats.pictures += (unsigned) n;
+    if (report) {
+        pic_info.assign((size_t) n, DSVB_PICINFO());
+        pic_info_ok.assign((size_t) n, 0);
+        for (int k = 0; k < n; k++) {
+            const EncLane &l = lanes_[(size_t) lane_ids[k]];
+            if (h_frames_[k].overflow) {
+                continue;
+            }
+            DSVB_PICINFO &r = pic_info[(size_t) k];
+            for (int p = 0; p < 3; p++) {
+                r.sse[p] = h_sse_[3 * k + p];
+                r.samples[p] = (int64_t) g.pw[p] * g.ph[p];
+            }
+            r.fnum = (int64_t) l.fnum;
+            r.is_p = l.has_ref;
+            r.forced_intra = plan ? plan[k].forced_intra : (inter_ && !l.has_ref && !l.gop_start);
+            r.quant = l.quant;
+            r.bytes = (int32_t) h_frames_[k].total_bytes;
+            pic_info_ok[(size_t) k] = 1;
+        }
+    }
     if (timed) {
         float ms = 0;
         CUDA_CHECK(cudaEventElapsedTime(&ms, ev_[0], ev_[1]));
@@ -1046,7 +1124,7 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
             bytes += (unsigned long long) g.cw[p] * g.ph[p] + 4ull * g.cw[p] * g.ch[p];
         }
         stats.sbt_fwd_bytes += bytes * (unsigned) n;
-        if (n_ref) {
+        if (n_inv) {
             CUDA_CHECK(cudaEventElapsedTime(&ms, ev_[2], ev_[3]));
             stats.sbt_inv_ms += ms;
             stats.sbt_inv_launches++;

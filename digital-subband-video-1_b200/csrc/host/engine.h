@@ -19,6 +19,7 @@
 #include <vector>
 
 #include "dsv1_b200.h"
+#include "dsv1_b200_batch.h"
 
 #include "../frame.cuh"
 #include "../hzcc.cuh"
@@ -63,6 +64,8 @@ void enc_fill_plane(SbtJob *s, HzJob *h, const CodecGeom &g, int p, int k, int i
 /* bytes of a lane's packet buffer: the largest coded picture of the format plus its head */
 size_t enc_packet_cap(const CodecGeom &g);
 void enc_fill_frame(HzFrame *f, uint8_t *pkt, unsigned cap, unsigned start_byte, int k);
+/* squared-error jobs of the three planes of a picture: out[p] receives plane p's sum */
+void sse_fill_picture(SseJob *j, const CodecGeom &g, const DevFrame &src, const DevFrame &rec, unsigned long long *out);
 void dec_fill_plane(SbtJob *s, HzJob *h, HzCleanItem *c, const CodecGeom &g, int p, int isP, int quant, const DevFrame &cur,
                     int32_t *coef, int32_t *llx, uint8_t *tflags, const uint8_t *stable);
 /* a lane's decoder tile flags before its first picture: every tile at the plane's base value (hz_flag_base) */
@@ -196,6 +199,7 @@ private:
 struct EncLane {
     DSV_ENCODER *enc = nullptr; /* host-side state of this sequence */
     DevFrame pad[2], recon[2], pyr[2][DSV_MAX_PYRAMID_LEVELS], xf, pred;
+    DevFrame qrec; /* picture report of an intra-only engine: the reconstruction its pictures otherwise never get */
     int cur = 0, have_ref = 0;
     DevMV *d_mvf[DSV_MAX_PYRAMID_LEVELS + 1] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     int2 *d_aux = nullptr;
@@ -242,6 +246,7 @@ struct LongPlan {
     /* code: */
     DSV_FNUM fnum;
     int has_ref, is_ref, quant;
+    int forced_intra;      /* an I picture where the GOP asked for a P picture (picture report only) */
     const DevMV *mvs;      /* has_ref: vectors from the analysis pass */
     const uint8_t *stable; /* stable_blocks of this picture (nblk bytes) */
     const uint8_t *head;   /* packet head: header .. quantiser, head_bytes long */
@@ -301,9 +306,17 @@ public:
      * ~40 us to EVERY launch (measured: device-resident encode 40 -> 81 ms next to an unrelated bulk D2H copy).
      * Off unless asked for (dsvb_*_set_kernel_timing, DSV_KERNEL_TIMES=1). */
     bool time_kernels = false;
+    /* Per-picture report (dsvb_enc_set_picture_info): when on, every coding step also measures each picture's squared
+     * error against its reconstruction and fills pic_info[k] (pic_info_ok[k] = 0: picture k was dropped, no record).
+     * Costs one more launch per step, plus the inverse transform (3 launches) in steps whose pictures are not
+     * references.  Off: nothing of it runs or is allocated. */
+    bool picture_info = false;
+    std::vector<DSVB_PICINFO> pic_info;
+    std::vector<char> pic_info_ok;
     int device = 0;
 
 private:
+    void enable_picture_info();
     void alloc_lane(EncLane &l);
     void free_lane(EncLane &l);
     CodecGeom g_;
@@ -324,6 +337,8 @@ private:
     HzChunk *d_chunks_ = nullptr;
     HzFrame *d_frames_ = nullptr, *h_frames_ = nullptr;
     void *h_pk_ = nullptr; /* packet egress copy list (mapped pinned) */
+    bool pi_ready_ = false; /* the picture report's buffers exist */
+    unsigned long long *d_sse_ = nullptr, *h_sse_ = nullptr; /* 3 sums per lane; h_sse_ mapped pinned */
     HostPool *pool_ = nullptr;
     uint8_t *d_in_all_[ENC_STAGE_SLOTS] = {}; /* packed-picture staging of all lanes, lane pitch in_pitch_ */
     size_t in_pitch_ = 0;

@@ -63,6 +63,7 @@ struct LongCtx {
     std::vector<char> gop_start;
     std::vector<int> chain_first;  /* first picture of every chain, plus nframes as the sentinel */
     std::vector<std::vector<uint8_t>> pkt; /* coded picture packets */
+    std::vector<DSVB_PICINFO> info;         /* picture report, by picture index */
     int forced = 0;
     int err = 0;
 };
@@ -88,6 +89,7 @@ void ctx_init(LongCtx &c, const DSVB_ENC *e, int nframes, const uint8_t *yuv, in
     c.plan.assign(n, LongPlan());
     c.gop_start.assign(n, 0);
     c.pkt.resize(n);
+    c.info.assign(e->eng->picture_info ? n : 0, DSVB_PICINFO());
 }
 
 /*
@@ -270,12 +272,13 @@ void long_decide(LongCtx &c)
         p.has_ref = has_ref;
         p.is_ref = is_ref;
         p.quant = quant;
+        p.forced_intra = (c.inter && !has_ref && !gop_start) ? 1 : 0;
         p.mvs = an.mvs;
         p.stable = c.stab.data() + (size_t) t * g.nblk;
         p.head = head;
         p.head_bytes = head_bytes;
         c.gop_start[(size_t) t] = (char) gop_start;
-        c.forced += (c.inter && !has_ref && !gop_start) ? 1 : 0; /* I pictures that are not GOP starts */
+        c.forced += p.forced_intra; /* I pictures that are not GOP starts */
         if (!has_ref) {
             c.chain_first.push_back(t);
         }
@@ -371,6 +374,9 @@ void long_code(DSVB_ENC *e, LongCtx &c, PicSource &ps, int k0, int k1)
             }
             const DSV_BUF &b = bufs[(size_t) 2 * q];
             c.pkt[(size_t) t].assign(b.data, b.data + b.len);
+            if (!c.info.empty()) {
+                c.info[(size_t) t] = eng->pic_info[(size_t) q];
+            }
         }
         /* now commit the lane -> chain assignment the prefetch was made for (a lane that takes a new chain forgets
          * its reference only after the last picture of its old chain has been coded) */
@@ -422,6 +428,14 @@ int long_gather(LongCtx &c, uint8_t *stream, long cap, long *len)
     return rc;
 }
 
+/* the picture report of a long encode (ctx_init sized it when the report was on): one sequence */
+void take_info(LongCtx &c, int rc, bool *valid, std::vector<std::vector<DSVB_PICINFO>> *info)
+{
+    *valid = rc == 0 && !c.info.empty();
+    info->assign(1, std::vector<DSVB_PICINFO>());
+    (*info)[0].swap(c.info);
+}
+
 void fill_info(const LongCtx &c, int *info)
 {
     if (info) {
@@ -464,6 +478,8 @@ extern "C" int dsvb_encode_long(DSVB_ENC *e, int nframes, const uint8_t *yuv, in
 {
     DSV_API_BEGIN
     use_device(e->device);
+    e->info_valid = false;
+    e->info.clear();
     if (nframes <= 0) {
         return -2;
     }
@@ -485,7 +501,9 @@ extern "C" int dsvb_encode_long(DSVB_ENC *e, int nframes, const uint8_t *yuv, in
     long_decide(c);
     long_code(e, c, ps, 0, (int) c.chain_first.size() - 1);
     fill_info(c, info);
-    return long_gather(c, stream, cap, len);
+    const int rc = long_gather(c, stream, cap, len);
+    take_info(c, rc, &e->info_valid, &e->info);
+    return rc;
     DSV_API_END(-100)
 }
 
@@ -566,6 +584,9 @@ struct DSVB_MULTI {
     std::vector<int> devices;
     std::vector<DSVB_ENC *> enc;
     std::vector<DSVB_DEC *> dec;
+    bool picture_info = false;
+    bool info_valid = false; /* picture report of the last encode call, as DSVB_ENC */
+    std::vector<std::vector<DSVB_PICINFO>> info;
 };
 
 extern "C" DSVB_MULTI *dsvb_multi_create(const int *cfg, int lanes, int ndev, const int *devices)
@@ -635,6 +656,9 @@ bool multi_encoders(DSVB_MULTI *m)
             m->enc[(size_t) i] = dsvb_enc_create(m->cfg, m->lanes, m->devices[(size_t) i]);
         }
         ok[(size_t) i] = m->enc[(size_t) i] != nullptr;
+        if (ok[(size_t) i]) {
+            m->enc[(size_t) i]->eng->picture_info = m->picture_info;
+        }
     });
     for (int v : ok) {
         if (!v) {
@@ -655,11 +679,28 @@ void multi_decoders(DSVB_MULTI *m)
 
 } // namespace
 
+extern "C" void dsvb_multi_set_picture_info(DSVB_MULTI *m, int on)
+{
+    m->picture_info = on != 0;
+    for (DSVB_ENC *e : m->enc) {
+        if (e) {
+            e->eng->picture_info = m->picture_info;
+        }
+    }
+}
+
+extern "C" int dsvb_multi_picture_info(DSVB_MULTI *m, int seq, DSVB_PICINFO *out, int cap)
+{
+    return copy_picture_info(m->info_valid, m->info, seq, out, cap);
+}
+
 /* whole sequences dealt to the GPUs in contiguous runs */
 extern "C" int dsvb_multi_encode(DSVB_MULTI *m, int nseq, int nframes, const uint8_t *const *yuv, uint8_t *const *streams,
                                  const long *caps, long *lens)
 {
     DSV_API_BEGIN
+    m->info_valid = false;
+    m->info.clear();
     if (!multi_encoders(m)) {
         return -100;
     }
@@ -673,6 +714,16 @@ extern "C" int dsvb_multi_encode(DSVB_MULTI *m, int nseq, int nframes, const uin
         if (v) {
             return v;
         }
+    }
+    if (m->picture_info) { /* device i coded sequences [s0, s1) as its sequences 0 .. s1 - s0 - 1 */
+        m->info.resize((size_t) nseq);
+        for (int i = 0; i < nd; i++) {
+            const int s0 = (int) ((long long) nseq * i / nd), s1 = (int) ((long long) nseq * (i + 1) / nd);
+            for (int s = s0; s < s1; s++) {
+                m->info[(size_t) s].swap(m->enc[(size_t) i]->info[(size_t) (s - s0)]);
+            }
+        }
+        m->info_valid = true;
     }
     return 0;
     DSV_API_END(-100)
@@ -702,11 +753,16 @@ extern "C" int dsvb_multi_decode(DSVB_MULTI *m, int nseq, const uint8_t *const *
 extern "C" int dsvb_multi_encode_long(DSVB_MULTI *m, int nframes, const uint8_t *yuv, uint8_t *stream, long cap, long *len, int *info)
 {
     DSV_API_BEGIN
+    m->info_valid = false;
+    m->info.clear();
     if (!multi_encoders(m) || nframes <= 0) {
         return -100;
     }
     if (m->cfg[CFG_RC_MODE] != DSV_RATE_CONTROL_CRF || m->ndev == 1) {
-        return dsvb_encode_long(m->enc[0], nframes, yuv, 0, stream, cap, len, info);
+        const int rc = dsvb_encode_long(m->enc[0], nframes, yuv, 0, stream, cap, len, info);
+        m->info_valid = m->enc[0]->info_valid;
+        m->info.swap(m->enc[0]->info);
+        return rc;
     }
     LongCtx c;
     ctx_init(c, m->enc[0], nframes, yuv, 0);
@@ -757,7 +813,9 @@ extern "C" int dsvb_multi_encode_long(DSVB_MULTI *m, int nframes, const uint8_t 
     if (info) {
         info[3] = nd;
     }
-    return long_gather(c, stream, cap, len);
+    const int rc = long_gather(c, stream, cap, len);
+    take_info(c, rc, &m->info_valid, &m->info);
+    return rc;
     DSV_API_END(-100)
 }
 

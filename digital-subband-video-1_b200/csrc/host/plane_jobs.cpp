@@ -73,6 +73,19 @@ void enc_fill_frame(HzFrame *f, uint8_t *pkt, unsigned cap, unsigned start_byte,
     f->job[2] = 3 * k + 2;
 }
 
+void sse_fill_picture(SseJob *j, const CodecGeom &g, const DevFrame &src, const DevFrame &rec, unsigned long long *out)
+{
+    for (int p = 0; p < 3; p++) {
+        j[p].src = src.p[p];
+        j[p].src_stride = src.stride[p];
+        j[p].rec = rec.p[p];
+        j[p].rec_stride = rec.stride[p];
+        j[p].pw = g.pw[p];
+        j[p].ph = g.ph[p];
+        j[p].out = out + p;
+    }
+}
+
 void dec_fill_plane(SbtJob *s, HzJob *h, HzCleanItem *c, const CodecGeom &g, int p, int isP, int quant, const DevFrame &cur,
                     int32_t *coef, int32_t *llx, uint8_t *tflags, const uint8_t *stable)
 {

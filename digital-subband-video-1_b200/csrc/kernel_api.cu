@@ -815,6 +815,53 @@ extern "C" int dsvk_inv_batch(int n, const int *geo, const DSVK_PIC *pics, const
     DSV_API_END(-100)
 }
 
+extern "C" int dsvk_sse_batch(int n, const int *geo, const uint8_t *src, const uint8_t *rec, const uint8_t *border_fill, uint64_t *sse_out)
+{
+    DSV_API_BEGIN
+    if (n < 1) {
+        return -1;
+    }
+    std::vector<DevFrame> fs((size_t) n), fr((size_t) n);
+    std::vector<SseJob> jobs((size_t) 3 * n);
+    unsigned long long *d_out = dev_alloc<unsigned long long>((size_t) 3 * n);
+    const uint8_t *s_at = src, *r_at = rec;
+    int max_h = 0;
+    int rc = 0;
+    for (int k = 0; k < n && rc == 0; k++) {
+        if (geo[3 * k] < 16 || geo[3 * k + 1] < 16 || (geo[3 * k] & 1) || (geo[3 * k + 1] & 1)) {
+            rc = -1;
+            break;
+        }
+        CodecGeom g;
+        plan_geometry(&g, geo[3 * k], geo[3 * k + 1], geo[3 * k + 2]);
+        devframe_alloc(&fs[(size_t) k], g.w, g.h, g.subsamp);
+        devframe_alloc(&fr[(size_t) k], g.w, g.h, g.subsamp);
+        CUDA_CHECK(cudaMemset(fs[(size_t) k].alloc, border_fill[0], fs[(size_t) k].bytes));
+        CUDA_CHECK(cudaMemset(fr[(size_t) k].alloc, border_fill[1], fr[(size_t) k].bytes));
+        upload_packed(fs[(size_t) k], s_at);
+        upload_packed(fr[(size_t) k], r_at);
+        s_at += g.frame_bytes;
+        r_at += g.frame_bytes;
+        sse_fill_picture(&jobs[(size_t) 3 * k], g, fs[(size_t) k], fr[(size_t) k], d_out + 3 * k);
+        max_h = max_h > g.h ? max_h : g.h;
+    }
+    if (rc == 0) {
+        SseJob *d_jobs = dev_alloc<SseJob>(jobs.size(), false);
+        CUDA_CHECK(cudaMemcpy(d_jobs, jobs.data(), sizeof(SseJob) * jobs.size(), cudaMemcpyHostToDevice));
+        sse_launch(d_jobs, 3 * n, max_h, 0);
+        CUDA_CHECK(cudaDeviceSynchronize());
+        CUDA_CHECK(cudaMemcpy(sse_out, d_out, sizeof(uint64_t) * 3 * n, cudaMemcpyDeviceToHost));
+        cudaFree(d_jobs);
+    }
+    for (int k = 0; k < n; k++) {
+        devframe_free(&fs[(size_t) k]);
+        devframe_free(&fr[(size_t) k]);
+    }
+    cudaFree(d_out);
+    return rc;
+    DSV_API_END(-100)
+}
+
 /* one lane of DecEngine (decoder.cpp): coefficient planes and tile flags carry over from picture to picture */
 struct DsvkDec {
     CodecGeom g;

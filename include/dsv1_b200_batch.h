@@ -121,6 +121,32 @@ const char *dsvb_kernel_name(int i);
 void dsvb_enc_kernel_times(DSVB_ENC *e, double *ms, double *launches, int reset);
 void dsvb_dec_kernel_times(DSVB_DEC *d, double *ms, double *launches, int reset);
 
+/*
+ * Per-picture report of the encoders: squared error against the source, frame type, quantiser and size of every
+ * coded picture.  Off by default; while off the encoders do exactly what they do without it (same bytes, launches
+ * and allocations).  When on, the closed-loop reconstruction (what a decoder outputs) is compared with the source on
+ * the GPU, and pictures that are not references (every picture of a gop = 0 encoder) get the inverse transform they
+ * otherwise skip.  The streams do not change.
+ *   dsvb_enc_picture_info / dsvb_multi_picture_info: the records of sequence `seq` of the last dsvb_encode /
+ *   dsvb_multi_encode call (seq 0 for dsvb_encode_long / dsvb_multi_encode_long), in picture order.  Returns the
+ *   number of records and writes at most `cap` of them; -1 if the report was off during that call, the call failed,
+ *   or seq is out of range.
+ * PSNR of plane p: 10 * log10(255^2 * samples[p] / sse[p]) (infinite when sse[p] == 0).
+ */
+typedef struct DSVB_PICINFO { /* 72 bytes, no padding */
+    uint64_t sse[3];          /* sum over the plane of (source - reconstruction)^2, Y U V; the reconstruction is what a decoder outputs */
+    int64_t samples[3];       /* pw * ph per plane, so PSNR = 10 log10(255^2 * samples / sse) needs no subsampling rules */
+    int64_t fnum;             /* frame number written in the packet */
+    int32_t is_p;             /* 1: P picture, 0: I picture */
+    int32_t forced_intra;     /* a P picture turned into I (scene change / intra share) */
+    int32_t quant;            /* quantiser written in the packet */
+    int32_t bytes;            /* picture packet incl. head; metadata packets excluded */
+} DSVB_PICINFO;
+void dsvb_enc_set_picture_info(DSVB_ENC *e, int on);
+int dsvb_enc_picture_info(DSVB_ENC *e, int seq, DSVB_PICINFO *out, int cap);
+void dsvb_multi_set_picture_info(DSVB_MULTI *m, int on);
+int dsvb_multi_picture_info(DSVB_MULTI *m, int seq, DSVB_PICINFO *out, int cap);
+
 /* pinned host memory for inputs / outputs of the calls above */
 void *dsvb_host_alloc(size_t bytes);
 void dsvb_host_free(void *p);

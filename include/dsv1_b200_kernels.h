@@ -99,6 +99,11 @@ int dsvk_hz_enc_batch(int w, int h, int subsamp, int blk_w, int blk_h, int n, co
 int dsvk_inv_batch(int n, const int *geo, const DSVK_PIC *pics, const int32_t *coef, const uint8_t *tflags,
                    const uint8_t *pred, uint8_t *out);
 
+/* squared error of n picture pairs in one launch, as the batch encoder's picture report measures it: geo as for
+ * dsvk_inv_batch; src / rec hold n packed frames each.  Both are placed in bordered device frames whose border and
+ * padding bytes are set to border_fill[0] (src) and border_fill[1] (rec).  sse_out: 3 sums per picture, Y U V. */
+int dsvk_sse_batch(int n, const int *geo, const uint8_t *src, const uint8_t *rec, const uint8_t *border_fill, uint64_t *sse_out);
+
 /* decoder lane: coefficient planes and tile flags carry over from one picture to the next */
 void *dsvk_dec_create(int w, int h, int subsamp, int blk_w, int blk_h);
 void dsvk_dec_destroy(void *dec);
