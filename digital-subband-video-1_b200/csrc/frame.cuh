@@ -70,7 +70,8 @@ struct CopyItem { /* control-plane data moved by SMs through mapped pinned host 
     const void *src;
     size_t bytes;
 };
-struct SseJob { /* *out += sum over the pw x ph samples of (src - rec)^2 (quality.cu); both planes bordered DevFrame planes */
+struct SseJob { /* *out += sum over the pw x ph samples of (src - rec)^2 (quality.cu); both planes bordered DevFrame planes.
+                  ssim_kernel takes the same jobs and adds the plane's sum of rint(ssim_w * 2^32) to *out (two's complement) */
     const uint8_t *src;
     const uint8_t *rec;
     int src_stride, rec_stride;
@@ -137,6 +138,9 @@ void overlay_launch(const DrawItem *d_items, int n, cudaStream_t st);
 void to420_launch(const To420Item *d_items, int n, int max_dw, int max_dh, cudaStream_t st);
 /* squared error of every job's plane in ONE launch; the outputs must be zeroed before (quality.cu) */
 void sse_launch(const SseJob *d_jobs, int n, int max_h, cudaStream_t st);
+/* SSIM window sums of every job's plane in ONE launch (one launch even when no plane has a window); the outputs must be
+ * zeroed before (quality.cu) */
+void ssim_launch(const SseJob *d_jobs, int n, int max_pw, int max_ph, cudaStream_t st);
 
 /* single-frame conveniences used by the kernel-level API (kernel_api.cu) */
 void frame_extend_launch(const DevFrame &f, int nplanes, cudaStream_t st);

@@ -172,23 +172,16 @@ extern "C" void dsvb_dec_set_kernel_timing(DSVB_DEC *d, int on)
 }
 
 extern "C" void dsvb_enc_set_picture_info(DSVB_ENC *e, int on) { e->eng->picture_info = on != 0; }
-
-int dsv::copy_picture_info(bool valid, const std::vector<std::vector<DSVB_PICINFO>> &info, int seq, DSVB_PICINFO *out, int cap)
-{
-    if (!valid || seq < 0 || seq >= (int) info.size()) {
-        return -1;
-    }
-    const std::vector<DSVB_PICINFO> &r = info[(size_t) seq];
-    const int n = (int) r.size();
-    if (out && cap > 0) {
-        memcpy(out, r.data(), sizeof(DSVB_PICINFO) * (size_t) (n < cap ? n : cap));
-    }
-    return n;
-}
+extern "C" void dsvb_enc_set_picture_ssim(DSVB_ENC *e, int on) { e->eng->picture_ssim = on != 0; }
 
 extern "C" int dsvb_enc_picture_info(DSVB_ENC *e, int seq, DSVB_PICINFO *out, int cap)
 {
-    return copy_picture_info(e->info_valid, e->info, seq, out, cap);
+    return copy_records(e->info_valid, e->info, seq, out, cap);
+}
+
+extern "C" int dsvb_enc_picture_ssim(DSVB_ENC *e, int seq, DSVB_PICSSIM *out, int cap)
+{
+    return copy_records(e->ssim_valid, e->ssim, seq, out, cap);
 }
 
 extern "C" int dsvb_kernel_count(void) { return kt_count(); }
@@ -206,9 +199,10 @@ extern "C" int dsvb_encode(DSVB_ENC *e, int nseq, int nframes, const uint8_t *co
     const CodecGeom &g = e->eng->geom();
     const int L = e->lanes;
     int rc = 0;
-    const bool report = e->eng->picture_info;
-    e->info_valid = false;
+    const bool report = e->eng->picture_info, report_ssim = e->eng->picture_ssim;
+    e->info_valid = e->ssim_valid = false;
     e->info.assign(report ? (size_t) nseq : 0, std::vector<DSVB_PICINFO>());
+    e->ssim.assign(report_ssim ? (size_t) nseq : 0, std::vector<DSVB_PICSSIM>());
     std::vector<int> ids((size_t) L);
     std::vector<PicRef> src((size_t) L), next((size_t) L);
     std::vector<PktSink> sinks((size_t) L);
@@ -250,9 +244,12 @@ extern "C" int dsvb_encode(DSVB_ENC *e, int nseq, int nframes, const uint8_t *co
             }
             pictures(t, src);
             e->eng->step(n, ids.data(), src.data(), reinterpret_cast<DSV_BUF(*)[2]>(bufs.data()), nb.data(), sinks.data());
-            for (int k = 0; report && k < n; k++) {
-                if (e->eng->pic_info_ok[(size_t) k]) {
+            for (int k = 0; (report || report_ssim) && k < n; k++) {
+                if (e->eng->pic_info_ok[(size_t) k] && report) {
                     e->info[(size_t) (base + k)].push_back(e->eng->pic_info[(size_t) k]);
+                }
+                if (e->eng->pic_info_ok[(size_t) k] && report_ssim) {
+                    e->ssim[(size_t) (base + k)].push_back(e->eng->pic_ssim[(size_t) k]);
                 }
             }
         }
@@ -276,6 +273,7 @@ extern "C" int dsvb_encode(DSVB_ENC *e, int nseq, int nframes, const uint8_t *co
         }
     }
     e->info_valid = report && rc == 0;
+    e->ssim_valid = report_ssim && rc == 0;
     return rc;
     DSV_API_END(-100)
 }

@@ -3,6 +3,8 @@
  * share: the objects behind the opaque handles and the option-block helpers.
  */
 #pragma once
+#include <cstring>
+
 #include "dsv1_b200_batch.h"
 
 #include "dsv1_b200.h"
@@ -31,6 +33,8 @@ struct DSVB_ENC {
     /* picture report of the last encode call: records per sequence, valid when the report was on and the call succeeded */
     bool info_valid = false;
     std::vector<std::vector<DSVB_PICINFO>> info;
+    bool ssim_valid = false; /* SSIM report of the last encode call, the same way */
+    std::vector<std::vector<DSVB_PICSSIM>> ssim;
 };
 
 struct DSVB_DEC {
@@ -55,6 +59,17 @@ struct DecSegment {
     int frames;                /* out: pictures decoded */
 };
 int decode_segments(DSVB_DEC *d, int nseg, DecSegment *segs, int out_on_device);
-/* dsvb_enc_picture_info / dsvb_multi_picture_info */
-int copy_picture_info(bool valid, const std::vector<std::vector<DSVB_PICINFO>> &info, int seq, DSVB_PICINFO *out, int cap);
+/* dsvb_*_picture_info / dsvb_*_picture_ssim: the records of sequence seq, at most cap of them; their count, or -1 */
+template <typename R> int copy_records(bool valid, const std::vector<std::vector<R>> &recs, int seq, R *out, int cap)
+{
+    if (!valid || seq < 0 || seq >= (int) recs.size()) {
+        return -1;
+    }
+    const std::vector<R> &r = recs[(size_t) seq];
+    const int n = (int) r.size();
+    if (out && cap > 0) {
+        memcpy(out, r.data(), sizeof(R) * (size_t) (n < cap ? n : cap));
+    }
+    return n;
+}
 } // namespace dsv

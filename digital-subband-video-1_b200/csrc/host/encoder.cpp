@@ -13,6 +13,8 @@
  *            -> SBT inverse -> reconstruction + border (new references) || packets D2H   [sync]
  * There is no CPU implementation of those stages in this library.
  */
+#include <cmath>
+
 #include "dsv1_b200.h"
 
 #include "bits.h"
@@ -495,6 +497,8 @@ EncEngine::~EncEngine()
     cudaFreeHost(h_pk_);
     cudaFree(d_sse_);
     cudaFreeHost(h_sse_);
+    cudaFree(d_ssim_);
+    cudaFreeHost(h_ssim_);
     for (auto &e : ev_) {
         cudaEventDestroy(e);
     }
@@ -508,27 +512,34 @@ EncEngine::~EncEngine()
     cudaStreamDestroy(st_);
 }
 
-/* The picture report's buffers, made when a step first runs with it on (no step is in flight then: step() ends with a
- * stream synchronisation): the sums, the step arena and packet copy list grown by the SSE jobs, their zero item and
- * the sums' copy item, and for intra-only engines a reconstruction target per lane (their inverse would write in
- * place over the source). */
-void EncEngine::enable_picture_info()
+/* The per-picture reports' buffers, made when a step first runs with a report on whose buffers do not exist yet (no
+ * step is in flight then: step() ends with a stream synchronisation): per report the sums, the step arena and packet
+ * copy list grown by its jobs, its zero item and its sums' copy item; with the first report, for intra-only engines,
+ * a reconstruction target per lane (their inverse would write in place over the source). */
+void EncEngine::enable_reports(bool sse, bool ssim)
 {
     const size_t sums = (sizeof(unsigned long long) * 3 * (size_t) L_ + 15) & ~(size_t) 15;
-    const size_t arena = arena_.cap + (3 * sizeof(SseJob) + 16) * (size_t) L_ + sizeof(ZeroItem) + 64;
+    const size_t per_report = (3 * sizeof(SseJob) + 16) * (size_t) L_ + sizeof(ZeroItem) + 64;
+    const bool add_sse = sse && !d_sse_, add_ssim = ssim && !d_ssim_, first = !d_sse_ && !d_ssim_;
+    const size_t arena = arena_.cap + per_report * (size_t) ((add_sse ? 1 : 0) + (add_ssim ? 1 : 0));
     arena_.destroy();
     arena_.create(arena);
+    if (add_sse) {
+        CUDA_CHECK(cudaMalloc(&d_sse_, sums));
+        CUDA_CHECK(cudaMallocHost(&h_sse_, sums));
+    }
+    if (add_ssim) {
+        CUDA_CHECK(cudaMalloc(&d_ssim_, sums));
+        CUDA_CHECK(cudaMallocHost(&h_ssim_, sums));
+    }
     cudaFreeHost(h_pk_);
     h_pk_ = nullptr;
-    CUDA_CHECK(cudaMallocHost(&h_pk_, sizeof(CopyItem) * ((size_t) L_ + 1)));
-    CUDA_CHECK(cudaMalloc(&d_sse_, sums));
-    CUDA_CHECK(cudaMallocHost(&h_sse_, sums));
-    if (!inter_) {
+    CUDA_CHECK(cudaMallocHost(&h_pk_, sizeof(CopyItem) * ((size_t) L_ + (d_sse_ ? 1 : 0) + (d_ssim_ ? 1 : 0))));
+    if (!inter_ && first) {
         for (auto &l : lanes_) {
             devframe_alloc(&l.qrec, g_.w, g_.h, g_.subsamp);
         }
     }
-    pi_ready_ = true;
 }
 
 static bool packed_pic(const CodecGeom &g, const PicRef &r)
@@ -659,9 +670,10 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
     const bool timed = time_kernels;
     KtActivate kt_on(timed ? &ktimes : nullptr);
     ktimes.open(0);
-    const bool report = picture_info && !analyse;
-    if (report && !pi_ready_) {
-        enable_picture_info();
+    const bool sse_on = picture_info && !analyse, ssim_on = picture_ssim && !analyse;
+    const bool report = sse_on || ssim_on; /* a report measures the reconstruction: every picture gets one */
+    if ((sse_on && !d_sse_) || (ssim_on && !d_ssim_)) {
+        enable_reports(sse_on, ssim_on);
     }
     arena_.reset();
 
@@ -926,11 +938,12 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
     PlaneRef *ext = n_ref > 0 ? arena_.push_n<PlaneRef>((size_t) 3 * n_ref, &d_ext) : nullptr;
     int qi = 0;
     ZeroItem *d_zero;
-    ZeroItem *zero = arena_.push_n<ZeroItem>((size_t) 2 * n + (report ? 1 : 0), &d_zero);
+    ZeroItem *zero = arena_.push_n<ZeroItem>((size_t) 2 * n + (sse_on ? 1 : 0) + (ssim_on ? 1 : 0), &d_zero);
     int n_zero = 0;
     size_t max_zero = 0;
-    SseJob *d_sse_jobs = nullptr;
-    SseJob *sse_jobs = report ? arena_.push_n<SseJob>((size_t) 3 * n, &d_sse_jobs) : nullptr;
+    SseJob *d_sse_jobs = nullptr, *d_ssim_jobs = nullptr;
+    SseJob *sse_jobs = sse_on ? arena_.push_n<SseJob>((size_t) 3 * n, &d_sse_jobs) : nullptr;
+    SseJob *ssim_jobs = ssim_on ? arena_.push_n<SseJob>((size_t) 3 * n, &d_ssim_jobs) : nullptr;
     for (int k = 0; k < n; k++) {
         const int li = lane_ids[k];
         EncLane &l = lanes_[(size_t) li];
@@ -938,8 +951,12 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
         const DevFrame &fwd_in = isP ? l.xf : (inter_ ? l.pad[l.cur] : l.xf);
         /* P pictures: the inverse transform adds the prediction on its way out and writes the reconstruction */
         const DevFrame &inv_out = inter_ ? l.recon[l.cur] : (report ? l.qrec : l.xf);
-        if (report) { /* the ingested source against the reconstruction */
+        /* the ingested source against the reconstruction */
+        if (sse_on) {
             sse_fill_picture(&sse_jobs[3 * k], g, inter_ ? l.pad[l.cur] : l.xf, inv_out, d_sse_ + 3 * k);
+        }
+        if (ssim_on) {
+            sse_fill_picture(&ssim_jobs[3 * k], g, inter_ ? l.pad[l.cur] : l.xf, inv_out, d_ssim_ + 3 * k);
         }
         /* tile flags (sbt.cuh): the forward transform ORs into zeroed bytes */
         zero[n_zero].p = l.tflags;
@@ -976,11 +993,13 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
             qi++;
         }
     }
-    if (report) {
-        zero[n_zero].p = d_sse_;
-        zero[n_zero].bytes = (sizeof(unsigned long long) * 3 * (size_t) n + 15) & ~(size_t) 15;
-        max_zero = max_zero > zero[n_zero].bytes ? max_zero : zero[n_zero].bytes;
-        n_zero++;
+    for (unsigned long long *sums : {sse_on ? d_sse_ : nullptr, ssim_on ? d_ssim_ : nullptr}) {
+        if (sums) {
+            zero[n_zero].p = sums;
+            zero[n_zero].bytes = (sizeof(unsigned long long) * 3 * (size_t) n + 15) & ~(size_t) 15;
+            max_zero = max_zero > zero[n_zero].bytes ? max_zero : zero[n_zero].bytes;
+            n_zero++;
+        }
     }
     const SbtDims sdims = sbt_assign_tiles(sj, 3 * n);
     {
@@ -994,7 +1013,7 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
     stats.kernel_launches += 6;
     copy1_launch(h_frames_, d_hf, sizeof(HzFrame) * (size_t) n, st);
     CUDA_CHECK(cudaEventRecord(ev_sizes_, st));
-    /* the report also needs the reconstruction of pictures that are not references (intra-only engines) */
+    /* the reports also need the reconstruction of pictures that are not references (intra-only engines) */
     const int n_inv = report ? n : n_ref;
     if (n_inv) {
         /* closed loop: reconstruct exactly what the decoder will (dsv_encoder.c:525,662-674) */
@@ -1005,8 +1024,12 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
         extend_launch(d_ext, 3 * n_ref, g.w, g.h, st);
         stats.kernel_launches += 1;
     }
-    if (report) {
+    if (sse_on) {
         sse_launch(d_sse_jobs, 3 * n, g.h, st);
+        stats.kernel_launches += 1;
+    }
+    if (ssim_on) {
+        ssim_launch(d_ssim_jobs, 3 * n, g.w, g.h, st);
         stats.kernel_launches += 1;
     }
     CUDA_CHECK(cudaEventSynchronize(ev_sizes_)); /* packet sizes are known; reconstruction keeps running */
@@ -1082,23 +1105,35 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
         bufs[k][nb++] = outbuf;
         nbufs[k] = nb;
     }
-    if (report) { /* the sums leave with the packets */
-        pk[n_pk].dst = h_sse_;
-        pk[n_pk].src = d_sse_;
-        pk[n_pk].bytes = sizeof(unsigned long long) * 3 * (size_t) n;
-        max_pk = max_pk > pk[n_pk].bytes ? max_pk : pk[n_pk].bytes;
-        n_pk++;
+    for (int r = 0; r < 2; r++) { /* the reports' sums leave with the packets */
+        if (r == 0 ? sse_on : ssim_on) {
+            pk[n_pk].dst = r == 0 ? h_sse_ : h_ssim_;
+            pk[n_pk].src = r == 0 ? d_sse_ : d_ssim_;
+            pk[n_pk].bytes = sizeof(unsigned long long) * 3 * (size_t) n;
+            max_pk = max_pk > pk[n_pk].bytes ? max_pk : pk[n_pk].bytes;
+            n_pk++;
+        }
     }
     copy_launch(pk, n_pk, max_pk, st);
     CUDA_CHECK(cudaStreamSynchronize(st));
     ktimes.collect(0);
     stats.pictures += (unsigned) n;
     if (report) {
-        pic_info.assign((size_t) n, DSVB_PICINFO());
+        pic_info.assign(sse_on ? (size_t) n : 0, DSVB_PICINFO());
+        pic_ssim.assign(ssim_on ? (size_t) n : 0, DSVB_PICSSIM());
         pic_info_ok.assign((size_t) n, 0);
         for (int k = 0; k < n; k++) {
             const EncLane &l = lanes_[(size_t) lane_ids[k]];
             if (h_frames_[k].overflow) {
+                continue;
+            }
+            pic_info_ok[(size_t) k] = 1;
+            for (int p = 0; ssim_on && p < 3; p++) {
+                DSVB_PICSSIM &s = pic_ssim[(size_t) k];
+                s.windows[p] = ssim_windows(g.pw[p], g.ph[p]);
+                s.ssim[p] = s.windows[p] ? (double) (int64_t) h_ssim_[3 * k + p] / 4294967296.0 / (double) s.windows[p] : NAN;
+            }
+            if (!sse_on) {
                 continue;
             }
             DSVB_PICINFO &r = pic_info[(size_t) k];
@@ -1111,7 +1146,6 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
             r.forced_intra = plan ? plan[k].forced_intra : (inter_ && !l.has_ref && !l.gop_start);
             r.quant = l.quant;
             r.bytes = (int32_t) h_frames_[k].total_bytes;
-            pic_info_ok[(size_t) k] = 1;
         }
     }
     if (timed) {

@@ -66,6 +66,8 @@ size_t enc_packet_cap(const CodecGeom &g);
 void enc_fill_frame(HzFrame *f, uint8_t *pkt, unsigned cap, unsigned start_byte, int k);
 /* squared-error jobs of the three planes of a picture: out[p] receives plane p's sum */
 void sse_fill_picture(SseJob *j, const CodecGeom &g, const DevFrame &src, const DevFrame &rec, unsigned long long *out);
+/* SSIM windows of a pw x ph plane: (pw/4 - 1) * (ph/4 - 1), 0 when either factor is below 1 */
+int64_t ssim_windows(int pw, int ph);
 void dec_fill_plane(SbtJob *s, HzJob *h, HzCleanItem *c, const CodecGeom &g, int p, int isP, int quant, const DevFrame &cur,
                     int32_t *coef, int32_t *llx, uint8_t *tflags, const uint8_t *stable);
 /* a lane's decoder tile flags before its first picture: every tile at the plane's base value (hz_flag_base) */
@@ -312,11 +314,16 @@ public:
      * references.  Off: nothing of it runs or is allocated. */
     bool picture_info = false;
     std::vector<DSVB_PICINFO> pic_info;
-    std::vector<char> pic_info_ok;
+    /* SSIM report (dsvb_enc_set_picture_ssim), independent of picture_info: when on, every coding step also measures
+     * each plane's SSIM against the reconstruction and fills pic_ssim[k].  One more launch per step, plus the inverse
+     * transform as above.  Off: nothing of it runs or is allocated. */
+    bool picture_ssim = false;
+    std::vector<DSVB_PICSSIM> pic_ssim;
+    std::vector<char> pic_info_ok; /* with either report on: picture k of the last step has records (0: dropped) */
     int device = 0;
 
 private:
-    void enable_picture_info();
+    void enable_reports(bool sse, bool ssim);
     void alloc_lane(EncLane &l);
     void free_lane(EncLane &l);
     CodecGeom g_;
@@ -337,8 +344,9 @@ private:
     HzChunk *d_chunks_ = nullptr;
     HzFrame *d_frames_ = nullptr, *h_frames_ = nullptr;
     void *h_pk_ = nullptr; /* packet egress copy list (mapped pinned) */
-    bool pi_ready_ = false; /* the picture report's buffers exist */
-    unsigned long long *d_sse_ = nullptr, *h_sse_ = nullptr; /* 3 sums per lane; h_sse_ mapped pinned */
+    /* 3 sums per lane of each report, allocated when a step first runs with that report on; h_* mapped pinned */
+    unsigned long long *d_sse_ = nullptr, *h_sse_ = nullptr;
+    unsigned long long *d_ssim_ = nullptr, *h_ssim_ = nullptr;
     HostPool *pool_ = nullptr;
     uint8_t *d_in_all_[ENC_STAGE_SLOTS] = {}; /* packed-picture staging of all lanes, lane pitch in_pitch_ */
     size_t in_pitch_ = 0;

@@ -64,6 +64,7 @@ struct LongCtx {
     std::vector<int> chain_first;  /* first picture of every chain, plus nframes as the sentinel */
     std::vector<std::vector<uint8_t>> pkt; /* coded picture packets */
     std::vector<DSVB_PICINFO> info;         /* picture report, by picture index */
+    std::vector<DSVB_PICSSIM> ssim;         /* SSIM report, by picture index */
     int forced = 0;
     int err = 0;
 };
@@ -90,6 +91,7 @@ void ctx_init(LongCtx &c, const DSVB_ENC *e, int nframes, const uint8_t *yuv, in
     c.gop_start.assign(n, 0);
     c.pkt.resize(n);
     c.info.assign(e->eng->picture_info ? n : 0, DSVB_PICINFO());
+    c.ssim.assign(e->eng->picture_ssim ? n : 0, DSVB_PICSSIM());
 }
 
 /*
@@ -377,6 +379,9 @@ void long_code(DSVB_ENC *e, LongCtx &c, PicSource &ps, int k0, int k1)
             if (!c.info.empty()) {
                 c.info[(size_t) t] = eng->pic_info[(size_t) q];
             }
+            if (!c.ssim.empty()) {
+                c.ssim[(size_t) t] = eng->pic_ssim[(size_t) q];
+            }
         }
         /* now commit the lane -> chain assignment the prefetch was made for (a lane that takes a new chain forgets
          * its reference only after the last picture of its old chain has been coded) */
@@ -428,12 +433,12 @@ int long_gather(LongCtx &c, uint8_t *stream, long cap, long *len)
     return rc;
 }
 
-/* the picture report of a long encode (ctx_init sized it when the report was on): one sequence */
-void take_info(LongCtx &c, int rc, bool *valid, std::vector<std::vector<DSVB_PICINFO>> *info)
+/* a report of a long encode (ctx_init sized it when the report was on) as the records of one sequence */
+template <typename R> void take_records(std::vector<R> &recs, int rc, bool *valid, std::vector<std::vector<R>> *out)
 {
-    *valid = rc == 0 && !c.info.empty();
-    info->assign(1, std::vector<DSVB_PICINFO>());
-    (*info)[0].swap(c.info);
+    *valid = rc == 0 && !recs.empty();
+    out->assign(1, std::vector<R>());
+    (*out)[0].swap(recs);
 }
 
 void fill_info(const LongCtx &c, int *info)
@@ -478,8 +483,9 @@ extern "C" int dsvb_encode_long(DSVB_ENC *e, int nframes, const uint8_t *yuv, in
 {
     DSV_API_BEGIN
     use_device(e->device);
-    e->info_valid = false;
+    e->info_valid = e->ssim_valid = false;
     e->info.clear();
+    e->ssim.clear();
     if (nframes <= 0) {
         return -2;
     }
@@ -502,7 +508,8 @@ extern "C" int dsvb_encode_long(DSVB_ENC *e, int nframes, const uint8_t *yuv, in
     long_code(e, c, ps, 0, (int) c.chain_first.size() - 1);
     fill_info(c, info);
     const int rc = long_gather(c, stream, cap, len);
-    take_info(c, rc, &e->info_valid, &e->info);
+    take_records(c.info, rc, &e->info_valid, &e->info);
+    take_records(c.ssim, rc, &e->ssim_valid, &e->ssim);
     return rc;
     DSV_API_END(-100)
 }
@@ -584,9 +591,11 @@ struct DSVB_MULTI {
     std::vector<int> devices;
     std::vector<DSVB_ENC *> enc;
     std::vector<DSVB_DEC *> dec;
-    bool picture_info = false;
+    bool picture_info = false, picture_ssim = false;
     bool info_valid = false; /* picture report of the last encode call, as DSVB_ENC */
     std::vector<std::vector<DSVB_PICINFO>> info;
+    bool ssim_valid = false; /* SSIM report of the last encode call, as DSVB_ENC */
+    std::vector<std::vector<DSVB_PICSSIM>> ssim;
 };
 
 extern "C" DSVB_MULTI *dsvb_multi_create(const int *cfg, int lanes, int ndev, const int *devices)
@@ -658,6 +667,7 @@ bool multi_encoders(DSVB_MULTI *m)
         ok[(size_t) i] = m->enc[(size_t) i] != nullptr;
         if (ok[(size_t) i]) {
             m->enc[(size_t) i]->eng->picture_info = m->picture_info;
+            m->enc[(size_t) i]->eng->picture_ssim = m->picture_ssim;
         }
     });
     for (int v : ok) {
@@ -691,7 +701,22 @@ extern "C" void dsvb_multi_set_picture_info(DSVB_MULTI *m, int on)
 
 extern "C" int dsvb_multi_picture_info(DSVB_MULTI *m, int seq, DSVB_PICINFO *out, int cap)
 {
-    return copy_picture_info(m->info_valid, m->info, seq, out, cap);
+    return copy_records(m->info_valid, m->info, seq, out, cap);
+}
+
+extern "C" void dsvb_multi_set_picture_ssim(DSVB_MULTI *m, int on)
+{
+    m->picture_ssim = on != 0;
+    for (DSVB_ENC *e : m->enc) {
+        if (e) {
+            e->eng->picture_ssim = m->picture_ssim;
+        }
+    }
+}
+
+extern "C" int dsvb_multi_picture_ssim(DSVB_MULTI *m, int seq, DSVB_PICSSIM *out, int cap)
+{
+    return copy_records(m->ssim_valid, m->ssim, seq, out, cap);
 }
 
 /* whole sequences dealt to the GPUs in contiguous runs */
@@ -699,8 +724,9 @@ extern "C" int dsvb_multi_encode(DSVB_MULTI *m, int nseq, int nframes, const uin
                                  const long *caps, long *lens)
 {
     DSV_API_BEGIN
-    m->info_valid = false;
+    m->info_valid = m->ssim_valid = false;
     m->info.clear();
+    m->ssim.clear();
     if (!multi_encoders(m)) {
         return -100;
     }
@@ -715,16 +741,22 @@ extern "C" int dsvb_multi_encode(DSVB_MULTI *m, int nseq, int nframes, const uin
             return v;
         }
     }
-    if (m->picture_info) { /* device i coded sequences [s0, s1) as its sequences 0 .. s1 - s0 - 1 */
-        m->info.resize((size_t) nseq);
-        for (int i = 0; i < nd; i++) {
-            const int s0 = (int) ((long long) nseq * i / nd), s1 = (int) ((long long) nseq * (i + 1) / nd);
-            for (int s = s0; s < s1; s++) {
+    /* device i coded sequences [s0, s1) as its sequences 0 .. s1 - s0 - 1 */
+    m->info.resize(m->picture_info ? (size_t) nseq : 0);
+    m->ssim.resize(m->picture_ssim ? (size_t) nseq : 0);
+    for (int i = 0; i < nd; i++) {
+        const int s0 = (int) ((long long) nseq * i / nd), s1 = (int) ((long long) nseq * (i + 1) / nd);
+        for (int s = s0; s < s1; s++) {
+            if (m->picture_info) {
                 m->info[(size_t) s].swap(m->enc[(size_t) i]->info[(size_t) (s - s0)]);
             }
+            if (m->picture_ssim) {
+                m->ssim[(size_t) s].swap(m->enc[(size_t) i]->ssim[(size_t) (s - s0)]);
+            }
         }
-        m->info_valid = true;
     }
+    m->info_valid = m->picture_info;
+    m->ssim_valid = m->picture_ssim;
     return 0;
     DSV_API_END(-100)
 }
@@ -753,8 +785,9 @@ extern "C" int dsvb_multi_decode(DSVB_MULTI *m, int nseq, const uint8_t *const *
 extern "C" int dsvb_multi_encode_long(DSVB_MULTI *m, int nframes, const uint8_t *yuv, uint8_t *stream, long cap, long *len, int *info)
 {
     DSV_API_BEGIN
-    m->info_valid = false;
+    m->info_valid = m->ssim_valid = false;
     m->info.clear();
+    m->ssim.clear();
     if (!multi_encoders(m) || nframes <= 0) {
         return -100;
     }
@@ -762,6 +795,8 @@ extern "C" int dsvb_multi_encode_long(DSVB_MULTI *m, int nframes, const uint8_t 
         const int rc = dsvb_encode_long(m->enc[0], nframes, yuv, 0, stream, cap, len, info);
         m->info_valid = m->enc[0]->info_valid;
         m->info.swap(m->enc[0]->info);
+        m->ssim_valid = m->enc[0]->ssim_valid;
+        m->ssim.swap(m->enc[0]->ssim);
         return rc;
     }
     LongCtx c;
@@ -814,7 +849,8 @@ extern "C" int dsvb_multi_encode_long(DSVB_MULTI *m, int nframes, const uint8_t 
         info[3] = nd;
     }
     const int rc = long_gather(c, stream, cap, len);
-    take_info(c, rc, &m->info_valid, &m->info);
+    take_records(c.info, rc, &m->info_valid, &m->info);
+    take_records(c.ssim, rc, &m->ssim_valid, &m->ssim);
     return rc;
     DSV_API_END(-100)
 }

@@ -86,6 +86,11 @@ void sse_fill_picture(SseJob *j, const CodecGeom &g, const DevFrame &src, const 
     }
 }
 
+int64_t ssim_windows(int pw, int ph)
+{
+    return pw >= 8 && ph >= 8 ? (int64_t) (pw / 4 - 1) * (ph / 4 - 1) : 0;
+}
+
 void dec_fill_plane(SbtJob *s, HzJob *h, HzCleanItem *c, const CodecGeom &g, int p, int isP, int quant, const DevFrame &cur,
                     int32_t *coef, int32_t *llx, uint8_t *tflags, const uint8_t *stable)
 {

@@ -815,9 +815,9 @@ extern "C" int dsvk_inv_batch(int n, const int *geo, const DSVK_PIC *pics, const
     DSV_API_END(-100)
 }
 
-extern "C" int dsvk_sse_batch(int n, const int *geo, const uint8_t *src, const uint8_t *rec, const uint8_t *border_fill, uint64_t *sse_out)
+/* dsvk_sse_batch / dsvk_ssim_batch: n picture pairs placed in bordered device frames, one launch of the kernel */
+static int quality_batch(int n, const int *geo, const uint8_t *src, const uint8_t *rec, const uint8_t *border_fill, bool ssim, uint64_t *out)
 {
-    DSV_API_BEGIN
     if (n < 1) {
         return -1;
     }
@@ -825,7 +825,7 @@ extern "C" int dsvk_sse_batch(int n, const int *geo, const uint8_t *src, const u
     std::vector<SseJob> jobs((size_t) 3 * n);
     unsigned long long *d_out = dev_alloc<unsigned long long>((size_t) 3 * n);
     const uint8_t *s_at = src, *r_at = rec;
-    int max_h = 0;
+    int max_w = 0, max_h = 0;
     int rc = 0;
     for (int k = 0; k < n && rc == 0; k++) {
         if (geo[3 * k] < 16 || geo[3 * k + 1] < 16 || (geo[3 * k] & 1) || (geo[3 * k + 1] & 1)) {
@@ -843,14 +843,19 @@ extern "C" int dsvk_sse_batch(int n, const int *geo, const uint8_t *src, const u
         s_at += g.frame_bytes;
         r_at += g.frame_bytes;
         sse_fill_picture(&jobs[(size_t) 3 * k], g, fs[(size_t) k], fr[(size_t) k], d_out + 3 * k);
+        max_w = max_w > g.w ? max_w : g.w;
         max_h = max_h > g.h ? max_h : g.h;
     }
     if (rc == 0) {
         SseJob *d_jobs = dev_alloc<SseJob>(jobs.size(), false);
         CUDA_CHECK(cudaMemcpy(d_jobs, jobs.data(), sizeof(SseJob) * jobs.size(), cudaMemcpyHostToDevice));
-        sse_launch(d_jobs, 3 * n, max_h, 0);
+        if (ssim) {
+            ssim_launch(d_jobs, 3 * n, max_w, max_h, 0);
+        } else {
+            sse_launch(d_jobs, 3 * n, max_h, 0);
+        }
         CUDA_CHECK(cudaDeviceSynchronize());
-        CUDA_CHECK(cudaMemcpy(sse_out, d_out, sizeof(uint64_t) * 3 * n, cudaMemcpyDeviceToHost));
+        CUDA_CHECK(cudaMemcpy(out, d_out, sizeof(uint64_t) * 3 * n, cudaMemcpyDeviceToHost));
         cudaFree(d_jobs);
     }
     for (int k = 0; k < n; k++) {
@@ -858,6 +863,28 @@ extern "C" int dsvk_sse_batch(int n, const int *geo, const uint8_t *src, const u
         devframe_free(&fr[(size_t) k]);
     }
     cudaFree(d_out);
+    return rc;
+}
+
+extern "C" int dsvk_sse_batch(int n, const int *geo, const uint8_t *src, const uint8_t *rec, const uint8_t *border_fill, uint64_t *sse_out)
+{
+    DSV_API_BEGIN
+    return quality_batch(n, geo, src, rec, border_fill, false, sse_out);
+    DSV_API_END(-100)
+}
+
+extern "C" int dsvk_ssim_batch(int n, const int *geo, const uint8_t *src, const uint8_t *rec, const uint8_t *border_fill,
+                               int64_t *sum_out, int64_t *windows_out)
+{
+    DSV_API_BEGIN
+    const int rc = quality_batch(n, geo, src, rec, border_fill, true, reinterpret_cast<uint64_t *>(sum_out));
+    for (int k = 0; k < n && rc == 0; k++) {
+        CodecGeom g;
+        plan_geometry(&g, geo[3 * k], geo[3 * k + 1], geo[3 * k + 2]);
+        for (int p = 0; p < 3; p++) {
+            windows_out[3 * k + p] = ssim_windows(g.pw[p], g.ph[p]);
+        }
+    }
     return rc;
     DSV_API_END(-100)
 }

@@ -147,6 +147,34 @@ int dsvb_enc_picture_info(DSVB_ENC *e, int seq, DSVB_PICINFO *out, int cap);
 void dsvb_multi_set_picture_info(DSVB_MULTI *m, int on);
 int dsvb_multi_picture_info(DSVB_MULTI *m, int seq, DSVB_PICINFO *out, int cap);
 
+/*
+ * SSIM report of the encoders: the SSIM of every plane of every coded picture against the source, measured on the GPU
+ * on the same closed-loop reconstruction as the report above.  Independent of it: either can be on without the other.
+ * Off by default; while off the encoders do exactly what they do without it.  When on it costs one kernel per step,
+ * and pictures that are not references get the inverse transform they otherwise skip.  The streams do not change.
+ *   dsvb_enc_picture_ssim / dsvb_multi_picture_ssim: as dsvb_enc_picture_info / dsvb_multi_picture_info (records of
+ *   sequence `seq` of the last encode call in picture order, at most `cap` written, the count returned; -1 if the
+ *   SSIM report was off during that call, the call failed, or seq is out of range).
+ * Definition (x264 / ffmpeg, 8-bit), for a plane of pw x ph samples, source a, reconstruction b:
+ *   4x4 blocks: bw = pw / 4, bh = ph / 4 (the last pw % 4 columns and ph % 4 rows are not read);
+ *   windows: the 2x2 groups of blocks at block positions (i, j), 0 <= i < bw - 1, 0 <= j < bh - 1 (8x8 samples,
+ *   stride 4); per window, over its 64 samples in int64: s1 = sum a, s2 = sum b, ss = sum (a^2 + b^2), s12 = sum ab,
+ *   vars = 64 ss - s1^2 - s2^2, covar = 64 s12 - s1 s2,
+ *   ssim_w = (double) ((2 s1 s2 + 416) (2 covar + 235963)) / (double) ((s1^2 + s2^2 + 416) (vars + 235963))
+ *   (IEEE round to nearest); the plane's sum S = sum over windows of rint(ssim_w * 2^32) (ties to even), in int64,
+ *   and ssim = (double) S / 2^32 / windows.  The sum of integers makes the result independent of summation order,
+ *   lanes and devices.
+ * dB form: -10 * log10(1 - ssim) (infinite when ssim == 1).
+ */
+typedef struct DSVB_PICSSIM { /* 48 bytes, no padding */
+    double ssim[3];           /* mean SSIM over the plane's 8x8 windows (stride 4), Y U V; NaN when windows[p] == 0 */
+    int64_t windows[3];       /* (pw/4 - 1) * (ph/4 - 1), 0 when a plane has fewer than 8 samples in either direction */
+} DSVB_PICSSIM;
+void dsvb_enc_set_picture_ssim(DSVB_ENC *e, int on);
+int dsvb_enc_picture_ssim(DSVB_ENC *e, int seq, DSVB_PICSSIM *out, int cap);
+void dsvb_multi_set_picture_ssim(DSVB_MULTI *m, int on);
+int dsvb_multi_picture_ssim(DSVB_MULTI *m, int seq, DSVB_PICSSIM *out, int cap);
+
 /* pinned host memory for inputs / outputs of the calls above */
 void *dsvb_host_alloc(size_t bytes);
 void dsvb_host_free(void *p);

@@ -103,6 +103,11 @@ int dsvk_inv_batch(int n, const int *geo, const DSVK_PIC *pics, const int32_t *c
  * dsvk_inv_batch; src / rec hold n packed frames each.  Both are placed in bordered device frames whose border and
  * padding bytes are set to border_fill[0] (src) and border_fill[1] (rec).  sse_out: 3 sums per picture, Y U V. */
 int dsvk_sse_batch(int n, const int *geo, const uint8_t *src, const uint8_t *rec, const uint8_t *border_fill, uint64_t *sse_out);
+/* SSIM of n picture pairs in one launch, as the batch encoders' SSIM report measures it: geo / src / rec / border_fill
+ * as for dsvk_sse_batch.  sum_out: 3 per picture, Y U V = sum over the plane's windows of rint(ssim_w * 2^32) (the
+ * definition is at DSVB_PICSSIM, dsv1_b200_batch.h); windows_out: 3 per picture.  -1: a geometry is illegal. */
+int dsvk_ssim_batch(int n, const int *geo, const uint8_t *src, const uint8_t *rec, const uint8_t *border_fill,
+                    int64_t *sum_out, int64_t *windows_out);
 
 /* decoder lane: coefficient planes and tile flags carry over from one picture to the next */
 void *dsvk_dec_create(int w, int h, int subsamp, int blk_w, int blk_h);

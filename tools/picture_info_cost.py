@@ -1,4 +1,5 @@
-"""Cost of the encoders' per-picture report (dsvb_enc_set_picture_info) on the bench workload.
+"""Cost of the encoders' per-picture report (dsvb_enc_set_picture_info) or, with --report ssim, of the SSIM report
+(dsvb_enc_set_picture_ssim) on the bench workload.
 
 Configs (bench.py / BASELINE.json): 5 = 1920x1080 4:2:0 gop12, 64 lanes x 12 pictures, device-resident input made by
 dsvb_synth_device; 2 = the same with gop 0, where the report adds the whole inverse transform (intra-only pictures are
@@ -6,11 +7,12 @@ not references and are otherwise never reconstructed).
 
   1. Encode calls with the report off and on, alternating, `--reps` times each after one warm-up call of each, in one
      process; host clock around the calls (dsvb_encode returns when the streams are on the host).
-  2. A separate pass with live kernel timing: sse_kernel's device time per launch, against the time a copy of the same
-     bytes (2 per sample: source and reconstruction) takes at the device-to-device copy rate measured here.
+  2. A separate pass with live kernel timing: the report kernel's (sse_kernel / ssim_kernel) device time per launch,
+     against the time a copy of the same bytes (2 per sample: source and reconstruction) takes at the device-to-device
+     copy rate measured here.
 
 Prints the card's name and power limit (nvidia-smi, a read) and writes everything as JSON to --out.
-usage: python tools/picture_info_cost.py [--reps 6] [--out profiles/picture_info_cost.json]
+usage: python tools/picture_info_cost.py [--report sse|ssim] [--reps 6] [--out profiles/picture_info_cost.json]
 """
 import argparse
 import ctypes as C
@@ -23,8 +25,11 @@ import time
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
 import picinfo as PI  # noqa: E402  (the report's Python bindings, next to dsvlibs)
+import picssim as PS  # noqa: E402  (the SSIM report's)
 
 W, H, FMT, NFR, B = 1920, 1080, "420", 12, 64
+# report -> (switch, kernel)
+REPORTS = {"sse": (PI.set_picture_info, "sse_kernel"), "ssim": (PS.set_picture_ssim, "ssim_kernel")}
 
 
 def card():
@@ -53,7 +58,8 @@ def copy_peak_gbs(torch):
     return best
 
 
-def run_config(L, torch, gpu, gop, reps, peak):
+def run_config(L, torch, gpu, gop, reps, peak, report="sse"):
+    switch, kname = REPORTS[report]
     sub = L.SUBSAMP[FMT]
     fb = L.frame_bytes(W, H, sub)
     seq = fb * NFR
@@ -67,7 +73,7 @@ def run_config(L, torch, gpu, gop, reps, peak):
     sp = [h_streams.data_ptr() + s * cap for s in range(B)]
 
     def call(on):
-        PI.set_picture_info(enc, on)
+        switch(enc, on)
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         rc, lens = enc.encode_ptrs(yp, NFR, 1, sp, [cap] * B)
@@ -83,34 +89,39 @@ def run_config(L, torch, gpu, gop, reps, peak):
         for on in ((False, True) if r % 2 == 0 else (True, False)):
             ms[on].append(call(on)[0])
     # kernel time, in a pass of its own (timing events slow the steps)
-    PI.set_picture_info(enc, True)
+    switch(enc, True)
     enc.set_kernel_timing(True)
     enc.kernel_times(reset=True)
     enc.encode_ptrs(yp, NFR, 1, sp, [cap] * B)
     kt = enc.kernel_times(reset=True)
-    recs = PI.picture_info(enc, 0)
+    recs = PI.picture_info(enc, 0) if report == "sse" else PS.picture_ssim(enc, 0)
     enc.set_kernel_timing(False)
     enc.close()
-    sse = kt.get("sse_kernel", {"ms": 0.0, "launches": 0})
-    sse_ms = sse["ms"] / max(sse["launches"], 1)
+    kt_rep = kt.get(kname, {"ms": 0.0, "launches": 0})
+    k_ms = kt_rep["ms"] / max(kt_rep["launches"], 1)
     step_bytes = 2 * fb * B  # source + reconstruction, every sample of a step's pictures
     off, on = statistics.median(ms[False]), statistics.median(ms[True])
+    if report == "sse":
+        example = {"example_psnr_y_first_picture": float(PI.psnr(recs["sse"][0][0], recs["samples"][0][0]))}
+    else:
+        example = {"example_ssim_first_picture": [float(v) for v in recs["ssim"][0]]}
     return {
         "config": "%dx%d %s gop%d, %d lanes x %d pictures, device-resident input" % (W, H, FMT, gop, B, NFR),
         "call_ms_off": ms[False], "call_ms_on": ms[True],
         "median_call_ms_off": off, "median_call_ms_on": on,
         "median_step_ms_off": off / NFR, "median_step_ms_on": on / NFR,
         "delta_pct": 100.0 * (on - off) / off,
-        "sse_kernel_ms_per_launch": sse_ms, "sse_kernel_launches": sse["launches"],
-        "sse_bytes_per_launch": step_bytes,
-        "sse_share_of_copy_peak": (step_bytes / (peak * 1e9) * 1e3) / sse_ms if sse_ms > 0 else None,
+        kname + "_ms_per_launch": k_ms, kname + "_launches": kt_rep["launches"],
+        report + "_bytes_per_launch": step_bytes,
+        report + "_share_of_copy_peak": (step_bytes / (peak * 1e9) * 1e3) / k_ms if k_ms > 0 else None,
         "sbt_inv_kernel_ms": {k: v for k, v in kt.items() if k.startswith("sbt_inv")},
-        "example_psnr_y_first_picture": float(PI.psnr(recs["sse"][0][0], recs["samples"][0][0])),
+        **example,
     }
 
 
 def main():
     ap = argparse.ArgumentParser()
+    ap.add_argument("--report", choices=sorted(REPORTS), default="sse")
     ap.add_argument("--reps", type=int, default=6)
     ap.add_argument("--out", default=os.path.join("profiles", "picture_info_cost.json"))
     args = ap.parse_args()
@@ -122,13 +133,14 @@ def main():
     info = card()
     print("card: %s, power limit %s" % (info["name"], info["power_limit"]))
     peak = copy_peak_gbs(torch)
-    res = {"card": info, "copy_peak_GBps": peak, "reps": args.reps, "configs": {}}
+    kname = REPORTS[args.report][1]
+    res = {"card": info, "copy_peak_GBps": peak, "reps": args.reps, "report": args.report, "configs": {}}
     for name, gop in (("5", 12), ("2", 0)):
-        r = run_config(L, torch, gpu, gop, args.reps, peak)
+        r = run_config(L, torch, gpu, gop, args.reps, peak, args.report)
         res["configs"][name] = r
-        print("config %s: step %.3f -> %.3f ms (%+.2f %%), sse_kernel %.4f ms/launch (%.0f %% of the copy rate %.0f GB/s)" %
-              (name, r["median_step_ms_off"], r["median_step_ms_on"], r["delta_pct"], r["sse_kernel_ms_per_launch"],
-               100 * (r["sse_share_of_copy_peak"] or 0), peak))
+        print("config %s: step %.3f -> %.3f ms (%+.2f %%), %s %.4f ms/launch (%.0f %% of the copy rate %.0f GB/s)" %
+              (name, r["median_step_ms_off"], r["median_step_ms_on"], r["delta_pct"], kname, r[kname + "_ms_per_launch"],
+               100 * (r[args.report + "_share_of_copy_peak"] or 0), peak))
         torch.cuda.empty_cache()
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, "w") as f:
