@@ -482,10 +482,8 @@ void DecEngine::step(int n, const int *lane_ids, const PktRef *pkts, const OutRe
                 n_pack++;
             }
         }
-        if (isP) {
-            const MotionGeom mg = {g.w, g.h, g.hs, g.vs, g.blk_w, g.blk_h, g.nbh, g.nbv, 0};
-            bmc_fill_args(&ba[n_p++], mg, d_mv_ + (size_t) li * step_nblk, l.out[l.cur ^ 1], nullptr, cur, cur, 2);
-        }
+        const MotionGeom mg = {g.w, g.h, g.hs, g.vs, g.blk_w, g.blk_h, g.nbh, g.nbv, 0};
+        dec_bmc_fill(ba, &n_p, isP, mg, d_mv_, li, step_nblk, l.out[l.cur ^ 1], cur);
     }
     stats.host_ms += host_now_ms() - t_host0;
     if (n_sj == 0) {

@@ -342,12 +342,6 @@ static void rate_control_update(DSV_ENCODER *enc, int isP, unsigned pkt_len) /* 
 
 namespace dsv {
 
-struct LaneMisc { /* device/pinned per-lane scalars */
-    unsigned long long luma_sum;
-    int nintra;
-    int pad;
-};
-
 EncEngine::EncEngine(const DSV_META &md, int gop, int pyramid_levels, int lanes)
 {
     if (!meta_supported(md)) {
@@ -698,13 +692,13 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
         }
         uint8_t *stage_buf = prefetched ? l.d_in[pb] : l.d_in[l.in_sel];
         bool staged = false;
+        const uint8_t *packed[3];
         for (int p = 0; p < 3; p++) {
-            const uint8_t *packed;
             const size_t pbytes = (size_t) g.pw[p] * g.ph[p];
             if (src[k].on_device && src[k].stride[p] == g.pw[p]) {
-                packed = src[k].plane[p];
+                packed[p] = src[k].plane[p];
             } else if (prefetched) {
-                packed = stage_buf + g.plane_off[p];
+                packed[p] = stage_buf + g.plane_off[p];
             } else {
                 uint8_t *stage = stage_buf + g.plane_off[p];
                 CUDA_CHECK(cudaMemcpy2DAsync(stage, (size_t) g.pw[p], src[k].plane[p], (size_t) src[k].stride[p], (size_t) g.pw[p],
@@ -712,12 +706,11 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
                 if (!src[k].on_device) {
                     stats.h2d_bytes += pbytes;
                 }
-                packed = stage;
+                packed[p] = stage;
                 staged = true;
             }
-            ing[3 * k + p].src = packed;
-            ing[3 * k + p].dst = plane_ref(dst, p);
         }
+        ingest_fill_picture(&ing[3 * k], packed, dst);
         if (staged) {
             l.stage_src[l.in_sel] = nullptr;
             l.in_sel = (l.in_sel + 1) % ENC_STAGE_SLOTS;
@@ -757,8 +750,7 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
             Down2Item *dn = arena_.push_n<Down2Item>((size_t) n, &d_dn[lv]);
             for (int k = 0; k < n; k++) {
                 EncLane &l = lanes_[(size_t) lane_ids[k]];
-                dn[k].src = plane_ref(lv == 0 ? l.pad[l.cur] : l.pyr[l.cur][lv - 1], 0);
-                dn[k].dst = plane_ref(l.pyr[l.cur][lv], 0);
+                down2_fill_level(&dn[k], l.pad[l.cur], l.pyr[l.cur], lv);
             }
         }
         if (n_sum) {
@@ -767,9 +759,7 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
             for (int k = 0; k < n; k++) {
                 EncLane &l = lanes_[(size_t) lane_ids[k]];
                 if (analyse || l.enc->do_scd) {
-                    sm[q].src = plane_ref(l.pyr[l.cur][levels_ - 1], 0);
-                    sm[q].out = &d_misc[lane_ids[k]].luma_sum;
-                    q++;
+                    sum_fill_lane(&sm[q++], l.pyr[l.cur], levels_, d_misc, lane_ids[k]);
                 }
             }
         }
@@ -781,17 +771,8 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
                 if (!l.has_ref) {
                     continue;
                 }
-                DevFrame sf[DSV_MAX_PYRAMID_LEVELS + 1], rf[DSV_MAX_PYRAMID_LEVELS + 1];
-                sf[0] = l.pad[l.cur];
-                rf[0] = l.pad[l.cur ^ 1];
-                for (int lv = 0; lv < levels_; lv++) {
-                    sf[lv + 1] = l.pyr[l.cur][lv];
-                    rf[lv + 1] = l.pyr[l.cur ^ 1][lv];
-                }
-                for (int lv = 0; lv <= levels_; lv++) {
-                    hme_fill_args(&ha[(size_t) lv * n_search + q], mg, lv, sf, rf, l.d_mvf, l.d_aux, &d_misc[lane_ids[k]].nintra);
-                }
-                q++;
+                hme_fill_lane(ha, n_search, q++, mg, l.pad[l.cur], l.pyr[l.cur], l.pad[l.cur ^ 1], l.pyr[l.cur ^ 1], l.d_mvf, l.d_aux, d_misc,
+                              lane_ids[k]);
             }
         }
     }
@@ -806,7 +787,7 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
         for (int k = 0; k < n; k++) {
             EncLane &l = lanes_[(size_t) lane_ids[k]];
             if (l.has_ref) {
-                bmc_fill_args(&ba[q++], mg, l.d_mvf[0], l.recon[l.cur ^ 1], &l.pred, l.pad[l.cur], l.xf, 1);
+                enc_bmc_fill(&ba[q++], mg, l.d_mvf[0], l.recon[l.cur ^ 1], l.pred, l.pad[l.cur], l.xf);
             }
         }
     }

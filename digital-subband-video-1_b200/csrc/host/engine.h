@@ -73,6 +73,31 @@ void dec_fill_plane(SbtJob *s, HzJob *h, HzCleanItem *c, const CodecGeom &g, int
 /* a lane's decoder tile flags before its first picture: every tile at the plane's base value (hz_flag_base) */
 void dec_init_flags(uint8_t *d_tflags, const CodecGeom &g);
 
+/* per-lane scalars of the encoder's phase 1, one record per lane in a lane-major device array */
+struct LaneMisc {
+    unsigned long long luma_sum;
+    int nintra;
+    int pad;
+};
+/* motion descriptors of one picture of a step (plane_jobs.cpp), filled the same way by the encode / decode engines and
+ * by the kernel-level motion entry points (kernel_api.cu).  `pyr` is a lane's pyramid, levels 1.. of `top`. */
+/* ingest of the three packed planes src[p] into the bordered frame dst */
+void ingest_fill_picture(IngestItem *it, const uint8_t *const src[3], const DevFrame &dst);
+/* pyramid level lv + 1 from level lv (lv = 0: the ingested frame) */
+void down2_fill_level(Down2Item *it, const DevFrame &top, const DevFrame *pyr, int lv);
+/* luma sum of the smallest level into misc[lane] */
+void sum_fill_lane(SumItem *it, const DevFrame *pyr, int levels, LaneMisc *d_misc, int lane);
+/* the levels + 1 search rows of lane slot q: rows[level * n_search + q]; the intra count goes to misc[lane] */
+void hme_fill_lane(HmeArgs *rows, int n_search, int q, const MotionGeom &mg, const DevFrame &src, const DevFrame *src_pyr,
+                   const DevFrame &ref, const DevFrame *ref_pyr, DevMV *const *mvf, int2 *aux, LaneMisc *d_misc, int lane);
+/* encoder: prediction from the previous reconstruction into pred, residual of the ingested source into resid */
+void enc_bmc_fill(BmcArgs *a, const MotionGeom &mg, const DevMV *mv, const DevFrame &recon_ref, const DevFrame &pred,
+                  const DevFrame &src, const DevFrame &resid);
+/* decoder: lane li's compensation, appended to list[*n_p] when the picture is P: in place on cur, no prediction kept;
+ * the lane's vectors are at d_mv + li * nblk */
+void dec_bmc_fill(BmcArgs *list, int *n_p, int isP, const MotionGeom &mg, const DevMV *d_mv, int li, int nblk, const DevFrame &ref,
+                  const DevFrame &cur);
+
 /* where one input / output picture lives */
 struct PicRef {
     const uint8_t *plane[3];

@@ -130,4 +130,53 @@ void dec_init_flags(uint8_t *d_tflags, const CodecGeom &g)
     }
 }
 
+void ingest_fill_picture(IngestItem *it, const uint8_t *const src[3], const DevFrame &dst)
+{
+    for (int p = 0; p < 3; p++) {
+        it[p].src = src[p];
+        it[p].dst = plane_ref(dst, p);
+    }
+}
+
+void down2_fill_level(Down2Item *it, const DevFrame &top, const DevFrame *pyr, int lv)
+{
+    it->src = plane_ref(lv == 0 ? top : pyr[lv - 1], 0);
+    it->dst = plane_ref(pyr[lv], 0);
+}
+
+void sum_fill_lane(SumItem *it, const DevFrame *pyr, int levels, LaneMisc *d_misc, int lane)
+{
+    it->src = plane_ref(pyr[levels - 1], 0);
+    it->out = &d_misc[lane].luma_sum;
+}
+
+void hme_fill_lane(HmeArgs *rows, int n_search, int q, const MotionGeom &mg, const DevFrame &src, const DevFrame *src_pyr,
+                   const DevFrame &ref, const DevFrame *ref_pyr, DevMV *const *mvf, int2 *aux, LaneMisc *d_misc, int lane)
+{
+    DevFrame sf[DSV_MAX_PYRAMID_LEVELS + 1], rf[DSV_MAX_PYRAMID_LEVELS + 1];
+    sf[0] = src;
+    rf[0] = ref;
+    for (int lv = 0; lv < mg.levels; lv++) {
+        sf[lv + 1] = src_pyr[lv];
+        rf[lv + 1] = ref_pyr[lv];
+    }
+    for (int lv = 0; lv <= mg.levels; lv++) {
+        hme_fill_args(&rows[(size_t) lv * n_search + q], mg, lv, sf, rf, mvf, aux, &d_misc[lane].nintra);
+    }
+}
+
+void enc_bmc_fill(BmcArgs *a, const MotionGeom &mg, const DevMV *mv, const DevFrame &recon_ref, const DevFrame &pred,
+                  const DevFrame &src, const DevFrame &resid)
+{
+    bmc_fill_args(a, mg, mv, recon_ref, &pred, src, resid, 1);
+}
+
+void dec_bmc_fill(BmcArgs *list, int *n_p, int isP, const MotionGeom &mg, const DevMV *d_mv, int li, int nblk, const DevFrame &ref,
+                  const DevFrame &cur)
+{
+    if (isP) {
+        bmc_fill_args(&list[(*n_p)++], mg, d_mv + (size_t) li * nblk, ref, nullptr, cur, cur, 2);
+    }
+}
+
 } // namespace dsv

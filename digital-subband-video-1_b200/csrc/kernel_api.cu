@@ -993,3 +993,301 @@ extern "C" int dsvk_dec_run(void *handle, const DSVK_PIC *pic, const uint8_t *pl
     return nplanes;
     DSV_API_END(-100)
 }
+
+/* ---- batch entry points: the motion kernels configured as the engines launch them --------------------------------- */
+
+/* one lane of EncEngine's phase 1 (encoder.cpp alloc_lane): ingested frames and pyramids alternate with the picture
+ * parity (cur), so a lane's search reference is its previous call's ingested frame */
+struct DsvkMeLane {
+    DevFrame pad[2], recon[2], pyr[2][DSV_MAX_PYRAMID_LEVELS], xf, pred;
+    DevMV *d_mvf[DSV_MAX_PYRAMID_LEVELS + 1] = {};
+    int2 *d_aux = nullptr;
+    uint8_t *d_in = nullptr; /* staging buffer of host pictures */
+    int cur = 0, have_ref = 0;
+};
+
+struct DsvkMe {
+    CodecGeom g;
+    MotionGeom mg;
+    int levels, max_pics;
+    std::vector<DsvkMeLane> lanes;
+    DevMV *d_mv0 = nullptr, *h_mv0 = nullptr; /* level-0 fields of all lanes, lane-major (EncEngine::d_mv0_ / h_mv0_) */
+    LaneMisc *d_misc = nullptr;
+    StepArena arena;
+};
+
+#define DSVK_STAGE_SLACK 256 /* bytes past a staged picture: host pictures may be staged at offsets 0..255 */
+
+extern "C" void *dsvk_me_create(int w, int h, int subsamp, int blk_w, int blk_h, int levels, int max_pics)
+{
+    DSV_API_BEGIN
+    if (w < 16 || h < 16 || (w & 1) || (h & 1) || levels < 1 || levels > DSV_MAX_PYRAMID_LEVELS || max_pics < 1 || blk_w < 1 || blk_h < 1) {
+        return nullptr;
+    }
+    DsvkMe *m = new DsvkMe;
+    plan_geometry(&m->g, w, h, subsamp);
+    plan_blocks(&m->g, blk_w, blk_h);
+    const CodecGeom &g = m->g;
+    m->mg = {g.w, g.h, g.hs, g.vs, g.blk_w, g.blk_h, g.nbh, g.nbv, levels};
+    m->levels = levels;
+    m->max_pics = max_pics;
+    m->d_mv0 = dev_alloc<DevMV>((size_t) g.nblk * max_pics);
+    CUDA_CHECK(cudaMallocHost(&m->h_mv0, sizeof(DevMV) * (size_t) g.nblk * max_pics));
+    memset(m->h_mv0, 0, sizeof(DevMV) * (size_t) g.nblk * max_pics);
+    m->d_misc = dev_alloc<LaneMisc>((size_t) max_pics);
+    m->arena.create(((size_t) 3 * sizeof(IngestItem) + (size_t) levels * sizeof(Down2Item) + sizeof(SumItem) +
+                     (size_t) (levels + 1) * sizeof(HmeArgs) + sizeof(BmcArgs) + 3 * sizeof(PlaneRef) + 256) * max_pics + 4096);
+    m->lanes.resize((size_t) max_pics);
+    for (int i = 0; i < max_pics; i++) {
+        DsvkMeLane &l = m->lanes[(size_t) i];
+        devframe_alloc(&l.xf, w, h, subsamp);
+        devframe_alloc(&l.pred, w, h, subsamp);
+        for (int b = 0; b < 2; b++) {
+            devframe_alloc(&l.pad[b], w, h, subsamp);
+            devframe_alloc(&l.recon[b], w, h, subsamp);
+            for (int k = 0; k < levels; k++) {
+                devframe_alloc(&l.pyr[b][k], ceil_shift(w, k + 1), ceil_shift(h, k + 1), subsamp);
+            }
+        }
+        l.d_mvf[0] = m->d_mv0 + (size_t) i * g.nblk;
+        for (int k = 1; k <= levels; k++) {
+            l.d_mvf[k] = dev_alloc<DevMV>((size_t) g.nblk);
+        }
+        l.d_aux = dev_alloc<int2>((size_t) g.nblk);
+        l.d_in = dev_alloc<uint8_t>(g.frame_bytes + DSVK_STAGE_SLACK);
+    }
+    return m;
+    DSV_API_END(nullptr)
+}
+
+extern "C" void dsvk_me_destroy(void *handle)
+{
+    DsvkMe *m = static_cast<DsvkMe *>(handle);
+    if (!m) {
+        return;
+    }
+    for (auto &l : m->lanes) {
+        devframe_free(&l.xf);
+        devframe_free(&l.pred);
+        for (int b = 0; b < 2; b++) {
+            devframe_free(&l.pad[b]);
+            devframe_free(&l.recon[b]);
+            for (int k = 0; k < m->levels; k++) {
+                devframe_free(&l.pyr[b][k]);
+            }
+        }
+        for (int k = 1; k <= m->levels; k++) {
+            cudaFree(l.d_mvf[k]);
+        }
+        cudaFree(l.d_aux);
+        cudaFree(l.d_in);
+    }
+    cudaFree(m->d_mv0);
+    cudaFreeHost(m->h_mv0);
+    cudaFree(m->d_misc);
+    m->arena.destroy();
+    delete m;
+}
+
+extern "C" long dsvk_me_frame_bytes(void *handle, int level)
+{
+    const DsvkMe *m = static_cast<const DsvkMe *>(handle);
+    if (level < 0 || level > m->levels) {
+        return -1;
+    }
+    const DsvkMeLane &l = m->lanes[0];
+    return (long) (level == 0 ? l.pad[0].bytes : l.pyr[0][level - 1].bytes);
+}
+
+/* phase 1 of EncEngine::step (encoder.cpp) and its motion compensation on pictures 0..n-1 in lanes 0..n-1 */
+extern "C" int dsvk_me_run(void *handle, int n, const DSVK_ME_PIC *pics, const void *mvs, uint8_t *frames_out, int64_t *misc_out,
+                           void *mv_out, uint8_t *pred_out, uint8_t *resid_out)
+{
+    DSV_API_BEGIN
+    DsvkMe *m = static_cast<DsvkMe *>(handle);
+    const CodecGeom &g = m->g;
+    const MotionGeom &mg = m->mg;
+    const int levels = m->levels;
+    const bool code = mvs != nullptr;
+    if (n < 1 || n > m->max_pics) {
+        return -1;
+    }
+    int n_search = 0, n_sum = 0;
+    for (int k = 0; k < n; k++) {
+        if ((pics[k].has_ref && !m->lanes[(size_t) k].have_ref) || pics[k].stage_offset >= DSVK_STAGE_SLACK || !pics[k].src) {
+            return -1;
+        }
+        n_search += pics[k].has_ref != 0;
+        n_sum += pics[k].do_sum != 0;
+    }
+    StepArena &ar = m->arena;
+    ar.reset();
+    IngestItem *d_ing;
+    IngestItem *ing = ar.push_n<IngestItem>((size_t) 3 * n, &d_ing);
+    for (int k = 0; k < n; k++) {
+        DsvkMeLane &l = m->lanes[(size_t) k];
+        const uint8_t *base = pics[k].src;
+        if (!pics[k].src_on_device) {
+            uint8_t *stage = l.d_in + pics[k].stage_offset;
+            CUDA_CHECK(cudaMemcpy(stage, pics[k].src, g.frame_bytes, cudaMemcpyHostToDevice));
+            base = stage;
+        }
+        const uint8_t *packed[3] = {base + g.plane_off[0], base + g.plane_off[1], base + g.plane_off[2]};
+        ingest_fill_picture(&ing[3 * k], packed, l.pad[l.cur]);
+    }
+    Down2Item *d_dn[DSV_MAX_PYRAMID_LEVELS] = {};
+    SumItem *d_sum = nullptr;
+    HmeArgs *d_hme = nullptr;
+    if (!code) {
+        for (int lv = 0; lv < levels; lv++) {
+            Down2Item *dn = ar.push_n<Down2Item>((size_t) n, &d_dn[lv]);
+            for (int k = 0; k < n; k++) {
+                DsvkMeLane &l = m->lanes[(size_t) k];
+                down2_fill_level(&dn[k], l.pad[l.cur], l.pyr[l.cur], lv);
+            }
+        }
+        if (n_sum) {
+            SumItem *sm = ar.push_n<SumItem>((size_t) n_sum, &d_sum);
+            for (int k = 0, q = 0; k < n; k++) {
+                if (pics[k].do_sum) {
+                    sum_fill_lane(&sm[q++], m->lanes[(size_t) k].pyr[m->lanes[(size_t) k].cur], levels, m->d_misc, k);
+                }
+            }
+        }
+        if (n_search) {
+            HmeArgs *ha = ar.push_n<HmeArgs>((size_t) (levels + 1) * n_search, &d_hme);
+            for (int k = 0, q = 0; k < n; k++) {
+                DsvkMeLane &l = m->lanes[(size_t) k];
+                if (pics[k].has_ref) {
+                    hme_fill_lane(ha, n_search, q++, mg, l.pad[l.cur], l.pyr[l.cur], l.pad[l.cur ^ 1], l.pyr[l.cur ^ 1], l.d_mvf, l.d_aux,
+                                  m->d_misc, k);
+                }
+            }
+        }
+    }
+    BmcArgs *d_bmc = nullptr;
+    if (n_search) {
+        BmcArgs *ba = ar.push_n<BmcArgs>((size_t) n_search, &d_bmc);
+        for (int k = 0, q = 0; k < n; k++) {
+            DsvkMeLane &l = m->lanes[(size_t) k];
+            if (pics[k].has_ref) {
+                enc_bmc_fill(&ba[q++], mg, l.d_mvf[0], l.recon[l.cur ^ 1], l.pred, l.pad[l.cur], l.xf);
+            }
+        }
+    }
+    ZeroItem *d_zmisc;
+    ZeroItem *zmisc = ar.push_n<ZeroItem>(1, &d_zmisc);
+    zmisc->p = m->d_misc;
+    zmisc->bytes = sizeof(LaneMisc) * (size_t) m->max_pics;
+    PlaneRef *d_ext;
+    PlaneRef *ext = ar.push_n<PlaneRef>((size_t) 3 * n, &d_ext);
+    int n_ext = 0;
+    for (int k = 0; k < n; k++) {
+        if (pics[k].recon) {
+            for (int p = 0; p < 3; p++) {
+                ext[n_ext++] = plane_ref(m->lanes[(size_t) k].recon[m->lanes[(size_t) k].cur], p);
+            }
+        }
+    }
+    ar.upload(0);
+    /* the launch sequence of EncEngine::step: search pass, or (code pass) the caller's vectors and the compensation */
+    ingest_launch(d_ing, 3 * n, g.w, g.h, 0);
+    if (code) {
+        if (n_search) {
+            for (int k = 0; k < n; k++) {
+                if (pics[k].has_ref) {
+                    memcpy(m->h_mv0 + (size_t) k * g.nblk, static_cast<const DevMV *>(mvs) + (size_t) k * g.nblk, sizeof(DevMV) * (size_t) g.nblk);
+                }
+            }
+            copy1_launch(m->d_mv0, m->h_mv0, sizeof(DevMV) * (size_t) g.nblk * m->max_pics, 0);
+            bmc_launch(d_bmc, n_search, mg, 0);
+        }
+    } else {
+        for (int lv = 0; lv < levels; lv++) {
+            down2_launch(d_dn[lv], n, ceil_shift(g.w, lv + 1), ceil_shift(g.h, lv + 1), 0);
+        }
+        if (n_sum || n_search) {
+            zero_launch(d_zmisc, 1, zmisc->bytes, 0);
+        }
+        if (n_sum) {
+            sum_launch(d_sum, n_sum, ceil_shift(g.h, levels), 0);
+        }
+        if (n_search) {
+            hme_launch(d_hme, n_search, mg, 0);
+            bmc_launch(d_bmc, n_search, mg, 0);
+        }
+    }
+    CUDA_CHECK(cudaDeviceSynchronize());
+    /* phase 3's new reference: the caller's reconstruction, bordered */
+    for (int k = 0; k < n; k++) {
+        if (pics[k].recon) {
+            upload_packed(m->lanes[(size_t) k].recon[m->lanes[(size_t) k].cur], pics[k].recon);
+        }
+    }
+    if (n_ext) {
+        extend_launch(d_ext, n_ext, g.w, g.h, 0);
+    }
+    CUDA_CHECK(cudaDeviceSynchronize());
+    std::vector<LaneMisc> misc((size_t) n);
+    CUDA_CHECK(cudaMemcpy(misc.data(), m->d_misc, sizeof(LaneMisc) * (size_t) n, cudaMemcpyDeviceToHost));
+    CUDA_CHECK(cudaMemcpy(mv_out, m->d_mv0, sizeof(DevMV) * (size_t) g.nblk * n, cudaMemcpyDeviceToHost));
+    uint8_t *f_at = frames_out;
+    for (int k = 0; k < n; k++) {
+        DsvkMeLane &l = m->lanes[(size_t) k];
+        misc_out[2 * k] = (int64_t) misc[(size_t) k].luma_sum;
+        misc_out[2 * k + 1] = misc[(size_t) k].nintra;
+        CUDA_CHECK(cudaMemcpy(f_at, l.pad[l.cur].alloc, l.pad[l.cur].bytes, cudaMemcpyDeviceToHost));
+        f_at += l.pad[l.cur].bytes;
+        for (int lv = 0; lv < levels; lv++) {
+            CUDA_CHECK(cudaMemcpy(f_at, l.pyr[l.cur][lv].alloc, l.pyr[l.cur][lv].bytes, cudaMemcpyDeviceToHost));
+            f_at += l.pyr[l.cur][lv].bytes;
+        }
+        download_frame(l.pred, pred_out + g.frame_bytes * k);
+        download_frame(l.xf, resid_out + g.frame_bytes * k);
+        l.have_ref = 1;
+        l.cur ^= 1;
+    }
+    return 0;
+    DSV_API_END(-100)
+}
+
+/* the compensation of DecEngine::step (decoder.cpp) on n lanes: resid[k] is lane k's inverse-transform output, ref[k] its
+ * previous picture (bordered as the decoder's step leaves it); only the P lanes are in the launch's list */
+extern "C" int dsvk_add_pred_batch(int w, int h, int subsamp, int blk_w, int blk_h, int n, const int *isP, const void *mvs,
+                                   const uint8_t *resid, const uint8_t *ref, uint8_t *out)
+{
+    DSV_API_BEGIN
+    if (w < 16 || h < 16 || (w & 1) || (h & 1) || n < 1 || blk_w < 1 || blk_h < 1) {
+        return -1;
+    }
+    CodecGeom g;
+    plan_geometry(&g, w, h, subsamp);
+    plan_blocks(&g, blk_w, blk_h);
+    const MotionGeom mg = {g.w, g.h, g.hs, g.vs, g.blk_w, g.blk_h, g.nbh, g.nbv, 0};
+    std::vector<DevFrame> cur((size_t) n), prev((size_t) n);
+    DevMV *d_mv = dev_alloc<DevMV>((size_t) g.nblk * n, false);
+    CUDA_CHECK(cudaMemcpy(d_mv, mvs, sizeof(DevMV) * (size_t) g.nblk * n, cudaMemcpyHostToDevice));
+    std::vector<BmcArgs> ba((size_t) n);
+    int n_p = 0;
+    for (int k = 0; k < n; k++) {
+        devframe_alloc(&cur[(size_t) k], w, h, subsamp);
+        devframe_alloc(&prev[(size_t) k], w, h, subsamp);
+        upload_packed(cur[(size_t) k], resid + g.frame_bytes * k);
+        upload_packed(prev[(size_t) k], ref + g.frame_bytes * k);
+        frame_extend_launch(prev[(size_t) k], 3, 0);
+        dec_bmc_fill(ba.data(), &n_p, isP[k] != 0, mg, d_mv, k, g.nblk, prev[(size_t) k], cur[(size_t) k]);
+    }
+    BmcArgs *d_ba = dev_alloc<BmcArgs>((size_t) n, false);
+    CUDA_CHECK(cudaMemcpy(d_ba, ba.data(), sizeof(BmcArgs) * (size_t) n_p, cudaMemcpyHostToDevice));
+    bmc_launch(d_ba, n_p, mg, 0);
+    CUDA_CHECK(cudaDeviceSynchronize());
+    for (int k = 0; k < n; k++) {
+        download_frame(cur[(size_t) k], out + g.frame_bytes * k);
+        devframe_free(&cur[(size_t) k]);
+        devframe_free(&prev[(size_t) k]);
+    }
+    cudaFree(d_ba);
+    cudaFree(d_mv);
+    return 0;
+    DSV_API_END(-100)
+}

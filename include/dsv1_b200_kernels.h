@@ -116,6 +116,38 @@ void dsvk_dec_destroy(void *dec);
  * back.  Returns the number of planes decoded; coef_out / tflags_out receive the lane's planes and flags. */
 int dsvk_dec_run(void *dec, const DSVK_PIC *pic, const uint8_t *planes, int len, int32_t *coef_out, uint8_t *tflags_out);
 
+/* ---- batch entry points: the motion kernels configured as the engines launch them ----------------------------------
+ * The encoder's phase 1 (ingest with border, luma pyramid, luma sum, hierarchical search) and its motion compensation,
+ * and the decoder's compensation, with the engines' own descriptor filling and launch order over n lanes.  Frames are
+ * packed planar as above; motion fields are nbh * nbv DSV_MV records (12 bytes) per lane, lanes back to back. */
+typedef struct DSVK_ME_PIC {
+    const uint8_t *src;    /* the packed picture, at any byte address */
+    int src_on_device;     /* 1: src is device memory, ingested where it lies; 0: host memory, copied first */
+    unsigned stage_offset; /* host src: byte offset (0..255) in the lane's staging buffer it is copied to */
+    int has_ref;           /* search against the lane's previous picture, then compensate from its reconstruction */
+    int do_sum;            /* luma sum of the smallest pyramid level (scene-change detection) */
+    const uint8_t *recon;  /* NULL, or this picture's packed reconstruction: stored and bordered as the encoder's
+                              phase 3 stores it, it is the reference of the lane's next compensation */
+} DSVK_ME_PIC;
+
+/* lanes for up to max_pics pictures of one format and block grid, with `levels` (1..5) pyramid levels; each lane keeps
+ * its ingested frames, pyramids and reconstructions in two buffers that alternate from call to call */
+void *dsvk_me_create(int w, int h, int subsamp, int blk_w, int blk_h, int levels, int max_pics);
+void dsvk_me_destroy(void *me);
+/* bytes of a lane's device allocation of pyramid level `level` (0: the ingested frame), guard bands included */
+long dsvk_me_frame_bytes(void *me, int level);
+/* pictures 0..n-1 on lanes 0..n-1.  mvs NULL: ingest -> pyramid -> zero -> luma sum -> search -> compensation; mvs =
+ * n fields (the long encode's code pass): ingest, then the compensation with those vectors.  Out, per picture k:
+ * frames_out = the whole allocation of the ingested frame, then of pyramid levels 1..levels (dsvk_me_frame_bytes);
+ * misc_out[2k], [2k+1] = the lane's luma sum and intra-block count; mv_out = the level-0 field; pred_out / resid_out
+ * = prediction and residual (has_ref pictures).  -1: bad arguments, or a has_ref picture on a lane without a picture. */
+int dsvk_me_run(void *me, int n, const DSVK_ME_PIC *pics, const void *mvs, uint8_t *frames_out, int64_t *misc_out, void *mv_out,
+                uint8_t *pred_out, uint8_t *resid_out);
+/* the decoder's compensation of n lanes in one launch: out[k] = resid[k] + prediction from ref[k] - 128 with lane k's
+ * field (mvs + k * nbh * nbv) where isP[k], resid[k] unchanged otherwise */
+int dsvk_add_pred_batch(int w, int h, int subsamp, int blk_w, int blk_h, int n, const int *isP, const void *mvs, const uint8_t *resid,
+                        const uint8_t *ref, uint8_t *out);
+
 #ifdef __cplusplus
 }
 #endif
