@@ -84,6 +84,31 @@ static bool host_packed(const CodecGeom &g, const OutRef &r)
            r.plane[1] == r.plane[0] + g.plane_off[1] && r.plane[2] == r.plane[0] + g.plane_off[2];
 }
 
+/* dsv_decoder.c:383-413 */
+int parse_plane_dir(const uint8_t *pkt, unsigned len, unsigned at, const CodecGeom &g, const uint8_t *d_pkt, HzPlaneData pd[3])
+{
+    BitReader br(pkt, len);
+    br.skip_bytes(at);
+    int n = 0;
+    for (; n < 3; n++) {
+        const int plen = (int) br.get_bits(32);
+        const int framesz = g.cw[n] * g.ch[n] * (int) sizeof(int32_t);
+        if (plen <= 0 || plen > framesz * 2) {
+            DSV_ERROR(("plane length was strange: %d", plen));
+            break;
+        }
+        const unsigned start = br.byte_pos();
+        if (start >= len) {
+            DSV_ERROR(("plane starts past the end of the packet"));
+            break;
+        }
+        hzdec_parse_head(pkt + start, len - start, (unsigned) plen, &pd[n]);
+        pd[n].body = d_pkt + start;
+        br.skip_bytes((unsigned) plen);
+    }
+    return n;
+}
+
 DecEngine::DecEngine(const DSV_META &md, int lanes)
 {
     CUDA_CHECK(cudaGetDevice(&device));
@@ -127,21 +152,7 @@ DecEngine::DecEngine(const DSV_META &md, int lanes)
     CUDA_CHECK(cudaMalloc(&d_out_all_[1], out_pitch_ * L_ + 256));
     lanes_.resize((size_t) L_);
     for (auto &l : lanes_) {
-        /* coefficient planes are kept all-zero between pictures by the flag-guided clean-up (hzdec_clean_kernel) */
-        CUDA_CHECK(cudaMalloc(&l.coef, g.coef_total * sizeof(int32_t)));
-        CUDA_CHECK(cudaMemset(l.coef, 0, g.coef_total * sizeof(int32_t)));
-        CUDA_CHECK(cudaMalloc(&l.tflags, (size_t) g.total_tiles + 16));
-        dec_init_flags(l.tflags, g);
-        for (int p = 0; p < 3; p++) {
-            CUDA_CHECK(cudaMalloc(&l.llx[p], sbt_llx_elems(g.cw[p], g.ch[p]) * sizeof(int32_t)));
-            HzDecPlan pl;
-            hzdec_plan(&pl, g.cw[p], g.ch[p]);
-            hzdec_plane_alloc(&l.hz[p], pl);
-        }
-        devframe_alloc(&l.out[0], g.w, g.h, g.subsamp);
-        devframe_alloc(&l.out[1], g.w, g.h, g.subsamp);
-        /* packets are staged lazily: most are far smaller than the format's upper bound */
-        l.d_pkt = nullptr;
+        dec_lane_alloc(l, g);
     }
 }
 
@@ -150,18 +161,7 @@ DecEngine::~DecEngine()
     cudaStreamSynchronize(st_);
     cudaStreamSynchronize(st_copy_);
     for (auto &l : lanes_) {
-        cudaFree(l.coef);
-        cudaFree(l.tflags);
-        for (int p = 0; p < 3; p++) {
-            cudaFree(l.llx[p]);
-            hzdec_plane_free(&l.hz[p]);
-        }
-        devframe_free(&l.out[0]);
-        devframe_free(&l.out[1]);
-        cudaFree(l.d_pkt);
-        cudaFreeHost(l.h_pkt[0]);
-        cudaFreeHost(l.h_pkt[1]);
-        cudaFree(l.d_draw);
+        dec_lane_free(l);
     }
     arena_[0].destroy();
     arena_[1].destroy();
@@ -248,6 +248,7 @@ void DecEngine::step(int n, const int *lane_ids, const PktRef *pkts, const OutRe
     DevMV *const h_mv_ = this->h_mv_[par];
     cudaEvent_t *const ev_ = this->ev_[par];
     int step_nblk = 0; /* lanes of a step share the block grid: vectors / stability bits are packed at that pitch */
+    CodecGeom step_g = g_; /* that grid, planned from the step's first picture */
     arena_.reset();
     SbtJob *d_sj;
     void *d_hzj;
@@ -276,7 +277,6 @@ void DecEngine::step(int n, const int *lane_ids, const PktRef *pkts, const OutRe
     const double t_host0 = host_now_ms();
     HzDecDims dims;
     int n_sj = 0, n_p = 0, n_ext = 0, n_pack = 0;
-    int blk_w = 0, blk_h = 0, nbh = 0, nbv = 0;
 
     for (int k = 0; k < n; k++) {
         const int li = lane_ids[k];
@@ -303,12 +303,9 @@ void DecEngine::step(int n, const int *lane_ids, const PktRef *pkts, const OutRe
         }
         CodecGeom g = g_;
         plan_blocks(&g, bw_, bh_);
-        if (blk_w == 0) {
-            blk_w = bw_;
-            blk_h = bh_;
-            nbh = g.nbh;
-            nbv = g.nbv;
-        } else if (blk_w != bw_ || blk_h != bh_) {
+        if (step_nblk == 0) {
+            step_g = g;
+        } else if (step_g.blk_w != bw_ || step_g.blk_h != bh_) {
             /* lanes of one step share the block grid (same format => same encoder choice); a stream that
              * deviates is decoded in a later step by its caller */
             DSV_ERROR(("mixed block sizes inside one batch step"));
@@ -355,27 +352,9 @@ void DecEngine::step(int n, const int *lane_ids, const PktRef *pkts, const OutRe
             stats.h2d_bytes += pkt_len;
             d_pkt = l.d_pkt;
         }
-        /* plane directory (dsv_decoder.c:383-413) */
-        l.nplanes = 0;
-        for (int p = 0; p < 3; p++) {
-            br.align();
-            const int plen = (int) br.get_bits(32);
-            br.align();
-            const int framesz = g.cw[p] * g.ch[p] * (int) sizeof(int32_t);
-            if (plen <= 0 || plen > framesz * 2) {
-                DSV_ERROR(("plane length was strange: %d", plen));
-                break;
-            }
-            const unsigned at = br.byte_pos();
-            if (at >= pkt_len) {
-                DSV_ERROR(("plane starts past the end of the packet"));
-                break;
-            }
-            hzdec_parse_head(pkt + at, pkt_len - at, (unsigned) plen, &l.pd[p]);
-            l.pd[p].body = d_pkt + at;
-            br.skip_bytes((unsigned) plen);
-            l.nplanes++;
-        }
+        br.align();
+        /* corrupt side-info lengths can carry the reader past the end, further than a 32-bit byte offset reaches */
+        l.nplanes = parse_plane_dir(pkt, pkt_len, br.exhausted() ? pkt_len : br.byte_pos(), g, d_pkt, l.pd);
         fnums[k] = l.fnum;
         if (l.has_ref && !l.have_ref) {
             DSV_WARNING(("reference frame not found"));
@@ -482,8 +461,7 @@ void DecEngine::step(int n, const int *lane_ids, const PktRef *pkts, const OutRe
                 n_pack++;
             }
         }
-        const MotionGeom mg = {g.w, g.h, g.hs, g.vs, g.blk_w, g.blk_h, g.nbh, g.nbv, 0};
-        dec_bmc_fill(ba, &n_p, isP, mg, d_mv_, li, step_nblk, l.out[l.cur ^ 1], cur);
+        dec_bmc_fill(ba, &n_p, isP, motion_geom(g, 0), d_mv_, li, step_nblk, l.out[l.cur ^ 1], cur);
     }
     stats.host_ms += host_now_ms() - t_host0;
     if (n_sj == 0) {
@@ -510,10 +488,7 @@ void DecEngine::step(int n, const int *lane_ids, const PktRef *pkts, const OutRe
     if (n_p && timed) {
         CUDA_CHECK(cudaEventRecord(ev_[2], st));
     }
-    {
-        const MotionGeom mg = {g_.w, g_.h, g_.hs, g_.vs, blk_w, blk_h, nbh, nbv, 0};
-        bmc_launch(d_bmc, n_p, mg, st);
-    }
+    bmc_launch(d_bmc, n_p, motion_geom(step_g, 0), st);
     if (n_p && timed) {
         CUDA_CHECK(cudaEventRecord(ev_[3], st));
     }

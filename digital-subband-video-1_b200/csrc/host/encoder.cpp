@@ -79,6 +79,11 @@ void plan_blocks(CodecGeom *g, int blk_w, int blk_h)
     g->nblk = g->nbh * g->nbv;
 }
 
+MotionGeom motion_geom(const CodecGeom &g, int levels)
+{
+    return {g.w, g.h, g.hs, g.vs, g.blk_w, g.blk_h, g.nbh, g.nbv, levels};
+}
+
 bool meta_supported(const DSV_META &m)
 {
     if (m.width < 16 || m.height < 16 || (m.width & 1) || (m.height & 1) || m.width > 16384 || m.height > 16384) {
@@ -398,7 +403,7 @@ EncEngine::EncEngine(const DSV_META &md, int gop, int pyramid_levels, int lanes)
     }
     lanes_.resize((size_t) L_);
     for (int i = 0; i < L_; i++) {
-        alloc_lane(lanes_[(size_t) i]);
+        enc_lane_alloc(lanes_[(size_t) i], g_, inter_, levels_, enc_packet_cap(g_));
         lanes_[(size_t) i].d_mvf[0] = d_mv0_ + (size_t) i * g_.nblk;
         for (int b = 0; b < ENC_STAGE_SLOTS; b++) {
             lanes_[(size_t) i].d_in[b] = d_in_all_[b] + in_pitch_ * i;
@@ -406,74 +411,12 @@ EncEngine::EncEngine(const DSV_META &md, int gop, int pyramid_levels, int lanes)
     }
 }
 
-void EncEngine::alloc_lane(EncLane &l)
-{
-    const CodecGeom &g = g_;
-    CUDA_CHECK(cudaMalloc(&l.coef, g.coef_total * sizeof(int32_t)));
-    CUDA_CHECK(cudaMalloc(&l.tflags, (size_t) g.total_tiles + 16));
-    CUDA_CHECK(cudaMemset(l.tflags, 3, (size_t) g.total_tiles + 16));
-    CUDA_CHECK(cudaMalloc(&l.hz_dense, (size_t) g.total_chunks * HZ_DENSE_BYTES));
-    for (int p = 0; p < 3; p++) {
-        CUDA_CHECK(cudaMalloc(&l.llx[p], sbt_llx_elems(g.cw[p], g.ch[p]) * sizeof(int32_t)));
-        CUDA_CHECK(cudaMalloc(&l.dv[p], sbt_dv_elems(g.cw[p], g.ch[p]) * sizeof(int32_t)));
-        CUDA_CHECK(cudaMemset(l.dv[p], 0, sbt_dv_elems(g.cw[p], g.ch[p]) * sizeof(int32_t)));
-    }
-    const size_t pkt_cap = enc_packet_cap(g);
-    l.pkt_cap = pkt_cap;
-    CUDA_CHECK(cudaMalloc(&l.d_pkt, pkt_cap));
-    CUDA_CHECK(cudaMemset(l.d_pkt, 0, pkt_cap));
-    CUDA_CHECK(cudaMallocHost(&l.h_head, 512 + (size_t) g.nblk * 48));
-    devframe_alloc(&l.xf, g.w, g.h, g.subsamp);
-    if (inter_) {
-        devframe_alloc(&l.pred, g.w, g.h, g.subsamp);
-        for (int i = 0; i < 2; i++) {
-            devframe_alloc(&l.pad[i], g.w, g.h, g.subsamp);
-            devframe_alloc(&l.recon[i], g.w, g.h, g.subsamp);
-            for (int k = 0; k < levels_; k++) {
-                devframe_alloc(&l.pyr[i][k], ceil_shift(g.w, k + 1), ceil_shift(g.h, k + 1), g.subsamp);
-            }
-        }
-        for (int k = 1; k <= levels_; k++) {
-            CUDA_CHECK(cudaMalloc(&l.d_mvf[k], sizeof(DevMV) * (size_t) g.nblk));
-            CUDA_CHECK(cudaMemset(l.d_mvf[k], 0, sizeof(DevMV) * (size_t) g.nblk));
-        }
-        CUDA_CHECK(cudaMalloc(&l.d_aux, sizeof(int2) * (size_t) g.nblk));
-    }
-}
-
-void EncEngine::free_lane(EncLane &l)
-{
-    cudaFree(l.coef);
-    cudaFree(l.tflags);
-    cudaFree(l.hz_dense);
-    for (int p = 0; p < 3; p++) {
-        cudaFree(l.llx[p]);
-        cudaFree(l.dv[p]);
-    }
-    cudaFree(l.d_pkt);
-    cudaFreeHost(l.h_head);
-    devframe_free(&l.xf);
-    devframe_free(&l.pred);
-    devframe_free(&l.qrec);
-    for (int i = 0; i < 2; i++) {
-        devframe_free(&l.pad[i]);
-        devframe_free(&l.recon[i]);
-        for (int k = 0; k < DSV_MAX_PYRAMID_LEVELS; k++) {
-            devframe_free(&l.pyr[i][k]);
-        }
-    }
-    for (int k = 1; k <= DSV_MAX_PYRAMID_LEVELS; k++) {
-        cudaFree(l.d_mvf[k]);
-    }
-    cudaFree(l.d_aux);
-}
-
 EncEngine::~EncEngine()
 {
     cudaStreamSynchronize(st_);
     delete pool_;
     for (auto &l : lanes_) {
-        free_lane(l);
+        enc_lane_free(l);
     }
     arena_.destroy();
     for (auto &b : d_in_all_) {
@@ -659,7 +602,7 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
     const bool analyse = plan && plan[0].analyse, code = plan && !plan[0].analyse;
     const CodecGeom &g = g_;
     cudaStream_t st = st_;
-    const MotionGeom mg = {g.w, g.h, g.hs, g.vs, g.blk_w, g.blk_h, g.nbh, g.nbv, levels_};
+    const MotionGeom mg = motion_geom(g, levels_);
     LaneMisc *h_misc = reinterpret_cast<LaneMisc *>(h_misc_), *d_misc = reinterpret_cast<LaneMisc *>(d_misc_);
     const bool timed = time_kernels;
     KtActivate kt_on(timed ? &ktimes : nullptr);
@@ -1024,7 +967,7 @@ void EncEngine::step(int n, const int *lane_ids, const PicRef *src, DSV_BUF (*bu
         const unsigned total = h_frames_[k].total_bytes;
         DSV_BUF outbuf;
         int nb = 0;
-        if (h_frames_[k].overflow) { /* cannot happen for 8-bit input (see alloc_lane); never trust the size if it does */
+        if (h_frames_[k].overflow) { /* cannot happen for 8-bit input (see enc_packet_cap); never trust the size if it does */
             DSV_ERROR(("coded picture does not fit the packet buffer (%u bytes): picture dropped", (unsigned) l.pkt_cap));
             l.pkt_dirty = (unsigned) l.pkt_cap - 64;
             nbufs[k] = 0;

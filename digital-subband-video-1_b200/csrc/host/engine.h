@@ -44,6 +44,8 @@ struct CodecGeom {
 
 void plan_geometry(CodecGeom *g, int w, int h, int subsamp);
 void plan_blocks(CodecGeom *g, int blk_w, int blk_h);
+/* the motion kernels' view of a planned block grid, with `levels` pyramid levels */
+MotionGeom motion_geom(const CodecGeom &g, int levels);
 int size4dim(int dim);
 void predict_mv(const DevMV *mvs, int nbh, int x, int y, int *px, int *py);
 
@@ -244,6 +246,11 @@ struct EncLane {
     int gop_start = 0, is_ref = 0, has_ref = 0, forced_intra = 0, quant = 0;
     unsigned head_bytes = 0;
 };
+/* a lane's device buffers (plane_jobs.cpp), for EncEngine and the kernel-level encoder and motion handles alike: inter
+ * lanes also get the reference frames, `levels` pyramid levels and the search scratch.  d_mvf[0] and d_in[] point into
+ * the owner's lane-major arrays: they are neither allocated nor freed here. */
+void enc_lane_alloc(EncLane &l, const CodecGeom &g, bool inter, int levels, size_t pkt_bytes);
+void enc_lane_free(EncLane &l);
 
 /* optional destination for a lane's packets: written back to back at `at` instead of into fresh DSV_BUFs */
 struct PktSink {
@@ -349,8 +356,6 @@ public:
 
 private:
     void enable_reports(bool sse, bool ssim);
-    void alloc_lane(EncLane &l);
-    void free_lane(EncLane &l);
     CodecGeom g_;
     bool inter_;
     int levels_;
@@ -391,6 +396,14 @@ struct DecLane {
     DSV_FNUM fnum = 0;
     HzPlaneData pd[3];
 };
+/* a lane's device buffers (plane_jobs.cpp), for DecEngine and the kernel-level decoder handle alike; the free also
+ * releases the packet staging and overlay copy that DecEngine::step grows on demand */
+void dec_lane_alloc(DecLane &l, const CodecGeom &g);
+void dec_lane_free(DecLane &l);
+/* plane directory of a picture packet (decoder.cpp): from byte `at` of pkt (len bytes) on, up to three planes, each a
+ * 32-bit big-endian length and that many bytes.  Fills pd[] with bodies in d_pkt, the device copy of pkt, and returns
+ * the number of planes before the first whose length is out of range or which starts past the end. */
+int parse_plane_dir(const uint8_t *pkt, unsigned len, unsigned at, const CodecGeom &g, const uint8_t *d_pkt, HzPlaneData pd[3]);
 
 /* one packet of one lane */
 struct PktRef {

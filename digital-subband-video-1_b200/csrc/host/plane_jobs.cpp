@@ -1,6 +1,7 @@
 /*
- * plane_jobs.cpp -- the per-plane job descriptors of one picture, filled the same way by the engines (encoder.cpp,
- * decoder.cpp) and by the batch entry points of the kernel-level API (kernel_api.cu) that check them.
+ * plane_jobs.cpp -- the per-plane job descriptors of one picture and the lane buffers they point at, filled and
+ * allocated the same way by the engines (encoder.cpp, decoder.cpp) and by the batch entry points of the kernel-level
+ * API (kernel_api.cu) that check them.
  */
 #include "engine.h"
 
@@ -128,6 +129,100 @@ void dec_init_flags(uint8_t *d_tflags, const CodecGeom &g)
         sbt_fill_geometry(&probe, g.pw[p], g.ph[p], g.cw[p], g.ch[p], 1, p);
         CUDA_CHECK(cudaMemset(d_tflags + off, hz_flag_base(probe.dg), (size_t) g.tiles[p] + (p == 2 ? 16 : 0)));
     }
+}
+
+void enc_lane_alloc(EncLane &l, const CodecGeom &g, bool inter, int levels, size_t pkt_bytes)
+{
+    CUDA_CHECK(cudaMalloc(&l.coef, g.coef_total * sizeof(int32_t)));
+    CUDA_CHECK(cudaMalloc(&l.tflags, (size_t) g.total_tiles + 16));
+    CUDA_CHECK(cudaMemset(l.tflags, 3, (size_t) g.total_tiles + 16));
+    CUDA_CHECK(cudaMalloc(&l.hz_dense, (size_t) g.total_chunks * HZ_DENSE_BYTES));
+    for (int p = 0; p < 3; p++) {
+        CUDA_CHECK(cudaMalloc(&l.llx[p], sbt_llx_elems(g.cw[p], g.ch[p]) * sizeof(int32_t)));
+        CUDA_CHECK(cudaMalloc(&l.dv[p], sbt_dv_elems(g.cw[p], g.ch[p]) * sizeof(int32_t)));
+        CUDA_CHECK(cudaMemset(l.dv[p], 0, sbt_dv_elems(g.cw[p], g.ch[p]) * sizeof(int32_t)));
+    }
+    l.pkt_cap = pkt_bytes;
+    CUDA_CHECK(cudaMalloc(&l.d_pkt, pkt_bytes));
+    CUDA_CHECK(cudaMemset(l.d_pkt, 0, pkt_bytes));
+    CUDA_CHECK(cudaMallocHost(&l.h_head, head_capacity(g)));
+    devframe_alloc(&l.xf, g.w, g.h, g.subsamp);
+    if (inter) {
+        devframe_alloc(&l.pred, g.w, g.h, g.subsamp);
+        for (int i = 0; i < 2; i++) {
+            devframe_alloc(&l.pad[i], g.w, g.h, g.subsamp);
+            devframe_alloc(&l.recon[i], g.w, g.h, g.subsamp);
+            for (int k = 0; k < levels; k++) {
+                devframe_alloc(&l.pyr[i][k], ceil_shift(g.w, k + 1), ceil_shift(g.h, k + 1), g.subsamp);
+            }
+        }
+        for (int k = 1; k <= levels; k++) {
+            CUDA_CHECK(cudaMalloc(&l.d_mvf[k], sizeof(DevMV) * (size_t) g.nblk));
+            CUDA_CHECK(cudaMemset(l.d_mvf[k], 0, sizeof(DevMV) * (size_t) g.nblk));
+        }
+        CUDA_CHECK(cudaMalloc(&l.d_aux, sizeof(int2) * (size_t) g.nblk));
+    }
+}
+
+void enc_lane_free(EncLane &l)
+{
+    cudaFree(l.coef);
+    cudaFree(l.tflags);
+    cudaFree(l.hz_dense);
+    for (int p = 0; p < 3; p++) {
+        cudaFree(l.llx[p]);
+        cudaFree(l.dv[p]);
+    }
+    cudaFree(l.d_pkt);
+    cudaFreeHost(l.h_head);
+    devframe_free(&l.xf);
+    devframe_free(&l.pred);
+    devframe_free(&l.qrec);
+    for (int i = 0; i < 2; i++) {
+        devframe_free(&l.pad[i]);
+        devframe_free(&l.recon[i]);
+        for (int k = 0; k < DSV_MAX_PYRAMID_LEVELS; k++) {
+            devframe_free(&l.pyr[i][k]);
+        }
+    }
+    for (int k = 1; k <= DSV_MAX_PYRAMID_LEVELS; k++) {
+        cudaFree(l.d_mvf[k]);
+    }
+    cudaFree(l.d_aux);
+}
+
+void dec_lane_alloc(DecLane &l, const CodecGeom &g)
+{
+    /* coefficient planes are kept all-zero between pictures by the flag-guided clean-up (hzdec_clean_kernel) */
+    CUDA_CHECK(cudaMalloc(&l.coef, g.coef_total * sizeof(int32_t)));
+    CUDA_CHECK(cudaMemset(l.coef, 0, g.coef_total * sizeof(int32_t)));
+    CUDA_CHECK(cudaMalloc(&l.tflags, (size_t) g.total_tiles + 16));
+    dec_init_flags(l.tflags, g);
+    for (int p = 0; p < 3; p++) {
+        CUDA_CHECK(cudaMalloc(&l.llx[p], sbt_llx_elems(g.cw[p], g.ch[p]) * sizeof(int32_t)));
+        HzDecPlan pl;
+        hzdec_plan(&pl, g.cw[p], g.ch[p]);
+        hzdec_plane_alloc(&l.hz[p], pl);
+    }
+    devframe_alloc(&l.out[0], g.w, g.h, g.subsamp);
+    devframe_alloc(&l.out[1], g.w, g.h, g.subsamp);
+    /* packets are staged lazily: most are far smaller than the format's upper bound */
+}
+
+void dec_lane_free(DecLane &l)
+{
+    cudaFree(l.coef);
+    cudaFree(l.tflags);
+    for (int p = 0; p < 3; p++) {
+        cudaFree(l.llx[p]);
+        hzdec_plane_free(&l.hz[p]);
+    }
+    devframe_free(&l.out[0]);
+    devframe_free(&l.out[1]);
+    cudaFree(l.d_pkt);
+    cudaFreeHost(l.h_pkt[0]);
+    cudaFreeHost(l.h_pkt[1]);
+    cudaFree(l.d_draw);
 }
 
 void ingest_fill_picture(IngestItem *it, const uint8_t *const src[3], const DevFrame &dst)

@@ -467,23 +467,17 @@ void upload_packed(const DevFrame &f, const uint8_t *src)
     }
 }
 
-/* one lane of EncEngine (encoder.cpp alloc_lane): the buffers a picture's phase 3 reads and writes */
-struct KLane {
-    DevFrame in, pred, recon;
-    int32_t *coef = nullptr, *llx[3] = {}, *dv[3] = {};
-    uint8_t *tflags = nullptr, *hz_dense = nullptr, *pkt = nullptr;
-    unsigned pkt_dirty = 0;
-};
-
 } // namespace
 
 #define DSVK_PKT_GUARD 4096 /* bytes past the largest cap, where nothing may ever be written */
 
+/* EncEngine's lanes, lane k = picture k: its phase 3 reads the picture from xf and the prediction from pred, and leaves
+ * the reconstruction in recon[0] */
 struct DsvkEnc {
     CodecGeom g;
     int max_pics;
     size_t pkt_bytes, dv_pitch;
-    std::vector<KLane> lanes;
+    std::vector<EncLane> lanes;
     HzChunk *chunks = nullptr;
     HzFrame *frames = nullptr;
     SbtJob *d_sj = nullptr;
@@ -506,18 +500,7 @@ extern "C" void *dsvk_enc_create(int w, int h, int subsamp, int blk_w, int blk_h
     e->dv_pitch = sbt_dv_elems(g.cw[0], g.ch[0]);
     e->lanes.resize((size_t) max_pics);
     for (auto &l : e->lanes) {
-        devframe_alloc(&l.in, w, h, subsamp);
-        devframe_alloc(&l.pred, w, h, subsamp);
-        devframe_alloc(&l.recon, w, h, subsamp);
-        l.coef = dev_alloc<int32_t>(g.coef_total);
-        for (int p = 0; p < 3; p++) {
-            l.llx[p] = dev_alloc<int32_t>(sbt_llx_elems(g.cw[p], g.ch[p]));
-            l.dv[p] = dev_alloc<int32_t>(sbt_dv_elems(g.cw[p], g.ch[p]));
-        }
-        l.tflags = dev_alloc<uint8_t>((size_t) g.total_tiles);
-        CUDA_CHECK(cudaMemset(l.tflags, 3, (size_t) g.total_tiles + 16));
-        l.hz_dense = dev_alloc<uint8_t>((size_t) g.total_chunks * HZ_DENSE_BYTES, false);
-        l.pkt = dev_alloc<uint8_t>(e->pkt_bytes + DSVK_PKT_GUARD);
+        enc_lane_alloc(l, g, true, 0, e->pkt_bytes + DSVK_PKT_GUARD);
     }
     e->chunks = dev_alloc<HzChunk>((size_t) max_pics * g.total_chunks, false);
     e->frames = dev_alloc<HzFrame>((size_t) max_pics);
@@ -537,17 +520,7 @@ extern "C" void dsvk_enc_destroy(void *handle)
         return;
     }
     for (auto &l : e->lanes) {
-        devframe_free(&l.in);
-        devframe_free(&l.pred);
-        devframe_free(&l.recon);
-        cudaFree(l.coef);
-        for (int p = 0; p < 3; p++) {
-            cudaFree(l.llx[p]);
-            cudaFree(l.dv[p]);
-        }
-        cudaFree(l.tflags);
-        cudaFree(l.hz_dense);
-        cudaFree(l.pkt);
+        enc_lane_free(l);
     }
     cudaFree(e->chunks);
     cudaFree(e->frames);
@@ -574,19 +547,19 @@ extern "C" int dsvk_enc_run(void *handle, int n, const DSVK_PIC *pics, const uin
     size_t max_zero = 0;
     int n_p = 0;
     for (int k = 0; k < n; k++) {
-        KLane &l = e->lanes[(size_t) k];
+        EncLane &l = e->lanes[(size_t) k];
         const DSVK_PIC &pc = pics[k];
         if (pc.cap > e->pkt_bytes || pc.start_byte + 64 > pc.cap) {
             return -1;
         }
-        upload_packed(l.in, in + g.frame_bytes * k);
+        upload_packed(l.xf, in + g.frame_bytes * k);
         if (pred && pc.isP) {
             upload_packed(l.pred, pred + g.frame_bytes * k);
         }
         /* as the engine: the forward transform ORs its tile flags into zeroed bytes; the packet's dirty prefix is cleared */
         zero.push_back({l.tflags, ((size_t) g.total_tiles + 15) & ~(size_t) 15});
         if (l.pkt_dirty) {
-            zero.push_back({l.pkt, ((size_t) l.pkt_dirty + 64 + 15) & ~(size_t) 15});
+            zero.push_back({l.d_pkt, ((size_t) l.pkt_dirty + 64 + 15) & ~(size_t) 15});
         }
         n_p += pc.isP != 0;
     }
@@ -596,14 +569,14 @@ extern "C" int dsvk_enc_run(void *handle, int n, const DSVK_PIC *pics, const uin
     uint8_t *d_stab = dev_alloc<uint8_t>((size_t) g.nblk * n, false);
     for (int k = 0; k < n; k++) {
         CUDA_CHECK(cudaMemcpy(d_stab + (size_t) g.nblk * k, pics[k].stable, (size_t) g.nblk, cudaMemcpyHostToDevice));
-        KLane &l = e->lanes[(size_t) k];
+        EncLane &l = e->lanes[(size_t) k];
         const int isP = pics[k].isP != 0;
         for (int p = 0; p < 3; p++) {
             EncPlaneIO io;
-            io.in = l.in.p[p];
-            io.in_stride = l.in.stride[p];
-            io.out = l.recon.p[p];
-            io.out_stride = l.recon.stride[p];
+            io.in = l.xf.p[p];
+            io.in_stride = l.xf.stride[p];
+            io.out = l.recon[0].p[p];
+            io.out_stride = l.recon[0].stride[p];
             io.pred = pred ? l.pred.p[p] : nullptr;
             io.pred_stride = l.pred.stride[p];
             io.coef = l.coef + g.coef_off[p];
@@ -614,7 +587,7 @@ extern "C" int dsvk_enc_run(void *handle, int n, const DSVK_PIC *pics, const uin
             io.stable = d_stab + (size_t) g.nblk * k;
             enc_fill_plane(&sj[(size_t) 3 * k + p], &hj[(size_t) 3 * k + p], g, p, k, isP, pics[k].quant, io);
         }
-        enc_fill_frame(&hf[(size_t) k], l.pkt, pics[k].cap, pics[k].start_byte, k);
+        enc_fill_frame(&hf[(size_t) k], l.d_pkt, pics[k].cap, pics[k].start_byte, k);
     }
     const SbtDims sdims = sbt_assign_tiles(sj.data(), 3 * n);
     CUDA_CHECK(cudaMemcpy(e->d_sj, sj.data(), sizeof(SbtJob) * sj.size(), cudaMemcpyHostToDevice));
@@ -629,7 +602,7 @@ extern "C" int dsvk_enc_run(void *handle, int n, const DSVK_PIC *pics, const uin
     CUDA_CHECK(cudaMemcpy(hf.data(), e->frames, sizeof(HzFrame) * hf.size(), cudaMemcpyDeviceToHost));
     cudaFree(d_stab);
     for (int k = 0; k < n; k++) {
-        KLane &l = e->lanes[(size_t) k];
+        EncLane &l = e->lanes[(size_t) k];
         const HzFrame &f = hf[(size_t) k];
         /* as the engine: an overflowed packet is dirty up to its cap */
         l.pkt_dirty = f.overflow ? pics[k].cap - 64 : f.total_bytes;
@@ -640,14 +613,14 @@ extern "C" int dsvk_enc_run(void *handle, int n, const DSVK_PIC *pics, const uin
             info[2 + p] = f.plane_bytes[p];
             info[5 + p] = (unsigned) sj[(size_t) 3 * k + p].dg.total;
         }
-        CUDA_CHECK(cudaMemcpy(pkt_out + (e->pkt_bytes + DSVK_PKT_GUARD) * k, l.pkt, e->pkt_bytes + DSVK_PKT_GUARD, cudaMemcpyDeviceToHost));
+        CUDA_CHECK(cudaMemcpy(pkt_out + (e->pkt_bytes + DSVK_PKT_GUARD) * k, l.d_pkt, e->pkt_bytes + DSVK_PKT_GUARD, cudaMemcpyDeviceToHost));
         CUDA_CHECK(cudaMemcpy(coef_out + g.coef_total * k, l.coef, g.coef_total * sizeof(int32_t), cudaMemcpyDeviceToHost));
         for (int p = 0; p < 3; p++) {
             CUDA_CHECK(cudaMemcpy(dv_out + e->dv_pitch * (3 * k + p), l.dv[p], sbt_dv_elems(g.cw[p], g.ch[p]) * sizeof(int32_t),
                                   cudaMemcpyDeviceToHost));
         }
         CUDA_CHECK(cudaMemcpy(tflags_out + (size_t) g.total_tiles * k, l.tflags, (size_t) g.total_tiles, cudaMemcpyDeviceToHost));
-        download_frame(l.recon, recon_out + g.frame_bytes * k);
+        download_frame(l.recon[0], recon_out + g.frame_bytes * k);
     }
     return 0;
     DSV_API_END(-100)
@@ -889,12 +862,10 @@ extern "C" int dsvk_ssim_batch(int n, const int *geo, const uint8_t *src, const 
     DSV_API_END(-100)
 }
 
-/* one lane of DecEngine (decoder.cpp): coefficient planes and tile flags carry over from picture to picture */
+/* one lane of DecEngine: coefficient planes and tile flags carry over from picture to picture */
 struct DsvkDec {
     CodecGeom g;
-    int32_t *coef = nullptr;
-    uint8_t *tflags = nullptr;
-    HzDecPlaneBufs hz[3];
+    DecLane l;
 };
 
 extern "C" void *dsvk_dec_create(int w, int h, int subsamp, int blk_w, int blk_h)
@@ -906,14 +877,7 @@ extern "C" void *dsvk_dec_create(int w, int h, int subsamp, int blk_w, int blk_h
     DsvkDec *d = new DsvkDec;
     plan_geometry(&d->g, w, h, subsamp);
     plan_blocks(&d->g, blk_w, blk_h);
-    d->coef = dev_alloc<int32_t>(d->g.coef_total);
-    CUDA_CHECK(cudaMalloc(&d->tflags, (size_t) d->g.total_tiles + 16));
-    dec_init_flags(d->tflags, d->g);
-    for (int p = 0; p < 3; p++) {
-        HzDecPlan pl;
-        hzdec_plan(&pl, d->g.cw[p], d->g.ch[p]);
-        hzdec_plane_alloc(&d->hz[p], pl);
-    }
+    dec_lane_alloc(d->l, d->g);
     return d;
     DSV_API_END(nullptr)
 }
@@ -924,11 +888,7 @@ extern "C" void dsvk_dec_destroy(void *handle)
     if (!d) {
         return;
     }
-    cudaFree(d->coef);
-    cudaFree(d->tflags);
-    for (int p = 0; p < 3; p++) {
-        hzdec_plane_free(&d->hz[p]);
-    }
+    dec_lane_free(d->l);
     delete d;
 }
 
@@ -939,6 +899,7 @@ extern "C" int dsvk_dec_run(void *handle, const DSVK_PIC *pic, const uint8_t *pl
     DSV_API_BEGIN
     DsvkDec *d = static_cast<DsvkDec *>(handle);
     const CodecGeom &g = d->g;
+    DecLane &l = d->l;
     if (len <= 0) {
         return -1;
     }
@@ -946,35 +907,17 @@ extern "C" int dsvk_dec_run(void *handle, const DSVK_PIC *pic, const uint8_t *pl
     CUDA_CHECK(cudaMemcpy(d_pkt, planes, (size_t) len, cudaMemcpyHostToDevice));
     uint8_t *d_stab = dev_alloc<uint8_t>((size_t) g.nblk, false);
     CUDA_CHECK(cudaMemcpy(d_stab, pic->stable, (size_t) g.nblk, cudaMemcpyHostToDevice));
-    /* plane directory (decoder.cpp) */
     HzPlaneData pd[3];
-    int nplanes = 0;
-    unsigned at = 0;
-    for (int p = 0; p < 3; p++) {
-        if (at + 4 > (unsigned) len) {
-            break;
-        }
-        const int plen = (int) (((unsigned) planes[at] << 24) | ((unsigned) planes[at + 1] << 16) | ((unsigned) planes[at + 2] << 8) | planes[at + 3]);
-        at += 4;
-        const int framesz = g.cw[p] * g.ch[p] * (int) sizeof(int32_t);
-        if (plen <= 0 || plen > framesz * 2 || at >= (unsigned) len) {
-            break;
-        }
-        hzdec_parse_head(planes + at, (unsigned) len - at, (unsigned) plen, &pd[p]);
-        pd[p].body = d_pkt + at;
-        at += (unsigned) plen;
-        nplanes++;
-    }
-    DevFrame unused;
+    const int nplanes = parse_plane_dir(planes, (unsigned) len, 0, g, d_pkt, pd);
     SbtJob sj[3];
     HzCleanItem clean[3];
     std::vector<uint8_t> hzj(hzdec_job_size() * 3);
     HzDecDims dims;
     for (int p = 0; p < 3; p++) {
         HzJob h;
-        dec_fill_plane(&sj[p], &h, &clean[p], g, p, pic->isP != 0, pic->quant, unused, d->coef, nullptr, d->tflags, d_stab);
+        dec_fill_plane(&sj[p], &h, &clean[p], g, p, pic->isP != 0, pic->quant, l.out[l.cur], l.coef, l.llx[p], l.tflags, d_stab);
         if (p < nplanes) {
-            hzdec_fill_job(hzj.data() + hzdec_job_size() * (size_t) dims.njobs, h, pd[p], d->hz[p], &dims);
+            hzdec_fill_job(hzj.data() + hzdec_job_size() * (size_t) dims.njobs, h, pd[p], l.hz[p], &dims);
         }
     }
     HzCleanItem *d_clean = dev_alloc<HzCleanItem>(3, false);
@@ -984,8 +927,8 @@ extern "C" int dsvk_dec_run(void *handle, const DSVK_PIC *pic, const uint8_t *pl
     hzdec_clean_launch(d_clean, 3, g.tiles[0], 0);
     hzdec_launch_jobs(d_hzj, dims, 0);
     CUDA_CHECK(cudaDeviceSynchronize());
-    CUDA_CHECK(cudaMemcpy(coef_out, d->coef, g.coef_total * sizeof(int32_t), cudaMemcpyDeviceToHost));
-    CUDA_CHECK(cudaMemcpy(tflags_out, d->tflags, (size_t) g.total_tiles, cudaMemcpyDeviceToHost));
+    CUDA_CHECK(cudaMemcpy(coef_out, l.coef, g.coef_total * sizeof(int32_t), cudaMemcpyDeviceToHost));
+    CUDA_CHECK(cudaMemcpy(tflags_out, l.tflags, (size_t) g.total_tiles, cudaMemcpyDeviceToHost));
     cudaFree(d_pkt);
     cudaFree(d_stab);
     cudaFree(d_clean);
@@ -996,22 +939,15 @@ extern "C" int dsvk_dec_run(void *handle, const DSVK_PIC *pic, const uint8_t *pl
 
 /* ---- batch entry points: the motion kernels configured as the engines launch them --------------------------------- */
 
-/* one lane of EncEngine's phase 1 (encoder.cpp alloc_lane): ingested frames and pyramids alternate with the picture
- * parity (cur), so a lane's search reference is its previous call's ingested frame */
-struct DsvkMeLane {
-    DevFrame pad[2], recon[2], pyr[2][DSV_MAX_PYRAMID_LEVELS], xf, pred;
-    DevMV *d_mvf[DSV_MAX_PYRAMID_LEVELS + 1] = {};
-    int2 *d_aux = nullptr;
-    uint8_t *d_in = nullptr; /* staging buffer of host pictures */
-    int cur = 0, have_ref = 0;
-};
-
+/* EncEngine's lanes for its phase 1: ingested frames and pyramids alternate with the picture parity (cur), so a lane's
+ * search reference is its previous call's ingested frame */
 struct DsvkMe {
     CodecGeom g;
     MotionGeom mg;
     int levels, max_pics;
-    std::vector<DsvkMeLane> lanes;
+    std::vector<EncLane> lanes;
     DevMV *d_mv0 = nullptr, *h_mv0 = nullptr; /* level-0 fields of all lanes, lane-major (EncEngine::d_mv0_ / h_mv0_) */
+    uint8_t *d_stage = nullptr; /* staging of host pictures, one slot per lane (EncLane::d_in[0]) */
     LaneMisc *d_misc = nullptr;
     StepArena arena;
 };
@@ -1028,7 +964,7 @@ extern "C" void *dsvk_me_create(int w, int h, int subsamp, int blk_w, int blk_h,
     plan_geometry(&m->g, w, h, subsamp);
     plan_blocks(&m->g, blk_w, blk_h);
     const CodecGeom &g = m->g;
-    m->mg = {g.w, g.h, g.hs, g.vs, g.blk_w, g.blk_h, g.nbh, g.nbv, levels};
+    m->mg = motion_geom(g, levels);
     m->levels = levels;
     m->max_pics = max_pics;
     m->d_mv0 = dev_alloc<DevMV>((size_t) g.nblk * max_pics);
@@ -1037,24 +973,15 @@ extern "C" void *dsvk_me_create(int w, int h, int subsamp, int blk_w, int blk_h,
     m->d_misc = dev_alloc<LaneMisc>((size_t) max_pics);
     m->arena.create(((size_t) 3 * sizeof(IngestItem) + (size_t) levels * sizeof(Down2Item) + sizeof(SumItem) +
                      (size_t) (levels + 1) * sizeof(HmeArgs) + sizeof(BmcArgs) + 3 * sizeof(PlaneRef) + 256) * max_pics + 4096);
+    /* slots start 256-byte aligned, as a buffer of their own would */
+    const size_t stage_pitch = (g.frame_bytes + DSVK_STAGE_SLACK + 255) & ~(size_t) 255;
+    CUDA_CHECK(cudaMalloc(&m->d_stage, stage_pitch * max_pics));
     m->lanes.resize((size_t) max_pics);
     for (int i = 0; i < max_pics; i++) {
-        DsvkMeLane &l = m->lanes[(size_t) i];
-        devframe_alloc(&l.xf, w, h, subsamp);
-        devframe_alloc(&l.pred, w, h, subsamp);
-        for (int b = 0; b < 2; b++) {
-            devframe_alloc(&l.pad[b], w, h, subsamp);
-            devframe_alloc(&l.recon[b], w, h, subsamp);
-            for (int k = 0; k < levels; k++) {
-                devframe_alloc(&l.pyr[b][k], ceil_shift(w, k + 1), ceil_shift(h, k + 1), subsamp);
-            }
-        }
+        EncLane &l = m->lanes[(size_t) i];
+        enc_lane_alloc(l, g, true, levels, enc_packet_cap(g));
         l.d_mvf[0] = m->d_mv0 + (size_t) i * g.nblk;
-        for (int k = 1; k <= levels; k++) {
-            l.d_mvf[k] = dev_alloc<DevMV>((size_t) g.nblk);
-        }
-        l.d_aux = dev_alloc<int2>((size_t) g.nblk);
-        l.d_in = dev_alloc<uint8_t>(g.frame_bytes + DSVK_STAGE_SLACK);
+        l.d_in[0] = m->d_stage + stage_pitch * i;
     }
     return m;
     DSV_API_END(nullptr)
@@ -1067,21 +994,9 @@ extern "C" void dsvk_me_destroy(void *handle)
         return;
     }
     for (auto &l : m->lanes) {
-        devframe_free(&l.xf);
-        devframe_free(&l.pred);
-        for (int b = 0; b < 2; b++) {
-            devframe_free(&l.pad[b]);
-            devframe_free(&l.recon[b]);
-            for (int k = 0; k < m->levels; k++) {
-                devframe_free(&l.pyr[b][k]);
-            }
-        }
-        for (int k = 1; k <= m->levels; k++) {
-            cudaFree(l.d_mvf[k]);
-        }
-        cudaFree(l.d_aux);
-        cudaFree(l.d_in);
+        enc_lane_free(l);
     }
+    cudaFree(m->d_stage);
     cudaFree(m->d_mv0);
     cudaFreeHost(m->h_mv0);
     cudaFree(m->d_misc);
@@ -1095,7 +1010,7 @@ extern "C" long dsvk_me_frame_bytes(void *handle, int level)
     if (level < 0 || level > m->levels) {
         return -1;
     }
-    const DsvkMeLane &l = m->lanes[0];
+    const EncLane &l = m->lanes[0];
     return (long) (level == 0 ? l.pad[0].bytes : l.pyr[0][level - 1].bytes);
 }
 
@@ -1125,10 +1040,10 @@ extern "C" int dsvk_me_run(void *handle, int n, const DSVK_ME_PIC *pics, const v
     IngestItem *d_ing;
     IngestItem *ing = ar.push_n<IngestItem>((size_t) 3 * n, &d_ing);
     for (int k = 0; k < n; k++) {
-        DsvkMeLane &l = m->lanes[(size_t) k];
+        EncLane &l = m->lanes[(size_t) k];
         const uint8_t *base = pics[k].src;
         if (!pics[k].src_on_device) {
-            uint8_t *stage = l.d_in + pics[k].stage_offset;
+            uint8_t *stage = l.d_in[0] + pics[k].stage_offset;
             CUDA_CHECK(cudaMemcpy(stage, pics[k].src, g.frame_bytes, cudaMemcpyHostToDevice));
             base = stage;
         }
@@ -1142,7 +1057,7 @@ extern "C" int dsvk_me_run(void *handle, int n, const DSVK_ME_PIC *pics, const v
         for (int lv = 0; lv < levels; lv++) {
             Down2Item *dn = ar.push_n<Down2Item>((size_t) n, &d_dn[lv]);
             for (int k = 0; k < n; k++) {
-                DsvkMeLane &l = m->lanes[(size_t) k];
+                EncLane &l = m->lanes[(size_t) k];
                 down2_fill_level(&dn[k], l.pad[l.cur], l.pyr[l.cur], lv);
             }
         }
@@ -1157,7 +1072,7 @@ extern "C" int dsvk_me_run(void *handle, int n, const DSVK_ME_PIC *pics, const v
         if (n_search) {
             HmeArgs *ha = ar.push_n<HmeArgs>((size_t) (levels + 1) * n_search, &d_hme);
             for (int k = 0, q = 0; k < n; k++) {
-                DsvkMeLane &l = m->lanes[(size_t) k];
+                EncLane &l = m->lanes[(size_t) k];
                 if (pics[k].has_ref) {
                     hme_fill_lane(ha, n_search, q++, mg, l.pad[l.cur], l.pyr[l.cur], l.pad[l.cur ^ 1], l.pyr[l.cur ^ 1], l.d_mvf, l.d_aux,
                                   m->d_misc, k);
@@ -1169,7 +1084,7 @@ extern "C" int dsvk_me_run(void *handle, int n, const DSVK_ME_PIC *pics, const v
     if (n_search) {
         BmcArgs *ba = ar.push_n<BmcArgs>((size_t) n_search, &d_bmc);
         for (int k = 0, q = 0; k < n; k++) {
-            DsvkMeLane &l = m->lanes[(size_t) k];
+            EncLane &l = m->lanes[(size_t) k];
             if (pics[k].has_ref) {
                 enc_bmc_fill(&ba[q++], mg, l.d_mvf[0], l.recon[l.cur ^ 1], l.pred, l.pad[l.cur], l.xf);
             }
@@ -1233,7 +1148,7 @@ extern "C" int dsvk_me_run(void *handle, int n, const DSVK_ME_PIC *pics, const v
     CUDA_CHECK(cudaMemcpy(mv_out, m->d_mv0, sizeof(DevMV) * (size_t) g.nblk * n, cudaMemcpyDeviceToHost));
     uint8_t *f_at = frames_out;
     for (int k = 0; k < n; k++) {
-        DsvkMeLane &l = m->lanes[(size_t) k];
+        EncLane &l = m->lanes[(size_t) k];
         misc_out[2 * k] = (int64_t) misc[(size_t) k].luma_sum;
         misc_out[2 * k + 1] = misc[(size_t) k].nintra;
         CUDA_CHECK(cudaMemcpy(f_at, l.pad[l.cur].alloc, l.pad[l.cur].bytes, cudaMemcpyDeviceToHost));
@@ -1263,7 +1178,7 @@ extern "C" int dsvk_add_pred_batch(int w, int h, int subsamp, int blk_w, int blk
     CodecGeom g;
     plan_geometry(&g, w, h, subsamp);
     plan_blocks(&g, blk_w, blk_h);
-    const MotionGeom mg = {g.w, g.h, g.hs, g.vs, g.blk_w, g.blk_h, g.nbh, g.nbv, 0};
+    const MotionGeom mg = motion_geom(g, 0);
     std::vector<DevFrame> cur((size_t) n), prev((size_t) n);
     DevMV *d_mv = dev_alloc<DevMV>((size_t) g.nblk * n, false);
     CUDA_CHECK(cudaMemcpy(d_mv, mvs, sizeof(DevMV) * (size_t) g.nblk * n, cudaMemcpyHostToDevice));
