@@ -105,6 +105,7 @@ extern "C" DSVB_ENC *dsvb_enc_create(const int *cfg, int lanes, int device)
     e->lanes = lanes;
     e->device = device;
     e->state.resize((size_t) lanes);
+    e->live.assign((size_t) lanes, LIVE_FREE);
     /* one probe state fixes the block grid and the pyramid depth for the engine */
     DSV_ENCODER probe;
     apply_cfg(&probe, cfg);
@@ -119,6 +120,11 @@ extern "C" void dsvb_enc_destroy(DSVB_ENC *e)
 {
     if (e) {
         use_device(e->device);
+        for (int i = 0; i < e->lanes; i++) {
+            if (e->live[(size_t) i] != LIVE_FREE) { /* live streams never closed */
+                release_state(&e->state[(size_t) i]);
+            }
+        }
         delete e->eng;
         cudaFreeHost(e->h_stage);
         cudaFree(e->d_cache);
@@ -195,6 +201,9 @@ extern "C" int dsvb_encode(DSVB_ENC *e, int nseq, int nframes, const uint8_t *co
                            uint8_t *const *streams, const long *caps, long *lens)
 {
     DSV_API_BEGIN
+    if (e->live_open) {
+        return -2; /* the waves rebind lanes 0..n-1: open live streams hold some of them */
+    }
     use_device(e->device);
     const CodecGeom &g = e->eng->geom();
     const int L = e->lanes;
@@ -287,6 +296,7 @@ extern "C" DSVB_DEC *dsvb_dec_create(int lanes, int device)
     d->lanes = lanes;
     d->device = device;
     d->eng = nullptr;
+    d->live.assign((size_t) lanes, LIVE_FREE);
     return d;
 }
 
@@ -354,6 +364,23 @@ extern "C" void dsvb_dec_stats(DSVB_DEC *d, double *stats, int reset)
 }
 
 static unsigned be32(const uint8_t *p) { return ((unsigned) p[0] << 24) | ((unsigned) p[1] << 16) | ((unsigned) p[2] << 8) | p[3]; }
+
+void dsv::dec_use_format(DSVB_DEC *d, const DSV_META &md)
+{
+    if (d->eng && !d->eng->matches(md)) {
+        add_stats(d->carried, d->eng->stats);
+        delete d->eng;
+        d->eng = nullptr;
+    }
+    if (!d->eng) {
+        d->eng = new DecEngine(md, d->lanes);
+        if (d->time_kernels >= 0) {
+            d->eng->time_kernels = d->time_kernels != 0;
+        }
+        d->eng->draw_mode = d->draw_info;
+        d->eng->set_out420(d->out420 != 0);
+    }
+}
 
 /*
  * Lock-step decode of a set of container segments: every lane walks its segment packet by packet (metadata / EOS
@@ -423,24 +450,12 @@ int dsv::decode_segments(DSVB_DEC *d, int nseg, DecSegment *segs, int out_on_dev
                         rc = -5;
                         continue;
                     }
-                    if (d->eng && !d->eng->matches(md)) {
-                        if (stepped || m > 0) {
-                            cur[(size_t) k] = -1; /* one picture format per call */
-                            rc = -6;
-                            continue;
-                        }
-                        add_stats(d->carried, d->eng->stats);
-                        delete d->eng;
-                        d->eng = nullptr;
+                    if (d->eng && !d->eng->matches(md) && (stepped || m > 0)) {
+                        cur[(size_t) k] = -1; /* one picture format per call */
+                        rc = -6;
+                        continue;
                     }
-                    if (!d->eng) {
-                        d->eng = new DecEngine(md, L);
-                        if (d->time_kernels >= 0) {
-                            d->eng->time_kernels = d->time_kernels != 0;
-                        }
-                        d->eng->draw_mode = d->draw_info;
-                        d->eng->set_out420(d->out420 != 0);
-                    }
+                    dec_use_format(d, md);
                     got_meta[(size_t) k] = 1;
                     continue;
                 }
@@ -497,6 +512,9 @@ extern "C" int dsvb_decode(DSVB_DEC *d, int nseq, const uint8_t *const *streams,
                            const long *lens, uint8_t *const *out, const long *out_caps, int out_on_device, int *frames)
 {
     DSV_API_BEGIN
+    if (d->live_open) {
+        return -2; /* the segments would take over lanes that open live streams hold */
+    }
     use_device(d->device);
     std::vector<DecSegment> segs((size_t) nseq);
     for (int s = 0; s < nseq; s++) {

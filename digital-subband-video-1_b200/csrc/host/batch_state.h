@@ -35,6 +35,9 @@ struct DSVB_ENC {
     std::vector<std::vector<DSVB_PICINFO>> info;
     bool ssim_valid = false; /* SSIM report of the last encode call, the same way */
     std::vector<std::vector<DSVB_PICSSIM>> ssim;
+    /* live streams (live.cpp): stream id = lane, its DSV_ENCODER is state[lane]; live[lane] is one of LIVE_* */
+    std::vector<uint8_t> live;
+    int live_open = 0;
 };
 
 struct DSVB_DEC {
@@ -42,7 +45,14 @@ struct DSVB_DEC {
     int draw_info = 0, out420 = 0, time_kernels = -1; /* -1: the engine's default (DSV_KERNEL_TIMES) */
     dsv::DecEngine *eng;
     dsv::EngineStats carried; /* stats of engines replaced after a format change */
+    /* live streams (live.cpp): stream id = lane; live[lane] is one of LIVE_* */
+    std::vector<uint8_t> live;
+    int live_open = 0;
 };
+
+/* a lane's live-stream state: free; open; open and past the point the caller holds (encoder: an output buffer was too
+ * small) or open with its picture format known (decoder: a metadata packet arrived) */
+enum { LIVE_FREE = 0, LIVE_OPEN = 1, LIVE_BROKEN = 2, LIVE_HAS_META = 2 };
 
 namespace dsv {
 void use_device(int device);
@@ -59,6 +69,9 @@ struct DecSegment {
     int frames;                /* out: pictures decoded */
 };
 int decode_segments(DSVB_DEC *d, int nseg, DecSegment *segs, int out_on_device);
+/* make the decoder's engine one for md's picture format: created when there is none, replaced (every lane's references
+ * are lost, its stats carried) when the format differs */
+void dec_use_format(DSVB_DEC *d, const DSV_META &md);
 /* dsvb_*_picture_info / dsvb_*_picture_ssim: the records of sequence seq, at most cap of them; their count, or -1 */
 template <typename R> int copy_records(bool valid, const std::vector<std::vector<R>> &recs, int seq, R *out, int cap)
 {

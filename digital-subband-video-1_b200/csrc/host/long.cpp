@@ -482,6 +482,9 @@ extern "C" int dsvb_encode_long(DSVB_ENC *e, int nframes, const uint8_t *yuv, in
                                 int *info)
 {
     DSV_API_BEGIN
+    if (e->live_open) {
+        return -2; /* the chains run on lanes that open live streams hold */
+    }
     use_device(e->device);
     e->info_valid = e->ssim_valid = false;
     e->info.clear();
@@ -518,6 +521,9 @@ extern "C" int dsvb_decode_long(DSVB_DEC *d, const uint8_t *stream, const uint8_
                                 int out_on_device, int *frames)
 {
     DSV_API_BEGIN
+    if (d->live_open) {
+        return -2; /* the chains run on lanes that open live streams hold */
+    }
     use_device(d->device);
     /* chains: a new segment starts at every picture without a reference; the metadata packets right in front of it
      * go with it.  Segment 0 holds the stream's first metadata packet and is walked first (lane 0), so the engine

@@ -37,7 +37,8 @@ void dsvb_enc_destroy(DSVB_ENC *e);
  * Encode nseq sequences of nframes pictures each.  yuv[s]: packed planar pictures of sequence s back to
  * back, in host memory (on_device = 0; pinned memory avoids a staging copy) or device memory (1).
  * streams[s] (host, caps[s] bytes) receives the complete .dsv stream (META, PIC..., EOS) of sequence s,
- * lens[s] its length.  Returns 0, or -1 if a stream buffer is too small.
+ * lens[s] its length.  Returns 0, or -1 if a stream buffer is too small, or -2 while a live stream is open
+ * (dsvb_enc_open below: the waves rebind lanes 0..nseq-1; open streams are left untouched).
  */
 int dsvb_encode(DSVB_ENC *e, int nseq, int nframes, const uint8_t *const *yuv, int on_device,
                 uint8_t *const *streams, const long *caps, long *lens);
@@ -54,7 +55,8 @@ void dsvb_dec_destroy(DSVB_DEC *d);
  * heads are parsed on the host).  streams_dev (optional, may be NULL): device copies of the same bytes;
  * when given no packet is copied host->device.  out[s]: packed planar pictures at offset
  * fnum * frame_bytes, in host (out_on_device = 0) or device (1) memory of out_caps[s] bytes.
- * frames[s] receives the number of pictures decoded.  Returns 0, or a negative value on a malformed container.
+ * frames[s] receives the number of pictures decoded.  Returns 0, or a negative value on a malformed container;
+ * -2 while a live stream is open (dsvb_dec_open below).
  */
 int dsvb_decode(DSVB_DEC *d, int nseq, const uint8_t *const *streams, const uint8_t *const *streams_dev,
                 const long *lens, uint8_t *const *out, const long *out_caps, int out_on_device, int *frames);
@@ -78,13 +80,13 @@ void dsvb_dec_set_out420p(DSVB_DEC *d, int on);
  * pictures to dsv_enc one by one.  ABR streams (rc_mode != CRF) serialise on packet sizes and run on one lane.
  * yuv: nframes packed planar pictures (host, or device when on_device = 1).  info (optional, 4 ints):
  * chains, forced I pictures, longest chain, GPUs used (0: single-GPU entry, 1: serial ABR path).
- * Returns 0, -1 if `stream` (cap bytes) is too small, -100 on a CUDA failure.
+ * Returns 0, -1 if `stream` (cap bytes) is too small, -2 while a live stream is open, -100 on a CUDA failure.
  */
 int dsvb_encode_long(DSVB_ENC *e, int nframes, const uint8_t *yuv, int on_device, uint8_t *stream, long cap, long *len,
                      int *info);
 /* One container decoded with its chains (cut at every picture that has no reference, dsv_decoder.c:286-472)
  * spread over the lanes.  stream_dev (optional): device copy of the same bytes.  Pictures land at
- * out + fnum * frame_bytes like dsvb_decode. */
+ * out + fnum * frame_bytes like dsvb_decode.  -2 while a live stream is open. */
 int dsvb_decode_long(DSVB_DEC *d, const uint8_t *stream, const uint8_t *stream_dev, long len, uint8_t *out, long out_cap,
                      int out_on_device, int *frames);
 
@@ -130,7 +132,9 @@ void dsvb_dec_kernel_times(DSVB_DEC *d, double *ms, double *launches, int reset)
  *   dsvb_enc_picture_info / dsvb_multi_picture_info: the records of sequence `seq` of the last dsvb_encode /
  *   dsvb_multi_encode call (seq 0 for dsvb_encode_long / dsvb_multi_encode_long), in picture order.  Returns the
  *   number of records and writes at most `cap` of them; -1 if the report was off during that call, the call failed,
- *   or seq is out of range.
+ *   or seq is out of range.  After dsvb_enc_push, seq is a POSITION in that call's ids (not a stream id): the one
+ *   record of the picture pushed there, or 0 records if that stream's output did not fit (lens = -1) or the picture
+ *   was dropped.  A push refused with -2 leaves the records of the call before it.
  * PSNR of plane p: 10 * log10(255^2 * samples[p] / sse[p]) (infinite when sse[p] == 0).
  */
 typedef struct DSVB_PICINFO { /* 72 bytes, no padding */
@@ -154,7 +158,8 @@ int dsvb_multi_picture_info(DSVB_MULTI *m, int seq, DSVB_PICINFO *out, int cap);
  * and pictures that are not references get the inverse transform they otherwise skip.  The streams do not change.
  *   dsvb_enc_picture_ssim / dsvb_multi_picture_ssim: as dsvb_enc_picture_info / dsvb_multi_picture_info (records of
  *   sequence `seq` of the last encode call in picture order, at most `cap` written, the count returned; -1 if the
- *   SSIM report was off during that call, the call failed, or seq is out of range).
+ *   SSIM report was off during that call, the call failed, or seq is out of range; after dsvb_enc_push, seq is a
+ *   position in that call's ids, as above).
  * Definition (x264 / ffmpeg, 8-bit), for a plane of pw x ph samples, source a, reconstruction b:
  *   4x4 blocks: bw = pw / 4, bh = ph / 4 (the last pw % 4 columns and ph % 4 rows are not read);
  *   windows: the 2x2 groups of blocks at block positions (i, j), 0 <= i < bw - 1, 0 <= j < bh - 1 (8x8 samples,
@@ -174,6 +179,63 @@ void dsvb_enc_set_picture_ssim(DSVB_ENC *e, int on);
 int dsvb_enc_picture_ssim(DSVB_ENC *e, int seq, DSVB_PICSSIM *out, int cap);
 void dsvb_multi_set_picture_ssim(DSVB_MULTI *m, int on);
 int dsvb_multi_picture_ssim(DSVB_MULTI *m, int seq, DSVB_PICSSIM *out, int cap);
+
+/*
+ * LIVE STREAMS: pictures (packets) that arrive one per stream at a time -- cameras, screen capture, a transcoder fed
+ * from the network -- coded as they come, on the same lock-step engine.  A stream id is a lane of the object; each
+ * push is ONE engine step over the streams it lists, whatever their GOP phases (I and P pictures share steps).  Every
+ * stream runs its own copy of the reference's host state machine (frame numbers from 0, GOP, scene cuts, stability,
+ * ABR on its own packet sizes), so its bytes do not depend on the other streams.  All streams of an object use its
+ * cfg (encoder) / one picture format (decoder).  While any stream is open, dsvb_encode / dsvb_encode_long /
+ * dsvb_decode / dsvb_decode_long return -2.  One thread drives an object at a time, as for the calls above.
+ *
+ *   dsvb_enc_open       a fresh stream: its id in [0, lanes), or -1 when every lane holds one.
+ *   dsvb_enc_push_bound the most bytes one push can write for one stream (metadata packet + largest picture packet).
+ *   dsvb_enc_push       one packed planar picture per listed stream: pics[k] for stream ids[k], host memory (pinned or
+ *                       not, on_device = 0) or device memory (1).  out[k] (host, caps[k] bytes) receives exactly what
+ *                       dsv_enc returns for that picture -- the metadata packet at a GOP start, then the picture
+ *                       packet, back to back -- and lens[k] their length; the bytes are there when the call returns.
+ *                       A stream's push outputs in order followed by its close output are byte for byte the stream
+ *                       dsv_enc / dsvb_encode produce for the same pictures and cfg.
+ *                       Returns 0; -2 if an id is out of range, not open (or broken, below) or listed twice, checked
+ *                       before any work: nothing is consumed and no state changes; -1 if an out[k] was too small:
+ *                       lens[k] = -1 and that stream is BROKEN (its encoder went past bytes the caller does not hold),
+ *                       later pushes to it return -2 until it is closed, and the other streams of the call are
+ *                       complete and correct; -100 on a CUDA failure.
+ *   dsvb_enc_close      writes the end-of-stream packet (14 bytes) to out and frees the stream's lane.  Returns 0 and
+ *                       *len = its length; -1 and *len = -1 if out is NULL or cap too small (the lane is freed all the
+ *                       same: close a broken stream with out = NULL); -2 if id is not an open stream.
+ */
+int dsvb_enc_open(DSVB_ENC *e);
+long dsvb_enc_push_bound(DSVB_ENC *e);
+int dsvb_enc_push(DSVB_ENC *e, int n, const int *ids, const uint8_t *const *pics, int on_device, uint8_t *const *out,
+                  const long *caps, long *lens);
+int dsvb_enc_close(DSVB_ENC *e, int id, uint8_t *out, long cap, long *len);
+/*
+ *   dsvb_dec_open       a stream id, or -1 when every lane holds one.  The stream knows no picture format yet.
+ *   dsvb_dec_push       one packet of any type per listed stream: pkts[k] / lens[k] the host bytes of stream ids[k]'s
+ *                       packet (always required: heads are parsed on the host), pkts_dev (optional, may be NULL, as
+ *                       may an entry) a device copy of the same bytes.  codes[k] / fnums[k] are what dsv_dec returns:
+ *                         DSV_DEC_GOT_META  metadata packet (fnum -1);
+ *                         DSV_DEC_OK        picture written to out[k] (host, or device with out_on_device = 1) in the
+ *                                           layout of dsvb_decode (dsvb_dec_set_out420p / _set_draw_info apply);
+ *                                           out or out[k] NULL decodes for reference only.  fnum = -1: a picture
+ *                                           before any metadata, skipped (dsv_decoder.c:327-331);
+ *                         DSV_DEC_EOS       end-of-stream packet (fnum -1);
+ *                         DSV_DEC_ERROR     malformed packet, a P picture without a reference (fnum = its frame
+ *                                           number), or a metadata packet this object cannot take: an unsupported
+ *                                           format, or another format than the object's while another open stream
+ *                                           has had metadata (the format changes only when no other stream depends
+ *                                           on it; that stream stays as it was).
+ *                       The picture packets of all listed streams decode in one engine step, and the pictures are
+ *                       complete in out when the call returns.  Returns 0; -2 if an id is out of range, not open or
+ *                       listed twice (nothing is read, no state changes); -100 on a CUDA failure.
+ *   dsvb_dec_close      frees the stream's lane (no-op for an id that is not open).
+ */
+int dsvb_dec_open(DSVB_DEC *d);
+int dsvb_dec_push(DSVB_DEC *d, int n, const int *ids, const uint8_t *const *pkts, const uint8_t *const *pkts_dev,
+                  const long *lens, uint8_t *const *out, int out_on_device, int *codes, long long *fnums);
+void dsvb_dec_close(DSVB_DEC *d, int id);
 
 /* pinned host memory for inputs / outputs of the calls above */
 void *dsvb_host_alloc(size_t bytes);
